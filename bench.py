@@ -1,11 +1,15 @@
 """bench.py - agent-steps/sec of the fused MPE step + observe + reward + actor path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--envs B_per_gpu] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--envs B_per_gpu] [--impl reference] [--dump-outputs DIR]
 
 One JSON line on stdout (rank 0).  Workload = BASELINE.json configs[1]: simple_spread, N = L = 3,
 65,536 env instances per GPU, one launch of the fused kernel (observe -> actor forward -> hard Gumbel
 sample -> World.step -> reward -> auto-reset every 25 steps) per "step"; weak scaling (per-GPU
 work fixed).  See DESIGN.md "Measurement" for how every field is derived.
+
+--dump-outputs DIR writes what the last timed step returned (obs_next, rew, act of rank 0) as DIR/<name>.npy.
+The env, the actor weights and the sampling noise are seeded, so two builds run with the same arguments can be
+compared output for output.  The bench writes nothing into the source tree (no bytecode either).
 """
 import argparse
 import json
@@ -17,6 +21,8 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True  # the bench writes nothing into the tree: tools/ and oracle/ modules build() never
+#                                 imported would otherwise leave __pycache__ directories there
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -60,7 +66,34 @@ def parse():
     ap.add_argument('--impl', default='b200', choices=['b200', 'reference'])
     ap.add_argument('--cpu-seconds', type=float, default=12.0, help='budget of the cpu_baseline sample')
     ap.add_argument('--no-extras', action='store_true', help='skip the env-only / 1M-env side measurements')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the outputs of the last timed step as DIR/<name>.npy (float32)')
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs needs --impl b200')
+    return args
+
+
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Each array (env rows first) as out_dir/<name>.npy in float32; the action indices 0..4 are exact in it.  Above
+    DUMP_MAX_BYTES in all, the same fixed, seeded sample of env rows is kept from every array, and its row numbers go
+    to out_dir/env_index.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    rows = next(iter(arrays.values())).shape[0]
+    row_bytes = sum(4 * a[0].numel() for a in arrays.values())
+    keep = min(rows, (DUMP_MAX_BYTES - 8 * rows) // row_bytes)
+    idx = None
+    if keep < rows:
+        idx = np.sort(np.random.RandomState(0).choice(rows, keep, replace=False))
+        np.save(os.path.join(out_dir, 'env_index.npy'), idx.astype(np.float64))
+    for name, a in arrays.items():
+        a = a.detach().float().cpu().numpy()
+        np.save(os.path.join(out_dir, name + '.npy'), a if idx is None else a[idx])
 
 
 def peaks():
@@ -325,6 +358,8 @@ def run_b200(args):
     side.synchronize()
     sync_all()
     per_step = [a.elapsed_time(b) for a, b in ev]
+    if args.dump_outputs and rank == 0:  # 65,536 envs: 7.9 MB of observations, 0.8 MB each of rewards and actions
+        dump_outputs(args.dump_outputs, {'obs_next': obs_next[0], 'rew': rew[0], 'act': act[0]})
     ms = sum(per_step)
     ms = D.max_over_ranks(ms, device=dev)
     clk = clocks.stop()

@@ -94,12 +94,14 @@ def gen_mpe(scenario, n, B, seed):
 TREASURE_SEED = 20240607  # Philox key of the fixture's respawn draws (global env id = row index, episode 0)
 
 
-def gen_treasure(B, seed, T=T):
+def gen_treasure(B, seed, T=T, keep=24):
     """``mpe_fullobs_collect_treasure.npz``: the loop oracle of the MAAC-fork scenario (oracle/maac_ref.py) from
     crafted initial states - collectors on / next to treasures, collectors that hold a treasure next to the matching
     (and the wrong) deposit, a dead treasure that respawns in the first post_step, agents in contact across the three
     mass pairings - under seeded random actions.  Respawn draws come from the kernels' Philox stream
-    (seed TREASURE_SEED, env id = row, episode 0, step t), so a CUDA env seeded alike reproduces the file."""
+    (seed TREASURE_SEED, env id = row, episode 0, step t), so a CUDA env seeded alike reproduces the file.
+    Only the first ``keep`` of the B envs are stored (four of each of the six kinds of crafted state at 24), which
+    keeps the file under 1 MB; rows are independent, so they are the same as in a run of ``keep`` envs."""
     from oracle import maac_ref, mpe_ref
     rng = np.random.RandomState(seed)
     env = mpe_ref.make_env('fullobs_collect_treasure')
@@ -157,6 +159,8 @@ def gen_treasure(B, seed, T=T):
             vel[t, b] = np.stack([a.state.p_vel for a in env.world.agents])
             tr[t, b] = np.stack([l.state.p_pos for l in env.world.landmarks])
             flags[t, b] = maac_ref.get_flags(env)
+    pos0, vel0, tr0, flags0, obs0 = pos0[:keep], vel0[:keep], tr0[:keep], flags0[:keep], obs0[:keep]
+    act_u, pos, vel, tr, obs, rew, flags, info = (x[:, :keep] for x in (act_u, pos, vel, tr, obs, rew, flags, info))
     name = 'mpe_fullobs_collect_treasure.npz'
     np.savez_compressed(os.path.join(GOLD, name), pos0=pos0, vel0=vel0, tr0=tr0, flags0=flags0, act_u=act_u, obs0=obs0,
                         pos=pos, vel=vel, tr=tr, obs=obs, rew=rew, flags=flags, info=info, seed=np.int64(TREASURE_SEED))

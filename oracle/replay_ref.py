@@ -1,6 +1,6 @@
 """Restatement of the reference replay ring (rls/replay_buffer.py:9-60: ReplayBuffer.add / _encode_sample /
 sample_index) fed the way experiments/run.py:46,52 feeds it.  TEST INFRASTRUCTURE (see oracle/__init__.py).
-Pinned against the reference's own class in tests/test_oracle.py when /root/reference is importable."""
+Pinned against the reference's own class in tests/test_reference_exec.py where it is compiled into oracle/_ref."""
 import numpy as np
 
 

@@ -189,26 +189,6 @@ def test_init_state_dict_shapes():
     assert sum(v.size for v in actor_ref.init_state_dict(10, 5, 0).values()) == 26117
 
 
-def test_replay_restatement_matches_reference_class():
-    import sys
-    if not os.path.isdir('/root/reference'):
-        pytest.skip('reference tree not present')
-    sys.path.insert(0, '/root/reference')
-    from rls.replay_buffer import ReplayBuffer
-    from oracle import replay_ref
-    rng = np.random.RandomState(0)
-    ref, mine = ReplayBuffer(size=7), replay_ref.ReplayRing(7)
-    for t in range(19):
-        # ndarray entries: the reference's np.array(x, copy=False) (replay_buffer.py:44) rejects lists on numpy 2
-        tr = (rng.randn(3, 4), np.eye(5)[rng.randint(5, size=3)], np.float64(rng.randn()), rng.randn(3, 4),
-              np.float64(t % 2))
-        ref.add(*tr); mine.add(*tr)
-        assert len(ref) == len(mine) and ref._next_idx == mine._next_idx
-    idx = [0, 6, 3, 3, 1]
-    for a, b in zip(ref.sample_index(idx), mine.sample_index(idx)):
-        assert np.array_equal(a, b)
-
-
 @pytest.mark.parametrize('tag', ['spread_n3', 'reference', 'model_n12'])
 def test_critic_restatement_matches_reference_network(golden_dir, tag):
     """tests/golden/critic_*.npz are outputs of the reference's CriticNetwork classes (fp32, CPU)."""
