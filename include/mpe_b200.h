@@ -35,7 +35,7 @@
 extern "C" {
 #endif
 
-#define MPE_ABI_VERSION 2
+#define MPE_ABI_VERSION 3
 
 enum { MPE_OK = 0, MPE_EINVAL = -1, MPE_ECUDA = -2, MPE_EUNSUPPORTED = -3 };
 enum { MPE_SIMPLE_SPREAD = 0, MPE_SIMPLE_REFERENCE = 1, MPE_SIMPLE_SPEAKER_LISTENER = 2,
@@ -187,9 +187,8 @@ int actor_destroy(MpeActor *actor);
 int actor_load(MpeActor *actor, const ActorWeights *w, void *stream);
 
 /* Implementation of the actor GEMMs: 0 = auto (tensor cores where supported), 1 = fp32 SIMT (FFMA),
- * 2 = tcgen05 tensor cores with fp16 hi/lo split operands (fp32-level accuracy; 2/3/4/6/9/12 agents),
- * 3 = like 2, and mpe_rollout runs teams of 6 / 9 / 12 agents as ONE kernel for all T steps instead of actor + step
- *     kernels per step (same results bit for bit; measured slower at large batches, fewer launches at small ones). */
+ * 2 = tcgen05 tensor cores with fp16 hi/lo split operands (fp32-level accuracy; 2/3/4/6/8/9/12 agents).
+ * Other values: MPE_EINVAL. */
 int actor_set_impl(MpeActor *actor, int32_t impl);
 
 /* Trainer.get_exploration_action - rls/agent/multiagent/ddpg_gumbel_fix.py:86-107:

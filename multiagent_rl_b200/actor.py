@@ -33,7 +33,7 @@ class FusedActor(object):
     ``state_dict``: mapping with the reference's key names (torch tensors or numpy arrays).
     """
 
-    IMPLS = {'auto': 0, 'simt': 1, 'tc': 2, 'tc_fused_large': 3}
+    IMPLS = {'auto': 0, 'simt': 1, 'tc': 2}
 
     def __init__(self, state_dict, device=None, seed=0, impl='auto'):
         if not torch.cuda.is_available():
@@ -68,8 +68,7 @@ class FusedActor(object):
             self._h = None
 
     def set_impl(self, impl):
-        """'auto' (tensor cores where supported), 'simt' (fp32 FFMA), 'tc' (tcgen05, fp16 hi/lo split) or
-        'tc_fused_large' ('tc' + single-kernel rollouts for teams of 6 / 9 / 12 agents)."""
+        """'auto' (tensor cores where supported), 'simt' (fp32 FFMA) or 'tc' (tcgen05, fp16 hi/lo split)."""
         _lib.check(self._lib.actor_set_impl(self._h, self.IMPLS[impl]), 'actor_set_impl')
         self.impl = impl
 

@@ -1,10 +1,9 @@
-// Actor forward (dense1 -> BiLSTM over the agent axis -> dense2 heads -> hard Gumbel sample) and the
-// fused rollout step (observe -> actor -> sample -> physics -> reward -> auto-reset), fp32 SIMT.
+// Actor forward (dense1 -> BiLSTM over the agent axis -> dense2 heads -> hard Gumbel sample), fp32 SIMT, and the
+// dense3 head that follows the tensor-core forward.
 //
 // Reference rows: rls/model/ac_network_multi_gumbel.py:52-67 (forward), :7-21 (TimeDistributed),
 // rls/model/ac_network_model_multi_gumbel.py:49,65 (dense3 head),
-// rls/agent/multiagent/ddpg_gumbel_fix.py:86-116 (get_exploration_action, gumbel_softmax hard=True),
-// experiments/run.py:36-65 (the loop body the rollout kernel fuses).
+// rls/agent/multiagent/ddpg_gumbel_fix.py:86-116 (get_exploration_action, gumbel_softmax hard=True).
 //
 // Shape of the computation: per env the LSTM is N sequential steps of a [96 -> 128] GEMV per
 // direction; batching TB envs turns each step into a [TB x 96] x [96 x 128] GEMM whose B operand
@@ -18,7 +17,7 @@
 #include <cstring>
 
 #include "actor_launch.h"
-#include "env_core.cuh"
+#include "common.cuh"
 
 namespace mpe {
 
@@ -143,7 +142,7 @@ template <int N, int TB, int PAD>
 struct ActorSmem {
   static constexpr int TBP = TB + PAD;
   static constexpr int RT = TB / 8;
-  float *w, *h1, *hc, *obs, *rew;
+  float *w, *h1, *hc, *obs, *rew;  // rew: no reader; dropping it moves sm.act, a layout change to measure on its own
   int *act;
   uint64_t *bars;
   __host__ __device__ static size_t bytes(size_t blob_floats, int D) {
@@ -371,160 +370,6 @@ __global__ void __launch_bounds__(kActorThreads, 1) k_actor_forward(ActorDev w, 
   }
 }
 
-#ifdef MPE_AB_KERNELS  // the fp32 FFMA fused rollout: superseded by k_tc2, A/B builds only
-// ------------------------------------------------------------------------------------------------
-// fused rollout: T x (observe -> actor -> sample -> World.step -> reward -> auto-reset)
-// ------------------------------------------------------------------------------------------------
-template <int SC, int N, int TB, int PAD>
-__global__ void __launch_bounds__(kActorThreads, 1)
-    k_rollout(EnvState<float> s, ActorDev w, RolloutIO ro, int max_episode_len, int64_t ntiles) {
-  extern __shared__ __align__(128) float smem_f[];
-  using Dm = Dims<SC, N>;
-  constexpr int D = Dm::D, R = Dm::R;
-  ActorSmem<N, TB, PAD> sm;
-  sm.carve(smem_f, w.smem_floats, D);
-  const int tid = threadIdx.x;
-  if (tid == 0) {
-    mbar_init(&sm.bars[0], 1);
-    mbar_fence_init();
-    mbar_expect_tx(&sm.bars[0], (uint32_t)(w.smem_floats * sizeof(float)));
-    bulk_load(sm.w, w.blob, (uint32_t)(w.smem_floats * sizeof(float)), &sm.bars[0]);
-  }
-  __syncthreads();
-  bool have_w = false;
-  ActorIO io;  // only the sampling fields are used by actor_tile here
-  io.seed = s.seed; io.gid0 = s.gid0; io.B = s.B; io.N = N;
-  for (int64_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
-    const int64_t env0 = tile * TB;
-    const int valid = (int)((s.B - env0) < TB ? (s.B - env0) : TB);
-    const bool full = valid == TB;
-    const bool mine = tid < valid;  // thread e < valid owns env env0 + e in the env phases
-    const int64_t b = env0 + tid;
-    // observe: rows of this tile from the SoA state
-    if (tid < TB) {
-      if (mine) {
-        Env<float, SC, N> e;
-        float comm[2][10];
-        e.load(s, b);
-        if (SC == kReference) {
-#pragma unroll
-          for (int i = 0; i < 2; ++i)
-#pragma unroll
-            for (int k = 0; k < 10; ++k) comm[i][k] = s.comm[((int64_t)i * 10 + k) * s.B + b];
-        }
-#pragma unroll
-        for (int i = 0; i < N; ++i) e.obs_row(i, sm.obs + tid * R + i * D, SC == kReference ? comm[1 - (i & 1)] : nullptr);
-      } else {
-        for (int i = 0; i < R; ++i) sm.obs[tid * R + i] = 0.0f;
-      }
-    }
-    __syncthreads();
-    if (!have_w) {
-      mbar_wait(&sm.bars[0], 0);
-      have_w = true;
-    }
-#pragma unroll 1
-    for (int t = 0; t < ro.T; ++t) {
-      actor_tile<N, TB, PAD>(w, sm, io, env0, valid, ro.step0 + (uint64_t)t);
-      const int64_t toff = (int64_t)t * s.B;
-      write_actions<N, TB>(sm.act, ro.act_u ? ro.act_u + toff * N : nullptr, ro.act_c ? ro.act_c + toff * N : nullptr,
-                           nullptr, env0, valid, w.A0, w.A);
-      // env phase: one thread per env
-      bool do_reset = false;
-      Env<float, SC, N> e;
-      float comm[2][10];
-      double ret = 0.0, n_ep = 0.0, n_steps = 0.0;
-      if (mine) {
-        e.load(s, b);
-        int au[N];
-#pragma unroll
-        for (int i = 0; i < N; ++i) au[i] = sm.act[(tid * N + i) * 2];
-        e.physics(au, s);
-        if (SC == kReference) {
-#pragma unroll
-          for (int i = 0; i < 2; ++i) {
-            const int ci = sm.act[(tid * N + i) * 2 + 1];
-#pragma unroll
-            for (int k = 0; k < 10; ++k) comm[i][k] = k == ci ? 1.0f : 0.0f;
-          }
-        }
-        float r[N];
-        int coll[N], occ;
-        float md;
-        e.reward(r, coll, occ, md, s);
-        float sum = 0.0f;
-#pragma unroll
-        for (int i = 0; i < N; ++i) { sum += r[i]; sm.rew[tid * N + i] = r[i]; }
-        const float ep_ret = s.ep_ret[b] + sum;
-        const int ts = s.tstep[b] + 1;
-        do_reset = max_episode_len > 0 && ts >= max_episode_len;
-        // the transition's next observation (what experiments/run.py:52 stores)
-#pragma unroll
-        for (int i = 0; i < N; ++i) e.obs_row(i, sm.obs + tid * R + i * D, SC == kReference ? comm[1 - (i & 1)] : nullptr);
-        if (do_reset) {
-          ret = (double)ep_ret; n_ep = 1.0; n_steps = (double)ts;
-          s.ep_ret[b] = 0.0f; s.tstep[b] = 0;
-        } else {
-          s.ep_ret[b] = ep_ret; s.tstep[b] = ts;
-        }
-      }
-      if ((tid & ~31) < TB) fold_stats(s.stats, ret, n_ep, n_steps);  // whole warps that own envs
-      // hand the tile's next-obs / rewards to the TMA engine (contiguous spans of the [B][N][.] outputs)
-      const bool want_out = ro.obs_next != nullptr || ro.rew != nullptr;
-      if (want_out) {
-        float *g_obs = ro.obs_next != nullptr ? ro.obs_next + (toff + env0) * R : nullptr;
-        float *g_rew = ro.rew != nullptr ? ro.rew + (toff + env0) * N : nullptr;
-        // TMA bulk stores need 16 B aligned destinations ([t][B] slices are not when B is odd)
-        const bool tma_ok = ((reinterpret_cast<uintptr_t>(g_obs) | reinterpret_cast<uintptr_t>(g_rew)) & 15) == 0;
-        if (full && tma_ok) {
-          if (tid < TB) fence_proxy_async_smem();
-          __syncthreads();
-          if (tid == 0) {
-            if (g_obs != nullptr) bulk_store(g_obs, sm.obs, TB * R * sizeof(float));
-            if (g_rew != nullptr) bulk_store(g_rew, sm.rew, TB * N * sizeof(float));
-            bulk_commit();
-            bulk_wait_read_all();
-          }
-          __syncthreads();
-        } else {
-          __syncthreads();
-          if (ro.obs_next != nullptr)
-            for (int i = tid; i < valid * R; i += kActorThreads) ro.obs_next[(toff + env0) * R + i] = sm.obs[i];
-          if (ro.rew != nullptr)
-            for (int i = tid; i < valid * N; i += kActorThreads) ro.rew[(toff + env0) * N + i] = sm.rew[i];
-          __syncthreads();
-        }
-      }
-      if (mine) {
-        if (do_reset) {  // experiments/run.py:59-60: obs_n = env.reset()
-          const uint32_t ep = s.episode[b] + 1u;
-          s.episode[b] = ep;
-          e.reset(s.seed, (uint64_t)(s.gid0 + b), ep);
-          e.store_world(s, b);
-          if (SC == kReference) {
-#pragma unroll
-            for (int i = 0; i < 2; ++i)
-#pragma unroll
-              for (int k = 0; k < 10; ++k) comm[i][k] = 0.0f;
-          }
-#pragma unroll
-          for (int i = 0; i < N; ++i) e.obs_row(i, sm.obs + tid * R + i * D, SC == kReference ? comm[1 - (i & 1)] : nullptr);
-        }
-        e.store_agents(s, b);
-        if (SC == kReference) {
-#pragma unroll
-          for (int i = 0; i < 2; ++i)
-#pragma unroll
-            for (int k = 0; k < 10; ++k) s.comm[((int64_t)i * 10 + k) * s.B + b] = comm[i][k];
-        }
-      }
-      __syncthreads();  // sm.obs now holds the observations the next iteration's actor reads
-    }
-  }
-}
-
-#endif  // MPE_AB_KERNELS
-
 // ------------------------------------------------------------------------------------------------
 // dense3 head of the "+model" actor on top of the tensor-core forward: next_state[row][j] = b3[j] + sum_k
 // relu(hcat)[row][k] W3[k][j] (ac_network_model_multi_gumbel.py:49,65).  64 x D MACs per row - HBM-bound on reading
@@ -725,39 +570,5 @@ cudaError_t launch_actor_forward(const ActorDev &w, const ActorIO &io, cudaStrea
     default: return cudaErrorInvalidValue;
   }
 }
-
-#ifdef MPE_AB_KERNELS
-template <int SC, int N, int TB, int PAD>
-static cudaError_t launch_rollout_t(const EnvStateAny &a, const ActorDev &w, const RolloutIO &ro, cudaStream_t st) {
-  const size_t smem = ActorSmem<N, TB, PAD>::bytes(w.smem_floats, w.D);
-  cudaError_t e = cudaFuncSetAttribute(k_rollout<SC, N, TB, PAD>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (e != cudaSuccess) return e;
-  EnvState<float> s;
-  s.pv = static_cast<float *>(a.pv); s.lm = static_cast<float *>(a.lm); s.goal = a.goal; s.episode = a.episode;
-  s.tstep = a.tstep; s.ep_ret = static_cast<float *>(a.ep_ret); s.comm = static_cast<float *>(a.comm);
-  s.stats = a.stats; s.B = a.B; s.gid0 = a.gid0; s.seed = a.seed; s.max_speed = (float)a.max_speed;
-  s.accel = (float)a.accel; s.track = 1;
-  set_thresholds<float>(s, a.scenario);
-  const int64_t ntiles = (a.B + TB - 1) / TB;
-  const int grid = (int)(ntiles < sm_count() ? ntiles : sm_count());
-  k_rollout<SC, N, TB, PAD><<<grid, kActorThreads, smem, st>>>(s, w, ro, a.max_episode_len, ntiles);
-  return cudaGetLastError();
-}
-
-cudaError_t launch_rollout(const EnvStateAny &a, const ActorDev &w, const RolloutIO &ro, cudaStream_t st) {
-  if (a.scenario == kReference) return launch_rollout_t<kReference, 2, 64, 4>(a, w, ro, st);
-  if (a.scenario == kSpeaker) return launch_rollout_t<kSpeaker, 2, 64, 4>(a, w, ro, st);
-  switch (a.N) {
-    case 2: return launch_rollout_t<kSpread, 2, 64, 4>(a, w, ro, st);
-    case 3: return launch_rollout_t<kSpread, 3, 64, 4>(a, w, ro, st);
-    case 4: return launch_rollout_t<kSpread, 4, 32, 4>(a, w, ro, st);
-    case 6: return launch_rollout_t<kSpread, 6, 32, 0>(a, w, ro, st);
-    case 9: return launch_rollout_t<kSpread, 9, 16, 0>(a, w, ro, st);
-    case 12: return launch_rollout_t<kSpread, 12, 16, 0>(a, w, ro, st);
-    default: return cudaErrorInvalidValue;
-  }
-}
-
-#endif  // MPE_AB_KERNELS
 
 }  // namespace mpe

@@ -1,4 +1,4 @@
-// Host-side interface of the actor / fused-rollout kernels (actor_kernels.cu) used by cabi.cu.
+// Host-side interface of the actor kernels (actor_kernels.cu, tc_kernels.cu) used by cabi.cu.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -24,10 +24,10 @@ struct TcDev {
   int D = 0, Kx = 0, A0 = 0, A1 = 0, A = 0;
   uint32_t off_wih[2][2] = {}, off_whh[2][2] = {}, off_w1[2] = {};
   uint32_t off_w2f = 0, off_bg = 0, off_b1 = 0, off_b2 = 0;
-  float *scratch = nullptr;  // [148*2 pipelines][12 agents][16][128] forward-pass logits shares (teams of > 3 agents)
+  float *scratch = nullptr;  // tc_scratch_floats(SMs): per-CTA dense2 shares (teams of > 3 agents, two-head actors)
 };
 
-enum { kImplAuto = 0, kImplSimt = 1, kImplTc = 2, kImplTcFusedLarge = 3 };
+enum { kImplAuto = 0, kImplSimt = 1, kImplTc = 2 };
 
 struct ActorDev {
   TcDev tc;
@@ -70,7 +70,6 @@ struct RolloutIO {
   float *obs_next = nullptr;  // [T][B][N][D]
   float *rew = nullptr;       // [T][B][N]
   int32_t *act_u = nullptr, *act_c = nullptr;  // [T][B][N]
-  float *obs_work = nullptr;  // [B][N][D] large teams: holds the current observations on entry, rewritten every step
 };
 
 void actor_layout(int D, int A0, int A1, bool has_model, ActorDev *out);
@@ -88,6 +87,5 @@ cudaError_t launch_actor_forward_tc(const TcDev &w, const ActorIO &io, cudaStrea
 cudaError_t launch_rollout_tc(const EnvStateAny &env, const TcDev &w, const RolloutIO &io, cudaStream_t st);
 // next_state = dense3(hcat): the "+model" head (ac_network_model_multi_gumbel.py:49,65) on top of the tensor-core forward
 cudaError_t launch_dense3(const ActorDev &w, const float *hcat, int64_t rows, float *next_state, cudaStream_t st);
-cudaError_t launch_rollout(const EnvStateAny &env, const ActorDev &w, const RolloutIO &io, cudaStream_t st);
 
 }  // namespace mpe

@@ -58,7 +58,7 @@ struct MpeEnv {
   int32_t *h_act_u = nullptr, *h_act_c = nullptr;
   void *h_obs = nullptr, *h_rew = nullptr;
   uint8_t *h_done = nullptr;
-  // scratch of the multi-kernel rollout (teams of > 3 agents): current observations and sampled actions
+  // scratch of the per-step rollout (teams of > 3 agents, the FFMA actor): current observations and sampled actions
   float *r_obs = nullptr;
   int32_t *r_act = nullptr;
   // mpe_act_step_host_async: device mirror of the caller's observations and of its transition block
@@ -103,14 +103,51 @@ struct MpeReplay {
   int64_t idx_cap = 0;
 };
 
-// The tensor-core actor of large teams (N > 3) and of two-head actors writes per-cell logits shares to a scratch
-// buffer indexed by CTA: two launches in flight on different streams must not share it.
-static bool tc_uses_scratch(const MpeActor *a, int N) { return N > 3 || a->dev.tc.A > 8; }
 static cudaError_t ensure_tc_scratch(float **p, int device) {
   if (*p != nullptr) return cudaSuccess;
   int nsm = 0;
   cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, device);
   return cudaMalloc(p, mpe::tc_scratch_floats(nsm > 0 ? nsm : 148) * sizeof(float));
+}
+
+// The actor's tensor-core weights for a launch on the caller's stream.  The kernels of large teams (N > 3) and of
+// two-head actors write per-cell logits shares to a scratch buffer indexed by CTA: two launches in flight on
+// different streams must not share it, so a caller that passes `stream_scratch` gets that buffer (allocated on first
+// use) instead of the actor's own.
+static cudaError_t tc_for_stream(const MpeActor *a, int N, float **stream_scratch, mpe::TcDev *out) {
+  *out = a->dev.tc;
+  if (stream_scratch == nullptr || (N <= 3 && a->dev.tc.A <= 8)) return cudaSuccess;
+  cudaError_t e = ensure_tc_scratch(stream_scratch, a->device);
+  out->scratch = *stream_scratch;
+  return e;
+}
+
+static bool use_tc(const MpeActor *a, int N) {
+  return a->dev.impl != mpe::kImplSimt && mpe::tc_actor_supported(a->dev.tc, N);
+}
+
+// One actor forward on `st`: tensor cores where they cover the shape, else the fp32 FFMA kernel.
+static cudaError_t launch_actor(const MpeActor *a, const mpe::ActorIO &io, float **stream_scratch, cudaStream_t st) {
+  if (!use_tc(a, io.N)) return mpe::launch_actor_forward(a->dev, io, st);
+  mpe::TcDev tc;
+  cudaError_t e = tc_for_stream(a, io.N, stream_scratch, &tc);
+  return e != cudaSuccess ? e : mpe::launch_actor_forward_tc(tc, io, st);
+}
+
+// device mirrors of the mpe_*_host entry points, allocated on first use
+static cudaError_t ensure_host_mirrors(MpeEnv *env) {
+  const mpe::EnvStateAny &s = env->st;
+  const size_t rows = (size_t)s.B * s.N, rs = real_size(s.precision);
+  cudaError_t e = cudaSuccess;
+  auto alloc = [&](auto **p, size_t bytes) {
+    if (e == cudaSuccess && *p == nullptr) e = cudaMalloc(p, bytes);
+  };
+  alloc(&env->h_act_u, rows * sizeof(int32_t));
+  alloc(&env->h_act_c, rows * sizeof(int32_t));
+  alloc(&env->h_obs, rows * s.D * rs);
+  alloc(&env->h_rew, rows * rs);
+  alloc(&env->h_done, rows);
+  return e;
 }
 
 extern "C" {
@@ -278,13 +315,7 @@ static int mpe_step_host_impl(MpeEnv *env, const int32_t *act_u_host, const int3
   DeviceGuard g(env->device);
   const mpe::EnvStateAny &s = env->st;
   const size_t rows = (size_t)s.B * s.N, rs = real_size(s.precision);
-  if (env->h_act_u == nullptr) {
-    CK(cudaMalloc(&env->h_act_u, rows * sizeof(int32_t)));
-    CK(cudaMalloc(&env->h_act_c, rows * sizeof(int32_t)));
-    CK(cudaMalloc(&env->h_obs, rows * s.D * rs));
-    CK(cudaMalloc(&env->h_rew, rows * rs));
-    CK(cudaMalloc(&env->h_done, rows));
-  }
+  CK(ensure_host_mirrors(env));
   CK(cudaMemcpyAsync(env->h_act_u, act_u_host, rows * sizeof(int32_t), cudaMemcpyHostToDevice, st));
   if (act_c_host != nullptr)
     CK(cudaMemcpyAsync(env->h_act_c, act_c_host, rows * sizeof(int32_t), cudaMemcpyHostToDevice, st));
@@ -317,13 +348,7 @@ int mpe_reset_host_async(MpeEnv *env, void *obs_host, void *stream) {
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const mpe::EnvStateAny &s = env->st;
   const size_t rows = (size_t)s.B * s.N, rs = real_size(s.precision);
-  if (env->h_obs == nullptr) {
-    CK(cudaMalloc(&env->h_act_u, rows * sizeof(int32_t)));
-    CK(cudaMalloc(&env->h_act_c, rows * sizeof(int32_t)));
-    CK(cudaMalloc(&env->h_obs, rows * s.D * rs));
-    CK(cudaMalloc(&env->h_rew, rows * rs));
-    CK(cudaMalloc(&env->h_done, rows));
-  }
+  CK(ensure_host_mirrors(env));
   CK(mpe::launch_reset(s, nullptr, env->h_obs, 0, st));
   env->synced = true;
   env->host_tstep = 0;
@@ -375,11 +400,7 @@ int actor_create(const ActorConfig *cfg, MpeActor **out) {
   if (e == cudaSuccess) e = cudaMemset(a->dev.blob, 0, a->dev.blob_floats * sizeof(float));
   if (e == cudaSuccess) e = cudaMalloc(&a->dev.tc.blob, a->dev.tc.bytes);
   if (e == cudaSuccess) e = cudaMemset(a->dev.tc.blob, 0, a->dev.tc.bytes);
-  if (e == cudaSuccess) {
-    int nsm = 0;
-    cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, cfg->device);
-    e = cudaMalloc(&a->dev.tc.scratch, mpe::tc_scratch_floats(nsm > 0 ? nsm : 148) * sizeof(float));
-  }
+  if (e == cudaSuccess) e = ensure_tc_scratch(&a->dev.tc.scratch, cfg->device);
   if (e != cudaSuccess) {
     actor_destroy(a);  // frees whatever was allocated before the failure
     return fail_cuda(e, "actor_create: cudaMalloc");
@@ -436,13 +457,8 @@ int actor_load(MpeActor *a, const ActorWeights *w, void *stream) {
   return MPE_OK;
 }
 
-static bool use_tc(const MpeActor *a, int N, bool needs_simt) {
-  if (a->dev.impl == mpe::kImplSimt || needs_simt) return false;
-  return mpe::tc_actor_supported(a->dev.tc, N);
-}
-
 int actor_set_impl(MpeActor *a, int32_t impl) {
-  if (a == nullptr || impl < 0 || impl > 3) return fail(MPE_EINVAL, "actor_set_impl: bad argument");
+  if (a == nullptr || impl < mpe::kImplAuto || impl > mpe::kImplTc) return fail(MPE_EINVAL, "actor_set_impl: bad argument");
   a->dev.impl = impl;
   return MPE_OK;
 }
@@ -460,24 +476,21 @@ int actor_forward(MpeActor *a, const float *obs, int64_t B, int32_t N, const flo
   io.act_u = act_u; io.act_c = act_c; io.onehot = onehot;
   io.B = B; io.N = N; io.seed = seed; io.step = step; io.gid0 = env_id_offset;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if ((a->dev.impl == mpe::kImplTc || a->dev.impl == mpe::kImplTcFusedLarge) && !use_tc(a, N, false))
-    return fail(MPE_EUNSUPPORTED, "actor_forward: the tensor-core path covers 2/3/4/6/9/12 agents, obs_dim <= 32, <= 8 head entries for > 3 agents");
-  if (use_tc(a, N, false)) {
-    if (next_state != nullptr) {  // "+model" head: the forward leaves relu(hcat) behind, one small kernel applies dense3
-      const int64_t rows = B * N;
-      if (rows > a->hcat_rows) {
-        if (a->hcat != nullptr) { CK(cudaStreamSynchronize(st)); cudaFree(a->hcat); a->hcat = nullptr; a->hcat_rows = 0; }
-        CK(cudaMalloc(&a->hcat, (size_t)rows * 64 * sizeof(float)));
-        a->hcat_rows = rows;
-      }
-      io.hcat = a->hcat;
-      io.next_state = nullptr;
+  const bool tc = use_tc(a, N);
+  if (a->dev.impl == mpe::kImplTc && !tc)
+    return fail(MPE_EUNSUPPORTED, "actor_forward: the tensor-core path covers 2/3/4/6/8/9/12 agents, obs_dim <= 32, <= 8 head entries for > 3 agents");
+  if (tc && next_state != nullptr) {  // "+model" head: the forward leaves relu(hcat) behind, one small kernel applies dense3
+    const int64_t rows = B * N;
+    if (rows > a->hcat_rows) {
+      if (a->hcat != nullptr) { CK(cudaStreamSynchronize(st)); cudaFree(a->hcat); a->hcat = nullptr; a->hcat_rows = 0; }
+      CK(cudaMalloc(&a->hcat, (size_t)rows * 64 * sizeof(float)));
+      a->hcat_rows = rows;
     }
-    CK(mpe::launch_actor_forward_tc(a->dev.tc, io, st));
-    if (next_state != nullptr) CK(mpe::launch_dense3(a->dev, a->hcat, B * N, next_state, st));
-  } else {
-    CK(mpe::launch_actor_forward(a->dev, io, st));
+    io.hcat = a->hcat;
+    io.next_state = nullptr;
   }
+  CK(launch_actor(a, io, nullptr, st));
+  if (io.hcat != nullptr) CK(mpe::launch_dense3(a->dev, a->hcat, B * N, next_state, st));
   return MPE_OK;
 }
 
@@ -513,16 +526,7 @@ static int actor_forward_host_impl(MpeActor *a, const float *obs_host, int64_t B
   io.obs = m.obs; io.act_u = m.act_u; io.act_c = a->dev.A1 > 0 ? m.act_c : nullptr;
   io.onehot = onehot_host != nullptr ? m.onehot : nullptr;
   io.B = B; io.N = N; io.seed = seed; io.step = step; io.gid0 = env_id_offset;
-  if (use_tc(a, N, false)) {
-    mpe::TcDev tc = a->dev.tc;
-    if (slot > 0 && tc_uses_scratch(a, N)) {  // slots are in flight on different streams: own scratch each
-      CK(ensure_tc_scratch(&m.tc_scratch, a->device));
-      tc.scratch = m.tc_scratch;
-    }
-    CK(mpe::launch_actor_forward_tc(tc, io, st));
-  } else {
-    CK(mpe::launch_actor_forward(a->dev, io, st));
-  }
+  CK(launch_actor(a, io, slot > 0 ? &m.tc_scratch : nullptr, st));  // slots are in flight on different streams: own scratch each
   if (act_u_host != nullptr) CK(cudaMemcpyAsync(act_u_host, m.act_u, (size_t)rows * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
   if (act_c_host != nullptr && a->dev.A1 > 0)
     CK(cudaMemcpyAsync(act_c_host, m.act_c, (size_t)rows * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
@@ -591,16 +595,7 @@ int mpe_act_step_host_async(MpeEnv *env, MpeActor *actor, const float *obs_host,
   io.act_u = reinterpret_cast<int32_t *>(blk + l.off_act_u);
   io.act_c = actor->dev.A1 > 0 ? reinterpret_cast<int32_t *>(blk + l.off_act_c) : nullptr;
   io.B = s.B; io.N = s.N; io.seed = s.seed; io.step = step; io.gid0 = s.gid0;
-  if (use_tc(actor, s.N, false)) {
-    mpe::TcDev tc = actor->dev.tc;
-    if (tc_uses_scratch(actor, s.N)) {  // shards share the actor handle on different streams: scratch per env handle
-      CK(ensure_tc_scratch(&env->tc_scratch, env->device));
-      tc.scratch = env->tc_scratch;
-    }
-    CK(mpe::launch_actor_forward_tc(tc, io, st));
-  } else {
-    CK(mpe::launch_actor_forward(actor->dev, io, st));
-  }
+  CK(launch_actor(actor, io, &env->tc_scratch, st));  // shards share the actor handle on different streams: scratch per env handle
   CK(mpe::launch_step(s, io.act_u, io.act_c, nullptr, blk + l.off_obs, blk + l.off_rew, blk + l.off_done, nullptr, nullptr, st));
   if (s.track) env->host_tstep += 1; else env->synced = false;
   CK(cudaMemcpyAsync(block_host, blk, l.bytes, cudaMemcpyDeviceToHost, st));
@@ -637,38 +632,17 @@ int mpe_rollout(MpeEnv *env, MpeActor *actor, int32_t T, uint64_t step0, float *
     return fail(MPE_EUNSUPPORTED, "mpe_rollout: unsupported scenario / agent count");
   DeviceGuard g(env->device);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  mpe::RolloutIO io;
-  io.T = T; io.step0 = step0; io.obs_next = obs_next; io.rew = rew; io.act_u = act_u; io.act_c = act_c;
-  // One kernel for all T steps: teams of <= 3.  For the large simple_spread teams (6 / 9 / 12) the single-kernel form
-  // exists too but is 17 - 20 % SLOWER than actor + step kernels per step (measured, DESIGN.md 4.3: the env step wants
-  // the whole GPU's occupancy, inside the persistent actor kernel it runs on 8 warps per SM), so it is opt-in.
-  if (actor->dev.impl != mpe::kImplSimt && mpe::tc_rollout_supported(actor->dev.tc, env->st.N) &&
-      (env->st.N <= 3 || actor->dev.impl == mpe::kImplTcFusedLarge)) {
-    if (env->st.N > 3) {  // large teams: the kernel streams the observations from a work buffer it rewrites every step
-      const int64_t rows = env->st.B * env->st.N;
-      if (env->r_obs == nullptr) {
-        CK(cudaMalloc(&env->r_obs, (size_t)rows * env->st.D * sizeof(float)));
-        CK(cudaMalloc(&env->r_act, (size_t)rows * 2 * sizeof(int32_t)));
-      }
-      CK(mpe::launch_observe(env->st, env->r_obs, st));
-      io.obs_work = env->r_obs;
-    }
-    mpe::TcDev tcw = actor->dev.tc;
-    if (tc_uses_scratch(actor, env->st.N)) {
-      CK(ensure_tc_scratch(&env->tc_scratch, env->device));
-      tcw.scratch = env->tc_scratch;
-    }
+  // One kernel for all T steps: teams of 2 / 3 on the tensor cores (the large teams run faster as actor + step kernels
+  // per step, DESIGN.md 4.3)
+  if (actor->dev.impl != mpe::kImplSimt && mpe::tc_rollout_supported(actor->dev.tc, env->st.N)) {
+    mpe::RolloutIO io;
+    io.T = T; io.step0 = step0; io.obs_next = obs_next; io.rew = rew; io.act_u = act_u; io.act_c = act_c;
+    mpe::TcDev tcw;
+    CK(tc_for_stream(actor, env->st.N, &env->tc_scratch, &tcw));  // rollouts of several envs may share one actor
     CK(mpe::launch_rollout_tc(env->st, tcw, io, st));
     env->synced = false;
     return MPE_OK;
   }
-#ifdef MPE_AB_KERNELS
-  if (actor->dev.impl == mpe::kImplSimt) {  // A/B builds: the fp32 FFMA fused kernel
-    CK(mpe::launch_rollout(env->st, actor->dev, io, st));
-    env->synced = false;
-    return MPE_OK;
-  }
-#endif
   {
     // Every other combination (teams of > 3 agents, the fp32 FFMA actor): the same loop as kernels per step - actor
     // (tensor cores where the shape is covered, else FFMA), the env step kernel, and a reset kernel on the steps
@@ -680,12 +654,6 @@ int mpe_rollout(MpeEnv *env, MpeActor *actor, int32_t T, uint64_t step0, float *
       CK(cudaMalloc(&env->r_obs, (size_t)rows * s.D * sizeof(float)));
       CK(cudaMalloc(&env->r_act, (size_t)rows * 2 * sizeof(int32_t)));
     }
-    const bool tc = use_tc(actor, s.N, false);
-    mpe::TcDev tcw = actor->dev.tc;
-    if (tc && tc_uses_scratch(actor, s.N)) {  // rollouts of several envs may share one actor on different streams
-      CK(ensure_tc_scratch(&env->tc_scratch, env->device));
-      tcw.scratch = env->tc_scratch;
-    }
     CK(mpe::launch_observe(s, env->r_obs, st));
     const float *cur = env->r_obs;
     const int L = s.max_episode_len;
@@ -694,10 +662,7 @@ int mpe_rollout(MpeEnv *env, MpeActor *actor, int32_t T, uint64_t step0, float *
       aio.obs = cur; aio.B = s.B; aio.N = s.N; aio.seed = s.seed; aio.step = step0 + (uint64_t)t; aio.gid0 = s.gid0;
       aio.act_u = act_u != nullptr ? act_u + (int64_t)t * rows : env->r_act;
       if (s.act_c > 0) aio.act_c = act_c != nullptr ? act_c + (int64_t)t * rows : env->r_act + rows;
-      if (tc)
-        CK(mpe::launch_actor_forward_tc(tcw, aio, st));
-      else
-        CK(mpe::launch_actor_forward(actor->dev, aio, st));
+      CK(launch_actor(actor, aio, &env->tc_scratch, st));  // rollouts of several envs may share one actor on different streams
       float *o = obs_next != nullptr ? obs_next + (int64_t)t * rows * s.D : env->r_obs;
       CK(mpe::launch_step(s, aio.act_u, aio.act_c, nullptr, o, rew != nullptr ? rew + (int64_t)t * rows : nullptr, nullptr,
                           nullptr, nullptr, st));

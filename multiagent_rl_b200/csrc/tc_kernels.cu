@@ -1,4 +1,6 @@
-// Tensor-core (tcgen05 / TMEM) version of the actor forward and of the fused rollout step, N <= 3 agents.
+// Tensor-core (tcgen05 / TMEM) version of the actor forward (teams of 2, 3, 4, 6, 8, 9, 12) and of the fused
+// rollout step (teams of 2 and 3): one kernel, k_tc2, whose warp roles and TMEM / shared-memory layout are described
+// above its definition.
 //
 // Reference rows: same as actor_kernels.cu (rls/model/ac_network_multi_gumbel.py:52-67,
 // rls/agent/multiagent/ddpg_gumbel_fix.py:86-116, experiments/run.py:36-65).
@@ -9,17 +11,6 @@
 // split as x = hi + lo (two fp16 values, 22 significant bits) and each product is three kind::f16 MMAs
 // (hi*hi + lo*hi + hi*lo) accumulated in fp32 in TMEM.  Weights are pre-split (and pre-scaled by 16 so
 // that the lo halves stay normal) on the host; activations are split by the epilogue that produces them.
-//
-// One persistent CTA per SM, one tile = 128 envs = 128 TMEM lanes, thread r of each warpgroup owns env row r:
-//   warps 0-3  (WG0): epilogue of the forward  LSTM direction, sampling, physics/reward of env r
-//   warps 4-7  (WG1): epilogue of the backward LSTM direction
-//   warp  8         : lane 0 issues every tcgen05.mma of the CTA (one ordered stream)
-// TMEM columns:  [0,256)  gate accumulators G[dir] (aliased by the dense1 accumulators D1[t] before the LSTM)
-//                [256, 256+64N)  h1[t] as an fp16 hi/lo A operand (never leaves TMEM)
-//                [256+64N, +16N) logits[t] accumulators
-// Shared memory: fp16 hi/lo weight image (one TMA bulk load), obs A operands, recurrent h / relu(h) A operands.
-// The two directions form a natural ping-pong: while WG0 runs the cell math of step s, the tensor pipe runs
-// the gate GEMM of the other direction.
 #include <cuda_fp16.h>
 
 #include <cstdlib>
@@ -27,12 +18,10 @@
 
 #include "actor_launch.h"
 #include "env_core.cuh"
-#include "env_group.cuh"
 #include "tc_common.cuh"
 
 namespace mpe {
 
-constexpr int kTcThreads = 320;
 constexpr int kRows = 128;
 constexpr float kWScale = 16.0f, kWInv = 0.0625f, kLog2e = 1.4426950408889634f;
 constexpr uint32_t kChunkA = kRows * 16;  // bytes of one K-chunk (8 halves) of a 128-row A operand
@@ -157,16 +146,10 @@ __device__ unsigned long long g_tc_timeline[148 * 128];
 // barriers of one warpgroup's pipeline (indices into its own block of the barrier array)
 enum { B_X = 0, B_D1, B_H1, B_G, B_H, B_PER_WG };
 
-// observation A operands: all N agents resident for N <= 3; for larger teams a double buffer that is refilled just
-// in time, one cell ahead of the dense1 GEMM that consumes it
 // operand buffers: all agents resident (N <= 3); a ring of 4 (teams of 4 / 6: 16-wide operands, shared memory to
 // spare) or 2 (9 / 12 agents: 32-wide operands) buffers refilled ahead of the dense1 GEMMs
 __host__ __device__ constexpr int tc_x_slots(int N) { return N <= 3 ? N : (N <= 6 ? 4 : 2); }
 __host__ __device__ inline size_t tc_x_bytes(int N, int Kx) { return (size_t)tc_x_slots(N) * 2 * (Kx / 8) * kChunkA; }
-__host__ __device__ inline size_t tc_smem_bytes(uint32_t wbytes, int N, int Kx) {
-  // weight image + per warpgroup: obs operands, recurrent h operand (hi/lo), action indices; + barriers
-  return (size_t)wbytes + 2 * (tc_x_bytes(N, Kx) + 16384 + (size_t)((kRows * N * 2 + 127) / 128 * 128)) + (1 + 2 * B_PER_WG) * 8 + 64;
-}
 
 __device__ __forceinline__ float ex2_approx(float x) {
   float y;
@@ -281,459 +264,10 @@ __device__ __forceinline__ void lstm_chunk(const uint32_t (&v)[32], const float 
   }
 }
 
-#ifdef MPE_AB_KERNELS  // the superseded two-pipeline kernel: A/B builds only (python -m multiagent_rl_b200.build --variant ab MPE_AB_KERNELS)
 // ------------------------------------------------------------------------------------------------
-// the kernel: two independent tile pipelines per CTA (one per warpgroup), sharing the weight image
-//   warps 0-3 / 4-7 : warpgroup g = 0 / 1, thread r of the group owns env row r of the group's tile
-//   warps 8 / 9     : lane 0 issues every tcgen05.mma of warpgroup 0 / 1
-// TMEM columns of warpgroup g (base 256 g):  [0,128) gate accumulators of the current (direction, step)
-//                                            [128,192) dense1 accumulators of the next agent
-//                                            [192,256) h1 of the current agent as fp16 hi (32 cols) / lo (32 cols)
-// A warpgroup walks the 2N (direction, step) cells of its tile sequentially; while it waits for its gate GEMM
-// the other warpgroup's cell math fills the SM (the MUFU pipe is the shared bottleneck).
-// ------------------------------------------------------------------------------------------------
-template <int SC, int N, bool FUSED, int APAD>
-__global__ void __launch_bounds__(kTcThreads, 1)
-    k_tc(EnvState<float> s, TcDev w, ActorIO io, RolloutIO ro, int max_episode_len, int64_t ntiles, int dbg) {
-  extern __shared__ __align__(128) unsigned char smem[];
-  using Dm = Dims<SC, N>;
-  const int D = FUSED ? Dm::D : w.D;
-  const int R = N * D;
-  const int Kx = w.Kx;
-  constexpr bool kJit = N > 3;  // large teams: actor only, obs operands refilled per cell, logits via global scratch
-  static_assert(!(kJit && FUSED), "the fused env phase keeps every entity in registers: N <= 3");
-  const int tid = threadIdx.x, warp = tid >> 5;
-  const size_t xb = tc_x_bytes(N, Kx);
-  const size_t wg_bytes = xb + 16384 + (size_t)((kRows * N * 2 + 127) / 128 * 128);  // x, h, action indices (bytes)
-  unsigned char *sm_w = smem;
-  uint64_t *bars = reinterpret_cast<uint64_t *>(smem + w.bytes + 2 * wg_bytes);  // [0] = weights, then 2 x B_PER_WG
-  uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(bars + 1 + 2 * B_PER_WG);
-
-  if (tid == 0) {
-    mbar_init(&bars[0], 1);
-    for (int g = 0; g < 2; ++g) {
-      uint64_t *bb = bars + 1 + g * B_PER_WG;
-      mbar_init(&bb[B_X], 128);
-      mbar_init(&bb[B_D1], 1);
-      mbar_init(&bb[B_H1], 128);
-      mbar_init(&bb[B_G], 1);
-      mbar_init(&bb[B_H], 128);
-    }
-    mbar_fence_init();
-    mbar_expect_tx(&bars[0], w.bytes);
-    bulk_load(sm_w, w.blob, w.bytes, &bars[0]);
-  }
-  if (warp == 8) tmem_alloc(tmem_slot, 512);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-  const int T = FUSED ? ro.T : 1;
-  const int g = warp >= 8 ? warp - 8 : (tid >> 7);  // pipeline index
-  unsigned char *sm_x = smem + w.bytes + g * wg_bytes;
-  unsigned char *sm_h = sm_x + xb;                  // [hl][4][128][8] halves
-  uint8_t *sm_act = sm_h + 16384;  // [128][N][2] sampled head indices
-  float *stage_obs = reinterpret_cast<float *>(sm_x);  // fp32 rows for the TMA store (x is dead by then)
-  float *stage_rew = stage_obs + kRows * R;
-  uint64_t *bb = bars + 1 + g * B_PER_WG;
-  const uint32_t tmem = tmem_base + g * 256;
-  const uint32_t col_d1 = 128, col_h1 = 192;
-  const int64_t tile0 = (int64_t)blockIdx.x * 2 + g, tile_stride = (int64_t)gridDim.x * 2;
-
-  if (warp >= 8) {
-    // =============================== MMA issuer of pipeline g ===============================
-    if ((tid & 31) == 0) {
-      uint32_t ph_x = 0, ph_h1 = 0, ph_h = 0;
-      const uint32_t id_g = make_idesc_f16(128, 128), id_d1 = make_idesc_f16(128, 64);
-      mbar_wait(&bars[0], 0);
-      for (int64_t tile = tile0; tile < ntiles; tile += tile_stride) {
-        [[maybe_unused]] const bool first_tile = tile == tile0;
-        for (int it = 0; it < T; ++it) {
-          mbar_wait(&bb[B_X], ph_x); ph_x ^= 1;
-          tc_fence_after();
-          TL(2 + g, 0);
-          auto dense1 = [&](int t, int k) {  // k = cell that consumes it; large teams: x lives in slot k & 1
-            const int slot = kJit ? (k & 1) : t;
-            const unsigned char *xh = sm_x + (size_t)(slot * 2) * (Kx / 8) * kChunkA, *xl = xh + (size_t)(Kx / 8) * kChunkA;
-            mma3_ss(tmem + col_d1, xh, xl, kChunkA, sm_w + w.off_w1[0], sm_w + w.off_w1[1], kHid * 16, Kx / 16, id_d1, false);
-            mma_commit(&bb[B_D1]);
-          };
-          dense1(0, 0);
-          for (int k = 0; k < 2 * N; ++k) {
-            const int d = k / N, st = k - d * N;
-            mbar_wait(&bb[B_H1], ph_h1); ph_h1 ^= 1;  // h1 of this cell's agent is in TMEM (and D1 is free again)
-            if (k > 0) { mbar_wait(&bb[B_H], ph_h); ph_h ^= 1; }  // previous cell done: G free, recurrent h in smem
-            tc_fence_after();
-            TL(2 + g, 1 + 2 * k);
-            mma3_ts(tmem, tmem + col_h1, tmem + col_h1 + 32, sm_w + (d ? w.off_wih[1][0] : w.off_wih[0][0]), sm_w + (d ? w.off_wih[1][1] : w.off_wih[0][1]), kGateN * 16, 4,
-                    id_g, false);
-            if (st > 0) mma3_ss(tmem, sm_h, sm_h + 8192, kChunkA, sm_w + (d ? w.off_whh[1][0] : w.off_whh[0][0]),
-                                sm_w + (d ? w.off_whh[1][1] : w.off_whh[0][1]), kGateN * 16, 2, id_g, true);
-            mma_commit(&bb[B_G]);
-            if (k + 1 < 2 * N) {  // dense1 of the next cell's agent runs behind the gates on the tensor pipe
-              const int d2 = (k + 1) / N, s2 = k + 1 - d2 * N;
-              dense1(d2 == 0 ? s2 : N - 1 - s2, k + 1);
-            }
-            TL(2 + g, 2 + 2 * k);
-          }
-          mbar_wait(&bb[B_H], ph_h); ph_h ^= 1;  // keep the phase in step with the last cell
-        }
-      }
-    }
-    __syncwarp();
-  } else {
-    // =============================== epilogue warpgroup g ===============================
-    const int row = tid & 127;
-    const uint32_t lane_base = (uint32_t)(row & ~31) << 16;
-    const float *b1 = reinterpret_cast<const float *>(sm_w + w.off_b1);
-    const float *b2 = reinterpret_cast<const float *>(sm_w + w.off_b2);
-    const float *w2f = reinterpret_cast<const float *>(sm_w + w.off_w2f);  // [64][16] fp32
-    uint32_t ph_d1 = 0, ph_g = 0;
-    mbar_wait(&bars[0], 0);  // biases / dense2 weights are read from the weight image
-    // De-phase the two pipelines: group 1 starts once group 0 is waiting for its first gate GEMM, so that one
-    // group's tensor-pipe wait is covered by the other group's cell math instead of both idling in lockstep.
-    bool staggered = false;
-    if (g == 1) bar_sync_n(3, 256);
-    else if (tile0 >= ntiles) { asm volatile("bar.arrive 3, 256;" ::: "memory"); staggered = true; }
-    for (int64_t tile = tile0; tile < ntiles; tile += tile_stride) {
-      const int64_t env0 = tile * kRows;
-      const int64_t nb = FUSED ? s.B : io.B;
-      const int valid = (int)((nb - env0) < kRows ? (nb - env0) : kRows);
-      const bool mine = row < valid;
-      const int64_t b = env0 + row;
-      [[maybe_unused]] const bool first_tile = tile == tile0 && row == 0;
-      for (int it = 0; it < T; ++it) {
-        TL(g, 0);
-        // ---- observations -> fp16 hi/lo A operands ----
-        auto write_x_from_global = [&](int t, int slot) {  // actor mode: obs[b][t][:] -> x operand slot
-          float xr[32];
-#pragma unroll
-          for (int k = 0; k < 32; ++k) xr[k] = 0.0f;
-          if (mine) {
-            const float *src = io.obs + b * R + t * D;
-#pragma unroll
-            for (int k = 0; k < 32; ++k)
-              if (k < D) xr[k] = src[k];
-          }
-          unsigned char *xh = sm_x + (size_t)(slot * 2) * (Kx / 8) * kChunkA, *xl = xh + (size_t)(Kx / 8) * kChunkA;
-#pragma unroll
-          for (int c = 0; c < 4; ++c) {
-            if (c * 8 < Kx) {
-              const float v[8] = {xr[c * 8], xr[c * 8 + 1], xr[c * 8 + 2], xr[c * 8 + 3],
-                                  xr[c * 8 + 4], xr[c * 8 + 5], xr[c * 8 + 6], xr[c * 8 + 7]};
-              store_chunk_split(xh + c * kChunkA, xl + c * kChunkA, row, v);
-            }
-          }
-        };
-        if constexpr (kJit) {
-          write_x_from_global(0, 0);  // the first cell's agent; later cells refill one cell ahead
-        } else {
-          Env<float, SC, N> e;
-          float comm[2][10];
-          if (FUSED && mine) {
-            e.load(s, b);
-            if (SC == kReference) {
-#pragma unroll
-              for (int i = 0; i < 2; ++i)
-#pragma unroll
-                for (int k = 0; k < 10; ++k) comm[i][k] = s.comm[((int64_t)i * 10 + k) * s.B + b];
-            }
-          }
-#pragma unroll
-          for (int t = 0; t < N; ++t) {
-            if (FUSED) {
-              float xr[32];
-#pragma unroll
-              for (int k = 0; k < 32; ++k) xr[k] = 0.0f;
-              if (mine) e.obs_row(t, xr, SC == kReference ? comm[1 - (t & 1)] : nullptr);
-              unsigned char *xh = sm_x + (size_t)(t * 2) * (Kx / 8) * kChunkA, *xl = xh + (size_t)(Kx / 8) * kChunkA;
-#pragma unroll
-              for (int c = 0; c < 4; ++c) {
-                if (c * 8 < Kx) {
-                  const float v[8] = {xr[c * 8], xr[c * 8 + 1], xr[c * 8 + 2], xr[c * 8 + 3],
-                                      xr[c * 8 + 4], xr[c * 8 + 5], xr[c * 8 + 6], xr[c * 8 + 7]};
-                  store_chunk_split(xh + c * kChunkA, xl + c * kChunkA, row, v);
-                }
-              }
-            } else {
-              write_x_from_global(t, t);
-            }
-          }
-        }
-        fence_proxy_async_smem();
-        mbar_arrive(&bb[B_X]);
-        TL(g, 1);
-
-        // dense2 accumulators (both directions add into them): registers for small teams; for large teams the
-        // forward pass parks its share in a global scratch row and the backward pass finishes + samples per cell
-        constexpr int NLG = kJit ? 1 : N;
-        float lg[NLG][APAD];
-#pragma unroll
-        for (int t = 0; t < NLG; ++t)
-#pragma unroll
-          for (int a = 0; a < APAD; ++a) lg[t][a] = b2[a];
-        float *scratch = kJit ? w.scratch + ((size_t)(blockIdx.x * 2 + g) * N) * APAD * kRows : nullptr;
-        const uint64_t samp_step = FUSED ? ro.step0 + (uint64_t)it : io.step;
-        const uint64_t samp_seed = FUSED ? s.seed : io.seed;
-        const int64_t samp_gid0 = FUSED ? s.gid0 : io.gid0;
-        // F.gumbel_softmax(hard=True) of one agent's logits -> head indices (+ optional logits output)
-        auto sample_agent = [&](int t, const float (&lgt)[APAD], int &bu, int &bc) {
-          float z[APAD];
-          const int64_t orow = b * N + t;
-          if (!FUSED && io.gumbel != nullptr) {
-#pragma unroll
-            for (int a = 0; a < APAD; ++a) z[a] = (a < w.A && mine) ? lgt[a] + io.gumbel[orow * w.A + a] : lgt[a];
-          } else {
-#pragma unroll
-            for (int j = 0; j < APAD / 4; ++j) {
-              if (4 * j >= w.A) {  // uniform: no head entries in this block of four
-                z[4 * j] = z[4 * j + 1] = z[4 * j + 2] = z[4 * j + 3] = 0.0f;
-                continue;
-              }
-              const uint4 rr = philox_raw(samp_seed, (uint64_t)(samp_gid0 + b), (uint32_t)samp_step, kDomainGumbel, t * 8 + j);
-              const uint32_t bits[4] = {rr.x, rr.y, rr.z, rr.w};
-#pragma unroll
-              for (int q = 0; q < 4; ++q)
-                z[4 * j + q] = (4 * j + q < w.A) ? lgt[4 * j + q] + bits_to_gumbel(bits[q]) : 0.0f;
-            }
-          }
-          bu = 0; bc = 0;
-          float best = z[0];
-#pragma unroll
-          for (int a = 1; a < APAD; ++a)
-            if (a < w.A0 && z[a] > best) { best = z[a]; bu = a; }
-          if (w.A1 > 0) {
-            float bcv = -INFINITY;
-#pragma unroll
-            for (int a = 0; a < APAD; ++a)
-              if (a >= w.A0 && a < w.A && z[a] > bcv) { bcv = z[a]; bc = a - w.A0; }
-          }
-          sm_act[(row * N + t) * 2] = bu;
-          sm_act[(row * N + t) * 2 + 1] = bc;
-          if (!FUSED && mine && io.logits != nullptr) {
-#pragma unroll
-            for (int a = 0; a < APAD; ++a)
-              if (a < w.A) io.logits[orow * w.A + a] = lgt[a];
-          }
-        };
-
-#pragma unroll 1
-        for (int d = 0; d < 2; ++d) {
-          const float *bg = reinterpret_cast<const float *>(sm_w + w.off_bg) + d * kGateN;
-          f2 c[4][4];  // cell state of this thread's row: 4 chunks x 4 packed pairs of units
-#pragma unroll
-          for (int u = 0; u < 16; ++u) c[u >> 2][u & 3] = 0ull;
-#pragma unroll 1
-          for (int st = 0; st < N; ++st) {
-            const int t = d == 0 ? st : N - 1 - st;
-            f2 pl[APAD / 2];  // this cell's dense2 contribution (packed pairs), folded into lg[t] below
-#pragma unroll
-            for (int a = 0; a < APAD / 2; ++a) pl[a] = 0ull;
-            // ---- dense1 epilogue: h1 = relu(D1/16 + b1) -> fp16 hi/lo A operand in TMEM ----
-            mbar_wait(&bb[B_D1], ph_d1); ph_d1 ^= 1;
-            tc_fence_after();
-            TL(g, 2 + 4 * (d * N + st));
-            {
-              uint32_t v0[32], v1[32];
-              tmem_ld32(tmem + lane_base + col_d1, v0);
-              tmem_wait_ld();
-              tmem_ld32(tmem + lane_base + col_d1 + 32, v1);  // in flight while the first half is converted
-              dense1_half(v0, b1, tmem + lane_base + col_h1);
-              tmem_wait_ld();
-              dense1_half(v1, b1 + 32, tmem + lane_base + col_h1 + 16);
-            }
-            if constexpr (kJit) {  // obs operand of the NEXT cell's agent (its dense1 GEMM is issued after this arrival)
-              const int k1 = d * N + st + 1;
-              if (k1 < 2 * N) {
-                const int d1 = k1 / N, s1 = k1 - d1 * N;
-                write_x_from_global(d1 == 0 ? s1 : N - 1 - s1, k1 & 1);
-                fence_proxy_async_smem();
-              }
-            }
-            tmem_wait_st();
-            tc_fence_before();
-            mbar_arrive(&bb[B_H1]);
-            if (g == 0 && !staggered) { asm volatile("bar.arrive 3, 256;" ::: "memory"); staggered = true; }
-            TL(g, 3 + 4 * (d * N + st));
-
-            // ---- LSTM cell math on the gate accumulators ----
-            mbar_wait(&bb[B_G], ph_g); ph_g ^= 1;
-            tc_fence_after();
-            TL(g, 4 + 4 * (d * N + st));
-            // Two chunks (2 x 8 units x [i f g o]) per rolled iteration: the loop body stays inside the
-            // instruction cache, the TMEM load of the next chunk flies while this chunk's cell math runs, and
-            // the cell state rotates through c[0..3] so that the live chunk always has compile-time indices.
-            uint32_t va[32], vb[32];
-            tmem_ld32(tmem + lane_base, va);
-#pragma unroll 1
-            for (int up = 0; up < 2; ++up) {
-              tmem_wait_ld();
-              tmem_ld32(tmem + lane_base + (2 * up + 1) * 32, vb);
-              lstm_chunk<APAD>(va, bg + (2 * up) * 32, w2f + (d * kH + (2 * up) * 8) * 16, c[0], pl,
-                               sm_h + (2 * up) * kChunkA, row, st < N - 1);
-              tmem_wait_ld();
-              if (up == 0) tmem_ld32(tmem + lane_base + 2 * 32, va);
-              lstm_chunk<APAD>(vb, bg + (2 * up + 1) * 32, w2f + (d * kH + (2 * up + 1) * 8) * 16, c[1], pl,
-                               sm_h + (2 * up + 1) * kChunkA, row, st < N - 1);
-#pragma unroll
-              for (int j = 0; j < 4; ++j) {  // rotate: after two iterations every group is back in place
-                const f2 t0 = c[0][j], t1 = c[1][j];
-                c[0][j] = c[2][j]; c[1][j] = c[3][j];
-                c[2][j] = t0; c[3][j] = t1;
-              }
-            }
-            fence_proxy_async_smem();
-            tc_fence_before();
-            mbar_arrive(&bb[B_H]);
-            if constexpr (kJit) {
-              float *srow = scratch + (size_t)t * APAD * kRows + row;
-              float p[APAD];
-#pragma unroll
-              for (int a = 0; a < APAD / 2; ++a) upk(pl[a], p[2 * a], p[2 * a + 1]);
-              if (d == 0) {  // park the forward share (coalesced over the rows of the tile)
-#pragma unroll
-                for (int a = 0; a < APAD; ++a) srow[a * kRows] = p[a];
-              } else {       // backward share arrives: logits of agent t are complete -> sample now
-                float lgt[APAD];
-#pragma unroll
-                for (int a = 0; a < APAD; ++a) lgt[a] = (lg[0][a] + srow[a * kRows]) + p[a];
-                int bu, bc;
-                sample_agent(t, lgt, bu, bc);
-              }
-            } else {
-#pragma unroll
-              for (int tt = 0; tt < N; ++tt)
-                if (tt == t) {
-#pragma unroll
-                  for (int a = 0; a < APAD / 2; ++a) {
-                    float p0, p1;
-                    upk(pl[a], p0, p1);
-                    lg[tt][2 * a] += p0; lg[tt][2 * a + 1] += p1;
-                  }
-                }
-            }
-            TL(g, 5 + 4 * (d * N + st));
-          }
-        }
-
-        // ---- Gumbel-max sampling (small teams; large teams sampled inside the backward pass) ----
-        int au[N], ac[N];
-        if constexpr (!kJit) {
-#pragma unroll
-          for (int t = 0; t < N; ++t) sample_agent(t, lg[t], au[t], ac[t]);
-        }
-        TL(g, 28);
-
-        if (FUSED) {
-          // ---- World.step + reward + outputs for env row `row` ----
-          const int64_t toff = (int64_t)it * s.B;
-          bool do_reset = false;
-          Env<float, SC, N> e;
-          float comm[2][10];
-          double ret = 0.0, n_ep = 0.0, n_steps = 0.0;
-          if (mine) {
-            e.load(s, b);
-            e.physics(au, s);
-            if (SC == kReference) {
-#pragma unroll
-              for (int i = 0; i < 2; ++i)
-#pragma unroll
-                for (int k = 0; k < 10; ++k) comm[i][k] = k == ac[i] ? 1.0f : 0.0f;
-            }
-            float r[N];
-            int coll[N], occ;
-            float md;
-            e.reward(r, coll, occ, md, s);
-            float sum = 0.0f;
-#pragma unroll
-            for (int i = 0; i < N; ++i) { sum += r[i]; stage_rew[row * N + i] = r[i]; }
-            const float ep_ret = s.ep_ret[b] + sum;
-            const int ts = s.tstep[b] + 1;
-            do_reset = max_episode_len > 0 && ts >= max_episode_len;
-#pragma unroll
-            for (int i = 0; i < N; ++i) e.obs_row(i, stage_obs + row * R + i * D, SC == kReference ? comm[1 - (i & 1)] : nullptr);
-            if (do_reset) {
-              ret = (double)ep_ret; n_ep = 1.0; n_steps = (double)ts;
-              s.ep_ret[b] = 0.0f; s.tstep[b] = 0;
-            } else {
-              s.ep_ret[b] = ep_ret; s.tstep[b] = ts;
-            }
-          }
-          fold_stats(s.stats, ret, n_ep, n_steps);
-          float *g_obs = ro.obs_next != nullptr ? ro.obs_next + (toff + env0) * R : nullptr;
-          float *g_rew = ro.rew != nullptr ? ro.rew + (toff + env0) * N : nullptr;
-          const bool tma_ok = valid == kRows && ((reinterpret_cast<uintptr_t>(g_obs) | reinterpret_cast<uintptr_t>(g_rew)) & 15) == 0;
-          if (tma_ok) fence_proxy_async_smem();
-          bar_sync_n(1 + g, 128);
-          if (g_obs != nullptr || g_rew != nullptr) {
-            if (tma_ok) {
-              if (row == 0) {
-                if (g_obs != nullptr) bulk_store(g_obs, stage_obs, kRows * R * 4);
-                if (g_rew != nullptr) bulk_store(g_rew, stage_rew, kRows * N * 4);
-                bulk_commit();
-              }
-            } else {
-              if (g_obs != nullptr)
-                for (int i = row; i < valid * R; i += 128) g_obs[i] = stage_obs[i];
-              if (g_rew != nullptr)
-                for (int i = row; i < valid * N; i += 128) g_rew[i] = stage_rew[i];
-            }
-          }
-          if (ro.act_u != nullptr)
-            for (int i = row; i < valid * N; i += 128) ro.act_u[(toff + env0) * N + i] = sm_act[i * 2];
-          if (ro.act_c != nullptr)
-            for (int i = row; i < valid * N; i += 128) ro.act_c[(toff + env0) * N + i] = sm_act[i * 2 + 1];
-          if (mine) {
-            if (do_reset) {  // experiments/run.py:59-60
-              const uint32_t ep = s.episode[b] + 1u;
-              s.episode[b] = ep;
-              e.reset(s.seed, (uint64_t)(s.gid0 + b), ep);
-              e.store_world(s, b);
-              if (SC == kReference) {
-#pragma unroll
-                for (int i = 0; i < 2; ++i)
-#pragma unroll
-                  for (int k = 0; k < 10; ++k) comm[i][k] = 0.0f;
-              }
-            }
-            e.store_agents(s, b);
-            if (SC == kReference) {
-#pragma unroll
-              for (int i = 0; i < 2; ++i)
-#pragma unroll
-                for (int k = 0; k < 10; ++k) s.comm[((int64_t)i * 10 + k) * s.B + b] = comm[i][k];
-            }
-          }
-          if (row == 0 && tma_ok && (g_obs != nullptr || g_rew != nullptr)) bulk_wait_read_all();
-        } else {
-          bar_sync_n(1 + g, 128);
-          const int rows = valid * N;
-          if (io.act_u != nullptr)
-            for (int i = row; i < rows; i += 128) io.act_u[env0 * N + i] = sm_act[i * 2];
-          if (io.act_c != nullptr)
-            for (int i = row; i < rows; i += 128) io.act_c[env0 * N + i] = sm_act[i * 2 + 1];
-          if (io.onehot != nullptr)
-            for (int i = row; i < rows * w.A; i += 128) {
-              const int rr = i / w.A, a = i - rr * w.A;
-              const bool hot = a < w.A0 ? (a == sm_act[rr * 2]) : (a - w.A0 == sm_act[rr * 2 + 1]);
-              io.onehot[env0 * N * w.A + i] = hot ? 1.0f : 0.0f;
-            }
-        }
-        TL(g, 29);
-        bar_sync_n(1 + g, 128);  // the group's staging (aliases x) and action buffer are free again
-        TL(g, 30);
-      }
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 8) tmem_free(tmem_base, 512);
-}
-
-#endif  // MPE_AB_KERNELS
-
-// ------------------------------------------------------------------------------------------------
-// k_tc2 (teams of <= 3 agents): the same two tiles per CTA, but BOTH warpgroups work on EVERY cell - warpgroup h
+// k_tc2: one persistent CTA per SM walks pairs of tiles (tile = 128 envs = 128 TMEM lanes).  Warps 0-7 are two
+// epilogue warpgroups, warp 8 / 9 issues the tcgen05.mma stream of tile 0 / 1, and for teams of > 3 agents warps
+// 10 / 11 are the operand warps described in the kernel.  BOTH warpgroups work on EVERY cell - warpgroup h
 // takes hidden units 16h..16h+15 of the cell (and 32 of the 64 dense1 columns), and the cells of the two tiles are
 // interleaved in one software pipeline:
 //      E1(A,k)  C(B,k-1)  E1(B,k)  C(A,k)  E1(A,k+1)  C(B,k) ...
@@ -748,7 +282,9 @@ __host__ __device__ inline size_t tc2_tile_bytes(int N, int Kx, int APAD) {
   // larger teams and the two-head simple_reference actor keep the dense2 shares in the global scratch instead
   return tc_x_bytes(N, Kx) + 16384 + (size_t)((kRows * N * 2 + 127) / 128 * 128) + (N <= 3 && APAD <= 8 ? (size_t)N * APAD * kRows * 4 : 0);
 }
-enum { B2_XR = 0, B2_XF = 4, B2_OBS = 8, B2_EXTRA = 9 };  // per tile: operand ring buffer q (< 4) ready / free again; fused large teams: next observations written
+// per tile: operand ring buffer q (< 4) ready / free again.  B2_OBS has no waiter; it stays (with its mbar_init)
+// because without it ptxas reschedules the large-team kernels, a change that wants its own measurement.
+enum { B2_XR = 0, B2_XF = 4, B2_OBS = 8, B2_EXTRA = 9 };
 __host__ __device__ inline size_t tc2_smem_bytes(uint32_t wbytes, int N, int Kx, int APAD) {
   return (size_t)wbytes + 2 * tc2_tile_bytes(N, Kx, APAD) + (1 + 2 * B_PER_WG + 2 * B2_EXTRA) * 8 + 64;
 }
@@ -765,15 +301,13 @@ __global__ void __launch_bounds__(tc2_threads(N), 1)
   // global scratch row (L2 resident) from which the owner warpgroup completes the logits and samples after the
   // pipeline.  Inside the pipeline the eight epilogue warps do nothing but the dense1 epilogue and the cell math.
   // (Measured alternatives: refilling from the epilogue warps - 400 B of spills and exposed load latency, slower than
-  // k_tc; a service warp that also samples one cell behind the pipeline - its ~11 k instructions per tile slow the
-  // two sub-partitions it shares and with them the whole barrier-coupled pipeline.)
+  // the earlier two-pipeline kernel; a service warp that also samples one cell behind the pipeline - its ~11 k
+  // instructions per tile slow the two sub-partitions it shares and with them the whole barrier-coupled pipeline.)
   constexpr bool kJit = N > 3;
   // two-head actors of small teams (simple_reference, A = 5 + 10): the exchange buffer does not fit into shared memory
   // any more, so the OTHER warpgroup's shares travel through the scratch rows as well (the own shares stay in registers)
   constexpr bool kXs = !kJit && APAD > 8;
-  // fused rollout of large teams: the env step runs after the sampling with G lanes per env (env_group.cuh), the
-  // observations of the next step go through an L2-resident work buffer that the operand warp streams back in
-  static_assert(!(kJit && FUSED) || (SC == kSpread && group_lanes(N) > 0), "fused large-team rollout: simple_spread, 6..12 agents");
+  static_assert(!(kJit && FUSED), "the fused rollout keeps every agent of an env in one thread: N <= 3");
   extern __shared__ __align__(128) unsigned char smem[];
 #ifdef MPE_TC_PHASES
   if (dbg && threadIdx.x == 0 && blockIdx.x < 148) {
@@ -809,7 +343,7 @@ __global__ void __launch_bounds__(tc2_threads(N), 1)
         mbar_init(&xbars[g * B2_EXTRA + B2_XR + q], 32);  // the service warp filled operand buffer q
         mbar_init(&xbars[g * B2_EXTRA + B2_XF + q], 1);   // the dense1 GEMM reading buffer q has completed
       }
-      mbar_init(&xbars[g * B2_EXTRA + B2_OBS], 128);      // the owner warpgroup wrote the tile's next observations
+      mbar_init(&xbars[g * B2_EXTRA + B2_OBS], 128);      // no waiter, see B2_OBS
     }
     mbar_fence_init();
     mbar_expect_tx(&bars[0], w.bytes);
@@ -843,66 +377,57 @@ __global__ void __launch_bounds__(tc2_threads(N), 1)
     const int X = warp - 10, lane = tid & 31;
     unsigned char *sm_x = tile_smem(X);
     uint64_t *xb2 = xbars + X * B2_EXTRA;
-    uint32_t ph_xf = 0, filled = 0, ph_obs = 0;  // bit q: phase parity of / first fill done for ring buffer q
-    const float *obs_src = FUSED ? ro.obs_work : io.obs;
-    const int64_t nbx = FUSED ? s.B : io.B;
-    const bool vec2 = (reinterpret_cast<uintptr_t>(obs_src) & 7) == 0 && (D & 1) == 0;
+    uint32_t ph_xf = 0, filled = 0;  // bit q: phase parity of / first fill done for ring buffer q
+    const bool vec2 = (reinterpret_cast<uintptr_t>(io.obs) & 7) == 0 && (D & 1) == 0;
     for (int64_t pair = blockIdx.x; pair < npairs; pair += gridDim.x) {
       const int64_t tile = pair * 2 + X, env0 = tile * kRows;
-      const int valid = tile < ntiles ? (int)((nbx - env0) < kRows ? (nbx - env0) : kRows) : 0;
+      const int valid = tile < ntiles ? (int)((io.B - env0) < kRows ? (io.B - env0) : kRows) : 0;
 #pragma unroll 1
-      for (int it = 0; it < T; ++it) {
-        if (FUSED && it > 0) {  // the env phase of step it - 1 has written this tile's observations (release / acquire)
-          mbar_wait(&xb2[B2_OBS], ph_obs);
-          ph_obs ^= 1;
-        }
+      for (int j = 0; j < 2 * N; ++j) {
+        if (!need_e1(j)) continue;
+        const int t = agent_of(j), q = d1_index(j) & (kRing - 1);
+        if ((filled >> q) & 1u) { mbar_wait(&xb2[B2_XF + q], (ph_xf >> q) & 1u); ph_xf ^= 1u << q; }
+        filled |= 1u << q;
+        unsigned char *xh = sm_x + (size_t)(q * 2) * (Kx / 8) * kChunkA, *xl = xh + (size_t)(Kx / 8) * kChunkA;
 #pragma unroll 1
-        for (int j = 0; j < 2 * N; ++j) {
-          if (!need_e1(j)) continue;
-          const int t = agent_of(j), q = d1_index(j) & (kRing - 1);
-          if ((filled >> q) & 1u) { mbar_wait(&xb2[B2_XF + q], (ph_xf >> q) & 1u); ph_xf ^= 1u << q; }
-          filled |= 1u << q;
-          unsigned char *xh = sm_x + (size_t)(q * 2) * (Kx / 8) * kChunkA, *xl = xh + (size_t)(Kx / 8) * kChunkA;
-#pragma unroll 1
-          for (int rp = 0; rp < 2; ++rp) {  // two rows per round: 2 x 32 values in registers, loads of both in flight
-            float xr[2][32];
+        for (int rp = 0; rp < 2; ++rp) {  // two rows per round: 2 x 32 values in registers, loads of both in flight
+          float xr[2][32];
 #pragma unroll
-            for (int u = 0; u < 2; ++u) {
-              const int r = lane + 32 * (2 * rp + u);
+          for (int u = 0; u < 2; ++u) {
+            const int r = lane + 32 * (2 * rp + u);
 #pragma unroll
-              for (int k = 0; k < 32; ++k) xr[u][k] = 0.0f;
-              if (r < valid) {
-                const float *src = obs_src + (env0 + r) * R + t * D;
-                if (vec2) {
+            for (int k = 0; k < 32; ++k) xr[u][k] = 0.0f;
+            if (r < valid) {
+              const float *src = io.obs + (env0 + r) * R + t * D;
+              if (vec2) {
 #pragma unroll
-                  for (int k = 0; k < 16; ++k)
-                    if (2 * k < D) {
-                      const float2 v = *reinterpret_cast<const float2 *>(src + 2 * k);
-                      xr[u][2 * k] = v.x; xr[u][2 * k + 1] = v.y;
-                    }
-                } else {
+                for (int k = 0; k < 16; ++k)
+                  if (2 * k < D) {
+                    const float2 v = *reinterpret_cast<const float2 *>(src + 2 * k);
+                    xr[u][2 * k] = v.x; xr[u][2 * k + 1] = v.y;
+                  }
+              } else {
 #pragma unroll
-                  for (int k = 0; k < 32; ++k)
-                    if (k < D) xr[u][k] = src[k];
-                }
-              }
-            }
-#pragma unroll
-            for (int u = 0; u < 2; ++u) {
-              const int r = lane + 32 * (2 * rp + u);
-#pragma unroll
-              for (int c = 0; c < 4; ++c) {
-                if (c * 8 < Kx) {
-                  const float v[8] = {xr[u][c * 8], xr[u][c * 8 + 1], xr[u][c * 8 + 2], xr[u][c * 8 + 3],
-                                      xr[u][c * 8 + 4], xr[u][c * 8 + 5], xr[u][c * 8 + 6], xr[u][c * 8 + 7]};
-                  store_chunk_split(xh + c * kChunkA, xl + c * kChunkA, r, v);
-                }
+                for (int k = 0; k < 32; ++k)
+                  if (k < D) xr[u][k] = src[k];
               }
             }
           }
-          fence_proxy_async_smem();
-          mbar_arrive(&xb2[B2_XR + q]);
+#pragma unroll
+          for (int u = 0; u < 2; ++u) {
+            const int r = lane + 32 * (2 * rp + u);
+#pragma unroll
+            for (int c = 0; c < 4; ++c) {
+              if (c * 8 < Kx) {
+                const float v[8] = {xr[u][c * 8], xr[u][c * 8 + 1], xr[u][c * 8 + 2], xr[u][c * 8 + 3],
+                                    xr[u][c * 8 + 4], xr[u][c * 8 + 5], xr[u][c * 8 + 6], xr[u][c * 8 + 7]};
+                store_chunk_split(xh + c * kChunkA, xl + c * kChunkA, r, v);
+              }
+            }
+          }
         }
+        fence_proxy_async_smem();
+        mbar_arrive(&xb2[B2_XR + q]);
       }
     }
   } else if (warp >= 8) {
@@ -1189,8 +714,6 @@ __global__ void __launch_bounds__(tc2_threads(N), 1)
           // groups of G agents: logits = bias + the four scratch shares (two warpgroups x two directions); the G * 2
           // Philox blocks and the G * 5 Gumbel transforms of a group run in lock-step
           constexpr int G = (N % 3 == 0) ? 3 : 2, NQ = APAD / 4;
-          const uint64_t jstep = FUSED ? ro.step0 + (uint64_t)it : io.step, jseed = FUSED ? s.seed : io.seed;
-          const int64_t jgid0 = FUSED ? s.gid0 : io.gid0;
 #pragma unroll 1
           for (int t0 = 0; t0 < N; t0 += G) {
             float lgt[G][APAD], gn[G][APAD];
@@ -1207,7 +730,7 @@ __global__ void __launch_bounds__(tc2_threads(N), 1)
 #pragma unroll
               for (int a = 0; a < APAD; ++a) gn[u][a] = 0.0f;
             }
-            if (!FUSED && io.gumbel != nullptr) {
+            if (io.gumbel != nullptr) {
               if (mine) {
 #pragma unroll
                 for (int u = 0; u < G; ++u)
@@ -1221,8 +744,8 @@ __global__ void __launch_bounds__(tc2_threads(N), 1)
               for (int u = 0; u < G; ++u)
 #pragma unroll
                 for (int jj = 0; jj < NQ; ++jj)
-                  c[u * NQ + jj] = philox_counter((uint64_t)(jgid0 + b), (uint32_t)jstep, kDomainGumbel, (t0 + u) * 8 + jj);
-              philox4x32_10_batch<G * NQ>(c, philox_key(jseed));
+                  c[u * NQ + jj] = philox_counter((uint64_t)(io.gid0 + b), (uint32_t)io.step, kDomainGumbel, (t0 + u) * 8 + jj);
+              philox4x32_10_batch<G * NQ>(c, philox_key(io.seed));
               if (w.A == 5) {
                 uint32_t r[G * 5];
                 float g[G * 5];
@@ -1272,7 +795,7 @@ __global__ void __launch_bounds__(tc2_threads(N), 1)
               }
               own_act[(row * N + t) * 2] = (uint8_t)bu;
               own_act[(row * N + t) * 2 + 1] = (uint8_t)bc;
-              if (!FUSED && mine && io.logits != nullptr) {
+              if (mine && io.logits != nullptr) {
 #pragma unroll
                 for (int a = 0; a < APAD; ++a)
                   if (a < w.A) io.logits[(b * N + t) * w.A + a] = lgt[u][a];
@@ -1380,67 +903,7 @@ __global__ void __launch_bounds__(tc2_threads(N), 1)
         }
 
         TL(half, 29);
-        if constexpr (FUSED && kJit) {
-          // ---- own tile, large teams: World.step + reward + outputs with G lanes per env (env_group.cuh) ----
-          // A warp of the owner warpgroup holds rows 32w .. 32w + 31 of the tile and walks them EPW envs at a time.
-          constexpr int G = group_lanes(N), A = N / G, EPW = 32 / G, PASSES = (32 + EPW - 1) / EPW;
-          const unsigned FULL = 0xffffffffu;
-          const int lane = row & 31, wq = row >> 5;
-          const int el = lane / G, q = lane - el * G, base_lane = el * G;
-          const bool lane_ok = lane < EPW * G;
-          const int64_t toff = (int64_t)it * s.B;
-          float *g_obs = ro.obs_next != nullptr ? ro.obs_next + toff * R : nullptr;
-          float *g_rew = ro.rew != nullptr ? ro.rew + toff * N : nullptr;
-          bar_sync_n(2 + own, 128);  // the tile's sampled actions are in own_act
-#pragma unroll 1
-          for (int p = 0; p < PASSES; ++p) {
-            const int e_in_warp = p * EPW + el, rloc = wq * 32 + e_in_warp;
-            const bool active = lane_ok && e_in_warp < 32 && rloc < valid;
-            const int64_t bb = env0 + rloc;
-            float px[A], py[A], vx[A], vy[A], lx[A], ly[A];
-            int au[A];
-            grp_load<float, N, G>(s, bb, q, active, px, py, vx, vy, lx, ly);
-#pragma unroll
-            for (int k = 0; k < A; ++k) au[k] = active ? (int)own_act[(rloc * N + q * A + k) * 2] : 0;
-            grp_physics<float, N, G>(s, au, q, base_lane, px, py, vx, vy);
-            float r[A], md;
-            int coll[A], occ;
-            grp_reward<float, N, G>(s, base_lane, px, py, lx, ly, r, coll, occ, md);
-            const float tot = grp_team_sum<float, N, G>(r, base_lane);
-            // episode bookkeeping lives with the env's first lane; its lanes learn whether the episode ends
-            int ts = 0;
-            uint32_t ep_old = 0;
-            float epr = 0.0f;
-            if (active && q == 0) { epr = s.ep_ret[bb] + tot; ts = s.tstep[bb] + 1; ep_old = s.episode[bb]; }
-            ts = __shfl_sync(FULL, ts, base_lane);
-            ep_old = __shfl_sync(FULL, ep_old, base_lane);
-            const bool do_reset = active && max_episode_len > 0 && ts >= max_episode_len;
-            GroupLanes<float, N, G> gl{0, lane, el, q, base_lane, bb - el, bb, lane_ok, active, false};
-            if (g_obs != nullptr || g_rew != nullptr)  // the step's recorded outputs (before a reset)
-              grp_emit<float, N, G>(gl, px, py, vx, vy, lx, ly, r, g_obs, g_rew, nullptr);
-            double ret = 0.0, n_ep = 0.0, n_steps = 0.0;
-            if (do_reset) {  // experiments/run.py:59-60
-              grp_reset_draw<float, N, G>(s, bb, ep_old + 1u, q, px, py, vx, vy, lx, ly);
-              if (q == 0) {
-                ret = (double)epr; n_ep = 1.0; n_steps = (double)ts;
-                s.episode[bb] = ep_old + 1u; s.tstep[bb] = 0; s.ep_ret[bb] = 0.0f;
-              }
-            } else if (active) {
-#pragma unroll
-              for (int k = 0; k < A; ++k) st4(s.pv + ((int64_t)(q * A + k) * s.B + bb) * 4, Vec4<float>{px[k], py[k], vx[k], vy[k]});
-              if (q == 0) { s.ep_ret[bb] = epr; s.tstep[bb] = ts; }
-            }
-            fold_stats(s.stats, ret, n_ep, n_steps);
-            // what the actor sees next: the observation of the (possibly fresh) state, via the L2-resident work buffer
-            if (it + 1 < T) grp_emit<float, N, G>(gl, px, py, vx, vy, lx, ly, nullptr, ro.obs_work, nullptr, nullptr);
-          }
-          if (ro.act_u != nullptr)
-            for (int i = row; i < valid * N; i += 128) ro.act_u[(toff + env0) * N + i] = own_act[i * 2];
-          if (it + 1 < T) {
-            __threadfence();
-            mbar_arrive(&xbars[own * B2_EXTRA + B2_OBS]);
-          }
-        } else if constexpr (FUSED) {
+        if constexpr (FUSED) {
           // ---- own tile: World.step + reward + outputs for env row `row` ----
           const int64_t toff = (int64_t)it * s.B;
           bool do_reset = false;
@@ -1598,6 +1061,7 @@ static cudaError_t launch_tc2_t(const EnvState<float> &s, const TcDev &w, const 
   static size_t have[64] = {0};
   const int dev = current_device();
   const size_t smem = tc2_smem_bytes(w.bytes, N, w.Kx, APAD);
+  if (smem > 227 * 1024) return cudaErrorInvalidValue;  // tc_*_supported rule these out
   cudaError_t e = ensure_smem(k_tc2<SC, N, FUSED, APAD>, smem, have, dev);
   if (e != cudaSuccess) return e;
   const int64_t ntiles = (nenvs + kRows - 1) / kRows;
@@ -1608,48 +1072,19 @@ static cudaError_t launch_tc2_t(const EnvState<float> &s, const TcDev &w, const 
   return cudaGetLastError();
 }
 
-template <int SC, int N, bool FUSED, int APAD>
-static cudaError_t launch_tc_t(const EnvState<float> &s, const TcDev &w, const ActorIO &io, const RolloutIO &ro,
-                               int max_episode_len, int64_t nenvs, cudaStream_t st) {
-#ifdef MPE_AB_KERNELS
-  static const bool v1 = getenv("MPE_TC_V1") != nullptr;  // A/B switch: the two-independent-pipelines kernel
-  if (v1) {
-    static size_t have[64] = {0};
-    const int dev = current_device();
-    const size_t smem = tc_smem_bytes(w.bytes, N, w.Kx);
-    cudaError_t e = ensure_smem(k_tc<SC, N, FUSED, APAD>, smem, have, dev);
-    if (e != cudaSuccess) return e;
-    const int64_t ntiles = (nenvs + kRows - 1) / kRows;
-    const int nsm = sm_count_tc(dev);
-    const int64_t pairs = (ntiles + 1) / 2;  // every CTA runs two tile pipelines
-    const int grid = (int)(pairs < nsm ? pairs : nsm);
-    k_tc<SC, N, FUSED, APAD><<<grid, kTcThreads, smem, st>>>(s, w, io, ro, max_episode_len, ntiles, tc_debug_flag());
-    return cudaGetLastError();
-  }
-#endif
-  if (tc2_smem_bytes(w.bytes, N, w.Kx, APAD) > 227 * 1024) return cudaErrorInvalidValue;  // tc_*_supported rule these out
-  return launch_tc2_t<SC, N, FUSED, APAD>(s, w, io, ro, max_episode_len, nenvs, st);
-}
-
 bool tc_actor_supported(const TcDev &w, int N) {
   // teams of > 3 agents keep one head of <= 8 entries (launch_actor_forward_tc); wider heads go to the FFMA kernel
   return tc_supported(w) && (N == 2 || N == 3 || ((N == 4 || N == 6 || N == 8 || N == 9 || N == 12) && w.A <= 8 && w.scratch != nullptr));
 }
 bool tc_rollout_supported(const TcDev &w, int N) {
-  // one kernel for all T steps: teams of <= 3 (every agent of an env in one thread's registers) and the large
-  // simple_spread teams with a tensor-core actor instantiation (env step with G lanes per env)
-  return tc_supported(w) && (N == 2 || N == 3 || ((N == 6 || N == 9 || N == 12) && w.A <= 8 && w.scratch != nullptr));
+  // one kernel for all T steps: every agent of an env in one thread's registers
+  return tc_supported(w) && (N == 2 || N == 3);
 }
 size_t tc_scratch_floats(int sm_count) {
-  // the largest of: k_tc's forward shares; k_tc2's per-cell shares for the instantiated large teams (N <= 12, one head
-  // of <= 8 entries) and for the two-head small teams (N <= 3, 16 entries)
-#ifdef MPE_AB_KERNELS
-  const size_t v1 = (size_t)sm_count * 2 * 12 * 16 * kRows;
-#else
-  const size_t v1 = 0;
-#endif
+  // the larger of k_tc2's per-cell shares for the instantiated large teams (N <= 12, one head of <= 8 entries) and
+  // for the two-head small teams (N <= 3, 16 entries)
   const size_t v2 = (size_t)sm_count * tc2_scratch_f2_per_cta(12, 8) * 2, v3 = (size_t)sm_count * tc2_scratch_f2_per_cta(3, 16) * 2;
-  return v1 > v2 ? (v1 > v3 ? v1 : v3) : (v2 > v3 ? v2 : v3);
+  return v2 > v3 ? v2 : v3;
 }
 
 cudaError_t launch_actor_forward_tc(const TcDev &w, const ActorIO &io, cudaStream_t st) {
@@ -1657,15 +1092,15 @@ cudaError_t launch_actor_forward_tc(const TcDev &w, const ActorIO &io, cudaStrea
   RolloutIO ro;
   const bool wide = w.A > 8;
   switch (io.N) {
-    case 2: return wide ? launch_tc_t<kSpread, 2, false, 16>(s, w, io, ro, 0, io.B, st)
-                        : launch_tc_t<kSpread, 2, false, 8>(s, w, io, ro, 0, io.B, st);
-    case 3: return wide ? launch_tc_t<kSpread, 3, false, 16>(s, w, io, ro, 0, io.B, st)
-                        : launch_tc_t<kSpread, 3, false, 8>(s, w, io, ro, 0, io.B, st);
-    case 4: return wide ? cudaErrorInvalidValue : launch_tc_t<kSpread, 4, false, 8>(s, w, io, ro, 0, io.B, st);
-    case 6: return wide ? cudaErrorInvalidValue : launch_tc_t<kSpread, 6, false, 8>(s, w, io, ro, 0, io.B, st);
-    case 8: return wide ? cudaErrorInvalidValue : launch_tc_t<kSpread, 8, false, 8>(s, w, io, ro, 0, io.B, st);
-    case 9: return wide ? cudaErrorInvalidValue : launch_tc_t<kSpread, 9, false, 8>(s, w, io, ro, 0, io.B, st);
-    case 12: return wide ? cudaErrorInvalidValue : launch_tc_t<kSpread, 12, false, 8>(s, w, io, ro, 0, io.B, st);
+    case 2: return wide ? launch_tc2_t<kSpread, 2, false, 16>(s, w, io, ro, 0, io.B, st)
+                        : launch_tc2_t<kSpread, 2, false, 8>(s, w, io, ro, 0, io.B, st);
+    case 3: return wide ? launch_tc2_t<kSpread, 3, false, 16>(s, w, io, ro, 0, io.B, st)
+                        : launch_tc2_t<kSpread, 3, false, 8>(s, w, io, ro, 0, io.B, st);
+    case 4: return wide ? cudaErrorInvalidValue : launch_tc2_t<kSpread, 4, false, 8>(s, w, io, ro, 0, io.B, st);
+    case 6: return wide ? cudaErrorInvalidValue : launch_tc2_t<kSpread, 6, false, 8>(s, w, io, ro, 0, io.B, st);
+    case 8: return wide ? cudaErrorInvalidValue : launch_tc2_t<kSpread, 8, false, 8>(s, w, io, ro, 0, io.B, st);
+    case 9: return wide ? cudaErrorInvalidValue : launch_tc2_t<kSpread, 9, false, 8>(s, w, io, ro, 0, io.B, st);
+    case 12: return wide ? cudaErrorInvalidValue : launch_tc2_t<kSpread, 12, false, 8>(s, w, io, ro, 0, io.B, st);
     default: return cudaErrorInvalidValue;
   }
 }
@@ -1678,14 +1113,10 @@ cudaError_t launch_rollout_tc(const EnvStateAny &a, const TcDev &w, const Rollou
   s.accel = (float)a.accel; s.track = 1;
   set_thresholds<float>(s, a.scenario);
   ActorIO io;
-  if (a.scenario == kReference) return launch_tc_t<kReference, 2, true, 16>(s, w, io, ro, a.max_episode_len, a.B, st);
-  if (a.scenario == kSpeaker) return launch_tc_t<kSpeaker, 2, true, 8>(s, w, io, ro, a.max_episode_len, a.B, st);
-  if (a.N == 2) return launch_tc_t<kSpread, 2, true, 8>(s, w, io, ro, a.max_episode_len, a.B, st);
-  if (a.N == 3) return launch_tc_t<kSpread, 3, true, 8>(s, w, io, ro, a.max_episode_len, a.B, st);
-  if (ro.obs_work == nullptr) return cudaErrorInvalidValue;  // large teams need the observation work buffer
-  if (a.N == 6) return launch_tc_t<kSpread, 6, true, 8>(s, w, io, ro, a.max_episode_len, a.B, st);
-  if (a.N == 9) return launch_tc_t<kSpread, 9, true, 8>(s, w, io, ro, a.max_episode_len, a.B, st);
-  if (a.N == 12) return launch_tc_t<kSpread, 12, true, 8>(s, w, io, ro, a.max_episode_len, a.B, st);
+  if (a.scenario == kReference) return launch_tc2_t<kReference, 2, true, 16>(s, w, io, ro, a.max_episode_len, a.B, st);
+  if (a.scenario == kSpeaker) return launch_tc2_t<kSpeaker, 2, true, 8>(s, w, io, ro, a.max_episode_len, a.B, st);
+  if (a.N == 2) return launch_tc2_t<kSpread, 2, true, 8>(s, w, io, ro, a.max_episode_len, a.B, st);
+  if (a.N == 3) return launch_tc2_t<kSpread, 3, true, 8>(s, w, io, ro, a.max_episode_len, a.B, st);
   return cudaErrorInvalidValue;
 }
 

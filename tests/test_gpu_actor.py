@@ -28,9 +28,9 @@ def _load(golden_dir, tag):
 
 
 def _impls(N, model=False, wide=False):
-    # tensor-core path: 2-3 agents (resident operands, fused env), 4/6/9/12 agents (just-in-time operands, single
+    # tensor-core path: 2-3 agents (resident operands, fused env), 4/6/8/9/12 agents (just-in-time operands, single
     # head of <= 8 entries); the dense3 model head is one small kernel on the relu(hcat) the tensor-core forward emits
-    if N in (2, 3) or (N in (4, 6, 9, 12) and not wide):
+    if N in (2, 3) or (N in (4, 6, 8, 9, 12) and not wide):
         return ['simt', 'tc']
     return ['simt']
 
@@ -135,10 +135,12 @@ def test_get_exploration_action_surface(golden_dir):
     assert a[0].shape == (64, 2, 5)
 
 
-@pytest.mark.parametrize('impl', ['simt', 'tc', 'tc_fused_large'])
+@pytest.mark.parametrize('impl', ['simt', 'tc'])
 @pytest.mark.parametrize('scenario,n,B', [('simple_spread', None, 10_000 + 13), ('simple_spread', 6, 2000),
                                           ('simple_spread', 9, 1000), ('simple_spread', 12, 500),
-                                          ('simple_reference', None, 3000), ('simple_speaker_listener', None, 3000)])
+                                          ('simple_reference', None, 3000), ('simple_speaker_listener', None, 3000),
+                                          ('simple_spread', 2, 3001), ('simple_spread', 4, 2000),
+                                          ('simple_spread', 8, 1000)])
 def test_fused_rollout_equals_stepwise_path(scenario, n, B, impl):
     """mpe_rollout (one kernel, T steps, in-kernel auto-reset) == actor_forward + mpe_step + mpe_reset
     called step by step with the same Philox keys: actions bit-exact, values bit-exact."""
@@ -150,7 +152,7 @@ def test_fused_rollout_equals_stepwise_path(scenario, n, B, impl):
     for k in sd:
         if 'dense2' in k:
             sd[k] = sd[k] * 3.0
-    if impl.replace('_fused_large', '') not in _impls(spec.N) or (impl == 'tc_fused_large' and spec.N <= 3):
+    if impl not in _impls(spec.N):
         pytest.skip('not covered by the tensor-core path')
     actor = m.FusedActor(sd, seed=seed, impl=impl)
     fused = m.make_env(scenario, n=n, num_envs=B, batched=True, seed=seed, max_episode_len=L)
@@ -178,11 +180,12 @@ def test_fused_rollout_equals_stepwise_path(scenario, n, B, impl):
 
 @pytest.mark.parametrize('scenario,n,B', [('simple_spread', None, 65_536), ('simple_spread', 6, 8_192),
                                           ('simple_spread', 12, 2_048), ('simple_reference', None, 16_384),
-                                          ('simple_speaker_listener', None, 16_384)])
+                                          ('simple_speaker_listener', None, 16_384), ('simple_spread', 4, 8_192),
+                                          ('simple_spread', 9, 4_096)])
 def test_fused_rollout_vs_float64_oracle_directly(scenario, n, B):
-    """The fused kernel's env phase against the float64 oracle, not via the stepwise kernels: a full 25-step episode
-    of ``rollout(record=True)`` at the bench size (65,536 envs) is replayed by oracle/mpe_vec.py from the same initial
-    state with the RECORDED actions.  fp32 tolerances of tests/test_gpu_env.py: positions 5e-5 worst case and 1e-5
+    """The rollout's env phase against the float64 oracle, not via the stepwise calls: a full 25-step episode of
+    ``rollout(record=True)`` (the fused kernel for teams of 2 / 3, actor + step kernels per step for larger teams) at
+    the bench size (65,536 envs) is replayed by oracle/mpe_vec.py from the same initial state with the RECORDED actions.  fp32 tolerances of tests/test_gpu_env.py: positions 5e-5 worst case and 1e-5
     at p99.99 per env, velocities 5e-4, rewards 2e-4 (a reward may be off by whole units only where a collision flag sits on its
     threshold: |dist - 0.30| within the band that env's position error explains)."""
     import multiagent_rl_b200 as m
@@ -191,7 +194,7 @@ def test_fused_rollout_vs_float64_oracle_directly(scenario, n, B):
     A = [5, 10] if scenario == 'simple_reference' else 5
     sd = actor_ref.init_state_dict(spec.obs_dim, A, 17)
     env = m.make_env(scenario, n=n, num_envs=B, batched=True, seed=seed, max_episode_len=T)
-    actor = m.FusedActor(sd, seed=seed, impl='tc_fused_large' if spec.N > 3 else 'auto')  # the single-kernel form everywhere
+    actor = m.FusedActor(sd, seed=seed, impl='auto')
     obs0 = env.reset()
     pos, vel, lm, goal = env.get_state()
     v = mpe_vec.VecEnv(spec, B)
@@ -342,13 +345,13 @@ def test_fused_rollout_full_size_properties(B):
     assert float((act_u[0] != act_u[1]).float().mean()) > 0.2
 
 
-@pytest.mark.parametrize('impl', ['auto', 'tc_fused_large'])
+@pytest.mark.parametrize('impl', ['auto', 'simt'])
 @pytest.mark.parametrize('scenario,n,A', [('simple_spread', None, 5), ('simple_reference', None, [5, 10]),
                                           ('simple_speaker_listener', None, 5), ('simple_spread', 6, 5)])
 def test_fused_rollout_equals_stepwise_path_tiny_batches(scenario, n, A, impl):
     """Batches of 1, 2 and 129 envs (one row of one tile, a tile pair whose second tile has one row): the rollout
-    (one kernel for small teams, actor + step kernels for large ones) equals the step-by-step calls bit for bit,
-    across auto-resets."""
+    (one kernel for small teams on the tensor cores, actor + step kernels for large teams and for the FFMA actor)
+    equals the step-by-step calls bit for bit, across auto-resets."""
     import multiagent_rl_b200 as m
     for B in (1, 2, 129):
         env = m.make_env(scenario, n=n, num_envs=B, batched=True, seed=3, max_episode_len=4)

@@ -22,7 +22,7 @@ CONFIGS = [('simple_spread', None, 65536), ('simple_spread', 6, 65536), ('simple
            ('fullobs_collect_treasure', None, 32768)]
 # SURVEY 8d configs 3-5: the same at 1,048,576 envs per GPU (no tail quantisation: thousands of tile pairs per SM)
 CONFIGS += [(s, n, 1 << 20 if s != 'fullobs_collect_treasure' else 1 << 19) for s, n, _ in CONFIGS]
-IMPL = sys.argv[1] if len(sys.argv) > 1 else 'auto'  # 'tc_fused_large': teams of 6 / 9 / 12 as one kernel per call
+IMPL = sys.argv[1] if len(sys.argv) > 1 else 'auto'  # a key of FusedActor.IMPLS: 'auto', 'simt' or 'tc'
 for scen, n, B in CONFIGS:
     env = m.make_env(scen, n=n, num_envs=B, batched=True, seed=1, max_episode_len=25)
     A = [5, 10] if scen == 'simple_reference' else 5

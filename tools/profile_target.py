@@ -51,10 +51,6 @@ if which in ('all', 'bign'):
         for _ in range(3):
             env.step(act)
         torch.cuda.synchronize()
-    # the opt-in single-kernel rollout of a 6-agent team (T = 2)
-    af = m.FusedActor(random_state_dict(16, 5, 1), device=dev, seed=1, impl='tc_fused_large')
-    env6.rollout(af, 2)
-    torch.cuda.synchronize()
 if which == 'critic':
     import numpy as np
     rng = np.random.RandomState(0)

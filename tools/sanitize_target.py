@@ -28,7 +28,7 @@ for scen, n, B, A in [('simple_spread', None, 333, 5), ('simple_spread', 6, 70, 
     env = m.make_env(scen, n=n, num_envs=B, batched=True, seed=3, max_episode_len=3)
     obs = env.reset()
     tc_ok = env.n in (2, 3, 4, 6, 8, 9, 12)
-    for impl in ['simt'] + (['tc'] if tc_ok else []) + (['tc_fused_large'] if env.n in (6, 9, 12) else []):
+    for impl in ['simt'] + (['tc'] if tc_ok else []):
         actor = m.FusedActor(random_state_dict(env.obs_dim, A, 1), impl=impl)
         actor.forward(obs, want_logits=True, want_onehot=True)
         env.rollout(actor, 5, record=True)
