@@ -258,6 +258,7 @@ typedef struct {
   int32_t device, reserved0;
 } ReplayConfig;
 
+/* MPE_EUNSUPPORTED when one transition record (record_bytes in csrc/replay_launch.h) exceeds 48 KB. */
 int replay_create(const ReplayConfig *cfg, MpeReplay **out);
 int replay_destroy(MpeReplay *replay);
 int replay_clear(MpeReplay *replay);               /* ReplayBuffer.clear  */
@@ -268,7 +269,7 @@ int64_t replay_next_idx(const MpeReplay *replay);  /* buffer._next_idx    */
 int replay_add(MpeReplay *replay, const float *obs, const int32_t *act_u, const int32_t *act_c, const float *rew,
                const float *obs_next, const float *done, int64_t B, void *stream);
 /* ReplayBuffer.make_index + sample_index: idx [batch] int64 device indices, or NULL to draw them uniformly with
- * replacement (Philox keyed by seed and the number of draws so far).  Caller-supplied indices follow Python list
+ * replacement (Philox domain 5, keyed by seed and the number of draws so far).  Caller-supplied indices follow Python list
  * indexing of ReplayBuffer._storage: negative values count from the end; values still outside [0, len) are clamped
  * into the ring (never read out of bounds) - validate host-side where an IndexError is wanted.  Outputs (each may be NULL): obs / obs_next
  * [batch][N][D], act_onehot [batch][N][act0+act1], rew [batch], done [batch], idx_out [batch]. */

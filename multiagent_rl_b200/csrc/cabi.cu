@@ -754,6 +754,10 @@ int replay_create(const ReplayConfig *cfg, MpeReplay **out) {
   if (cfg->capacity <= 0 || cfg->num_agents <= 0 || cfg->num_agents > 32 || cfg->obs_dim <= 0 || cfg->act0 <= 0 ||
       cfg->act0 > 127 || cfg->act1 < 0 || cfg->act1 > 127)
     return fail(MPE_EINVAL, "replay_create: bad configuration");
+  const int64_t rec = mpe::ReplayDev::record_bytes(cfg->num_agents, cfg->obs_dim);
+  if (rec > mpe::kReplayMaxRecordBytes)  // replay_add could never fill such a ring
+    return fail(MPE_EUNSUPPORTED, "replay_create: a transition record of " + std::to_string(rec) +
+                                      " bytes exceeds the " + std::to_string(mpe::kReplayMaxRecordBytes) + "-byte limit");
   DeviceGuard g(cfg->device);
   if (!g.ok) return fail(MPE_ECUDA, "replay_create: cannot select device");
   MpeReplay *r = new (std::nothrow) MpeReplay();
@@ -761,7 +765,7 @@ int replay_create(const ReplayConfig *cfg, MpeReplay **out) {
   r->device = cfg->device;
   mpe::ReplayDev &d = r->dev;
   d.capacity = cfg->capacity; d.N = cfg->num_agents; d.D = cfg->obs_dim; d.A0 = cfg->act0; d.A1 = cfg->act1;
-  d.rec_bytes = mpe::ReplayDev::record_bytes(d.N, d.D);
+  d.rec_bytes = rec;
   cudaError_t e = cudaMalloc(&d.ring, (size_t)d.capacity * (size_t)d.rec_bytes);
   if (e != cudaSuccess) {
     replay_destroy(r);

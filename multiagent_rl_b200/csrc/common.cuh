@@ -11,7 +11,7 @@ constexpr int kWarp = 32;
 // ----------------------------------------------------------------------------------------------
 // Philox4x32-10 (Salmon et al., SC'11).  counter = (gid_lo, gid_hi, t, domain<<16 | slot).
 // ----------------------------------------------------------------------------------------------
-enum : uint32_t { kDomainReset = 1, kDomainGoal = 2, kDomainGumbel = 3, kDomainRespawn = 4 };
+enum : uint32_t { kDomainReset = 1, kDomainGoal = 2, kDomainGumbel = 3, kDomainRespawn = 4, kDomainReplay = 5 };
 
 __device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {
 #pragma unroll

@@ -65,7 +65,8 @@ __global__ void __launch_bounds__(256) k_replay_add(ReplayDev r, int64_t slot0, 
 __global__ void __launch_bounds__(256) k_replay_make_index(int64_t size, int64_t batch, uint64_t seed, uint64_t counter,
                                                            int64_t *__restrict__ idx) {
   for (int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; j < batch; j += (int64_t)gridDim.x * blockDim.x) {
-    const uint4 rr = philox_raw(seed, (uint64_t)j, (uint32_t)counter, 4u, (uint32_t)(counter >> 32) & 0xFFFFu);
+    const uint4 rr = philox_raw(seed, (uint64_t)j, (uint32_t)counter, kDomainReplay,
+                                (uint32_t)(counter >> 32) & 0xFFFFu);
     idx[j] = (int64_t)__umul64hi(((uint64_t)rr.x << 32) | rr.y, (uint64_t)size);
   }
 }
@@ -183,7 +184,7 @@ cudaError_t launch_replay_add(const ReplayDev &r, int64_t head, int64_t B, const
   const int64_t R = (int64_t)r.N * r.D;
   int rpb = 128;  // records per block (32 KB of shared memory at 256 B per record)
   while (rpb > 1 && (int64_t)rpb * r.rec_bytes > 32 * 1024) rpb >>= 1;
-  if (r.rec_bytes > 48 * 1024) return cudaErrorInvalidValue;
+  if (r.rec_bytes > kReplayMaxRecordBytes) return cudaErrorInvalidValue;
   int64_t row0 = 0;
   while (row0 < B) {  // at most capacity rows per segment; a batch larger than the ring wraps more than once
     const int64_t slot0 = (head + row0) % r.capacity;

@@ -20,6 +20,9 @@ struct ReplayDev {
   __host__ __device__ static int64_t record_bytes(int N, int D) { return ((int64_t)N * D * 8 + 8 + 2 * N + 15) / 16 * 16; }
 };
 
+// add stages at least one whole record in shared memory; 48 KB is what a launch gets without opting in to more
+constexpr int64_t kReplayMaxRecordBytes = 48 * 1024;
+
 cudaError_t launch_replay_add(const ReplayDev &r, int64_t head, int64_t B, const float *obs, const int32_t *act_u,
                               const int32_t *act_c, const float *rew, const float *obs_next, const float *done,
                               cudaStream_t st);

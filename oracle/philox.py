@@ -26,6 +26,9 @@ Stream layout (must match multiagent_rl_b200/csrc/common.cuh):
   domain 2 = treasure types at reset, t = episode: slot 0 gives types 0..3, slot 1 types 4, 5 ; type = r >> 31.
   domain 4 = respawn, t = episode, slot = (step within the episode & 0xFFF) << 4 | treasure:
              r0, r1 -> position (scaled by 0.95), r2 >> 31 -> type, r3 -> the probability draw (prob = 1: passes).
+  replay ring (csrc/replay_kernels.cu, k_replay_make_index):
+  domain 5 = sampled indices, counter = (j, 0, draw_lo, 5 << 16 | draw_hi & 0xFFFF) for sample j of the ring's
+             draw-th make_index call: index = mulhi64((r0 << 32) | r1, len).
 """
 import numpy as np
 
@@ -39,6 +42,7 @@ DOMAIN_RESET = 1
 DOMAIN_GOAL = 2
 DOMAIN_GUMBEL = 3
 DOMAIN_RESPAWN = 4
+DOMAIN_REPLAY = 5
 
 
 def philox4x32_10(counter, key):
@@ -138,3 +142,22 @@ def treasure_respawn(seed, gid, episode, tstep, treasure):
     r = raw(seed, gid, episode, DOMAIN_RESPAWN, slot)
     pos = np.stack([bits_to_pos(r[0]), bits_to_pos(r[1])], axis=-1) * 0.95
     return pos, (r[2] >> np.uint32(31)).astype(np.int64)
+
+
+def mulhi64(x, y):
+    """High 64 bits of the 128-bit product of two uint64 arrays (CUDA's __umul64hi), from 32-bit limbs."""
+    x, y = np.asarray(x, dtype=np.uint64), np.asarray(y, dtype=np.uint64)
+    s32 = np.uint64(32)
+    xl, xh, yl, yh = x & MASK, x >> s32, y & MASK, y >> s32
+    ll, lh, hl, hh = xl * yl, xl * yh, xh * yl, xh * yh
+    mid = (ll >> s32) + (lh & MASK) + (hl & MASK)  # < 3 * 2^32: no overflow
+    return hh + (lh >> s32) + (hl >> s32) + (mid >> s32)
+
+
+def replay_index(seed, draw, batch, size):
+    """-> [batch] int64: the indices of the replay ring's draw-th make_index call on a ring holding `size`
+    transitions (uniform on [0, size) with replacement)."""
+    draw = int(draw)
+    r = raw(seed, np.arange(int(batch), dtype=np.uint64), draw & 0xFFFFFFFF, DOMAIN_REPLAY, (draw >> 32) & 0xFFFF)
+    x = (r[0].astype(np.uint64) << np.uint64(32)) | r[1].astype(np.uint64)
+    return mulhi64(x, np.uint64(size)).astype(np.int64)

@@ -68,6 +68,14 @@ def test_argument_errors_do_not_need_a_gpu():
     cc = _lib.CriticConfig(obs_dim=60, act_dim=10, out_dim=1)
     assert lib.critic_create(ctypes.byref(cc), ctypes.byref(h)) == _lib.MPE_EUNSUPPORTED
     assert lib.critic_forward(None, None, None, 1, 3, None, None, None) == _lib.MPE_EINVAL
+    # a ring whose records replay_add cannot stage (over 48 KB) is refused when it is created, not on every add:
+    # record_bytes(32, 191) = 48,976 is the largest accepted, record_bytes(32, 192) = 49,232
+    rc = _lib.ReplayConfig(capacity=16, num_agents=32, obs_dim=192, act0=5)
+    assert lib.replay_create(ctypes.byref(rc), ctypes.byref(h)) == _lib.MPE_EUNSUPPORTED
+    assert b'49232 bytes' in lib.mpe_last_error()
+    rc = _lib.ReplayConfig(capacity=16, num_agents=1, obs_dim=1 << 20, act0=5)
+    assert lib.replay_create(ctypes.byref(rc), ctypes.byref(h)) == _lib.MPE_EUNSUPPORTED
+    assert lib.replay_create(None, None) == _lib.MPE_EINVAL
 
 
 def test_no_cpu_fallback():

@@ -199,3 +199,79 @@ def test_critic_restatement_matches_reference_network(golden_dir, tag):
     assert ('r' in out) == ('r' in g.files)
     if 'r' in out:
         assert np.abs(out['r'] - g['r']).max() < 1e-6
+
+
+def _replay_batch(rng, B, N, D, act_dims, with_done):
+    obs, nxt = rng.randn(B, N, D).astype(np.float32), rng.randn(B, N, D).astype(np.float32)
+    rew = rng.randn(B, N).astype(np.float32)
+    au = rng.randint(0, act_dims[0], (B, N))
+    ac = rng.randint(0, act_dims[1], (B, N)) if len(act_dims) > 1 else None
+    done = (rng.rand(B) < 0.3).astype(np.float32) if with_done else None
+    return obs, au, ac, rew, nxt, done
+
+
+@pytest.mark.parametrize('cap,batches,act_dims', [
+    (50, [7, 13], [5]),                # partial fill
+    (50, [30, 31], [5]),               # the second add wraps
+    (50, [11, 50, 50], [5]),           # batches equal to the capacity, head != 0
+    (37, [20, 9, 37, 1, 25], [5, 10]),  # two heads, several wraps
+])
+def test_vectorised_replay_model_matches_reference_ring(cap, batches, act_dims):
+    """oracle/replay_ref.BatchedRing (index arithmetic) equals ReplayRing fed one transition at a time."""
+    from oracle import replay_ref
+    rng = np.random.RandomState(cap + len(batches))
+    N, D = 3, 4
+    model, ring = replay_ref.BatchedRing(cap, act_dims), replay_ref.ReplayRing(cap)
+    for i, B in enumerate(batches):
+        obs, au, ac, rew, nxt, done = _replay_batch(rng, B, N, D, act_dims, with_done=i % 2 == 0)
+        model.add(obs, au, rew, nxt, done, act_c=ac)
+        onehot = np.eye(act_dims[0], dtype=np.float32)[au]
+        if ac is not None:
+            onehot = np.concatenate([onehot, np.eye(act_dims[1], dtype=np.float32)[ac]], axis=-1)
+        replay_ref.add_batched_step(ring, obs, onehot, rew, nxt, done)
+        assert len(model) == len(ring) and model._next_idx == ring._next_idx
+        n = len(ring)
+        idx = np.concatenate([np.arange(n), rng.randint(-n, n, 40), [-n, n - 1, -1]])
+        got, want = model.sample_index(idx), ring.sample_index(idx)
+        for k in (0, 1, 3, 4):
+            assert np.array_equal(got[k], want[k].astype(np.float32)), k
+        # np.sum adds the agents in its own order; the model adds them the way the kernel does
+        assert np.allclose(got[2], want[2], rtol=1e-6, atol=1e-6)
+        with pytest.raises(IndexError):
+            model.sample_index([n])
+        with pytest.raises(IndexError):
+            model.sample_index([-n - 1])
+        # device indices: negatives wrap once, anything still out of range is clamped
+        assert np.array_equal(model.slots([n, 10 * n, -1, -n - 1, -10 * n], clamp=True), [n - 1, n - 1, n - 1, 0, 0])
+    for k, c in enumerate(model.collect()):
+        assert len(c) == len(ring), k
+
+
+def test_shared_reward_is_a_sequential_fp32_sum():
+    from oracle import replay_ref
+    rng = np.random.RandomState(3)
+    rew = (rng.randn(200, 12) * 10.0 ** rng.randint(-3, 4, (200, 12))).astype(np.float32)
+    want = []
+    for row in rew:
+        s = np.float32(0.0)
+        for v in row:
+            s = np.float32(s + v)
+        want.append(s)
+    assert np.array_equal(replay_ref.shared_reward(rew), np.array(want, dtype=np.float32))
+
+
+def test_replay_index_matches_big_integer_arithmetic():
+    """philox.replay_index against the formula in Python integers: mulhi64((r0 << 32) | r1, size)."""
+    for seed, draw, size in [(0, 0, 1), (1, 0, 3000), (7, 5, 1000003), (2 ** 40 + 9, 2 ** 33 + 17, 12345),
+                             (123, 1, 2 ** 20), (5, 2, 2 ** 63 - 25)]:
+        batch = 300
+        got = philox.replay_index(seed, draw, batch, size)
+        r = philox.raw(seed, np.arange(batch, dtype=np.uint64), draw & 0xFFFFFFFF, philox.DOMAIN_REPLAY,
+                       (draw >> 32) & 0xFFFF)
+        want = [((int(r[0][j]) << 32 | int(r[1][j])) * size) >> 64 for j in range(batch)]
+        assert got.tolist() == want
+        assert got.min() >= 0 and got.max() < size
+    # the replay stream is its own domain: no block is shared with the treasure env's respawn draws
+    r = philox.raw(1, np.arange(8, dtype=np.uint64), 0, philox.DOMAIN_REPLAY, 0)
+    q = philox.raw(1, np.arange(8, dtype=np.uint64), 0, philox.DOMAIN_RESPAWN, 0)
+    assert not np.array_equal(r[0], q[0])

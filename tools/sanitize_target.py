@@ -65,5 +65,19 @@ for scen, B, shards in (('simple_spread', 1001, 3), ('simple_reference', 130, 2)
         hr.step(lambda k, tr: float(tr.rew_np.sum()))
     hr.flush()
     hr.close()
+# replay ring: scalar (odd N*D) and vector tile paths, the element-parallel gather of records over 16 KB; adds across
+# the end of the ring, uniform samples, device indices out of range (clamped)
+for n, D, cap, B in ((3, 7, 331, 203), (3, 10, 331, 203), (31, 67, 53, 37)):
+    rng = np.random.RandomState(D)
+    rb = m.DeviceReplayBuffer(cap, n, D, 5, seed=1)
+    for _ in range(3):
+        rb.add(rng.randn(B, n, D).astype(np.float32), rng.randint(0, 5, (B, n)), rng.randn(B, n).astype(np.float32),
+               rng.randn(B, n, D).astype(np.float32), (rng.rand(B) < 0.5).astype(np.float32))
+    o = rb.sample(129)
+    assert bool(torch.isfinite(o[0]).all()) and bool(torch.isfinite(o[2]).all())
+    idx = rb.make_index(1001)
+    assert int(idx.min()) >= 0 and int(idx.max()) < len(rb)
+    rb.sample_index(torch.tensor([-1, 0, cap - 1, cap, -10 * cap, 7], device='cuda'))
+    rb.collect()
 torch.cuda.synchronize()
 print('sanitize target done')
