@@ -18,10 +18,10 @@
  *   - nothing synchronises the host except the *_host entry points, *_destroy
  *     and mpe_stats_read.
  *   - a handle is not thread-safe; handles on different devices are independent.
- *     One MpeActor may serve several MpeEnv handles on DIFFERENT streams at the same time through mpe_rollout,
- *     mpe_act_step_host_async (per-env scratch) and actor_forward_host_async (per-slot scratch); plain
- *     actor_forward calls on one actor must stay on one stream at a time (teams of > 3 agents and two-head actors
- *     park partial logits in the actor's own scratch buffer).
+ *     One MpeActor may serve several MpeEnv handles on DIFFERENT streams at the same time through mpe_rollout and
+ *     mpe_act_step_host_async (scratch per env handle); actor_forward and actor_forward_host calls on one actor must
+ *     stay on one stream at a time (teams of > 3 agents and two-head actors park partial logits in the actor's own
+ *     scratch buffer).
  *   - "real" is float for MPE_F32 handles and double for MPE_F64 (validation build).
  *   - tensor layouts are row-major with the env index outermost: obs[B][N][D],
  *     rew[B][N], done[B][N], act[B][N].
@@ -35,7 +35,7 @@
 extern "C" {
 #endif
 
-#define MPE_ABI_VERSION 3
+#define MPE_ABI_VERSION 4
 
 enum { MPE_OK = 0, MPE_EINVAL = -1, MPE_ECUDA = -2, MPE_EUNSUPPORTED = -3 };
 enum { MPE_SIMPLE_SPREAD = 0, MPE_SIMPLE_REFERENCE = 1, MPE_SIMPLE_SPEAKER_LISTENER = 2,
@@ -119,12 +119,8 @@ int mpe_step(MpeEnv *env, const int32_t *act_u, const int32_t *act_c, const void
  * obs/rew/done, then a stream synchronise.  This is what a list-of-numpy caller pays. */
 int mpe_step_host(MpeEnv *env, const int32_t *act_u_host, const int32_t *act_c_host, void *obs_host,
                   void *rew_host, uint8_t *done_host, void *stream);
-/* The same three stages ENQUEUED on `stream` without the final synchronise, so that a caller that splits its envs
- * over several handles and streams overlaps one shard's download with another shard's upload (PCIe is full
- * duplex; the blocking pair above alternates directions).  Host buffers must be pinned and stay untouched until
- * mpe_host_wait(stream).  mpe_reset_host_async: env.reset() (experiments/run.py:28,60) + D2H of the observations. */
-int mpe_step_host_async(MpeEnv *env, const int32_t *act_u_host, const int32_t *act_c_host, void *obs_host,
-                        void *rew_host, uint8_t *done_host, void *stream);
+/* env.reset() (experiments/run.py:28,60) + D2H of the observations, ENQUEUED on `stream` without a synchronise.
+ * obs_host must be pinned and stay untouched until mpe_host_wait(stream). */
 int mpe_reset_host_async(MpeEnv *env, void *obs_host, void *stream);
 /* cudaStreamSynchronize(stream): everything the *_host_async calls enqueued on it has landed in host memory. */
 int mpe_host_wait(void *stream);
@@ -133,10 +129,11 @@ int mpe_host_wait(void *stream);
  * as H2D obs_host [B][N][D] -> actor forward + sample (Philox keyed by the env's seed, global env ids and `step`) ->
  * env step on the sampled actions -> ONE D2H of the transition block {act_u, act_c, obs', rew, done} laid out as
  * mpe_host_block_layout says (offsets in bytes, each 256 B aligned; act_u / act_c int32 [B][N], obs' fp32 [B][N][D],
- * rew fp32 [B][N], done uint8 [B][N]; act_c has zero length - off_act_c == off_obs - for envs without a message head).  Compared with actor_forward_host_async + mpe_step_host_async the sampled
- * actions are not bounced through the host before the step reads them and the four downloads are one copy; every
- * step still uploads the observations and downloads everything the two calls return.  Enqueued on `stream`, no host
- * synchronisation (mpe_host_wait).  fp32 envs. */
+ * rew fp32 [B][N], done uint8 [B][N]; act_c has zero length - off_act_c == off_obs - for envs without a message head).
+ * Compared with the blocking actor_forward_host + mpe_step_host pair the sampled actions are not bounced through the
+ * host before the step reads them and the four downloads are one copy; every step still uploads the observations and
+ * downloads everything the two calls return.  Enqueued on `stream`, no host synchronisation (mpe_host_wait).
+ * fp32 envs. */
 typedef struct {
   uint64_t off_act_u, off_act_c, off_obs, off_rew, off_done, bytes;
 } MpeHostBlockLayout;
@@ -206,12 +203,6 @@ int actor_forward(MpeActor *actor, const float *obs, int64_t B, int32_t N, const
 int actor_forward_host(MpeActor *actor, const float *obs_host, int64_t B, int32_t N, uint64_t seed,
                        uint64_t step, int64_t env_id_offset, int32_t *act_u_host, int32_t *act_c_host,
                        float *onehot_host, void *stream);
-/* Same without the final synchronise (ddpg_gumbel_fix.py:93-100 split into enqueue + mpe_host_wait).  `slot`
- * (0..3) picks one of the handle's independent sets of device mirrors: calls in flight at the same time on
- * different streams must use different slots. */
-int actor_forward_host_async(MpeActor *actor, const float *obs_host, int64_t B, int32_t N, uint64_t seed,
-                             uint64_t step, int64_t env_id_offset, int32_t *act_u_host, int32_t *act_c_host,
-                             float *onehot_host, int32_t slot, void *stream);
 
 /* The loop body of experiments/run.py:36-65 fused: for t in [0, T): observe -> actor -> sample ->
  * step -> reward -> (episode_step == max_episode_len ? reset), state never leaving the SM between

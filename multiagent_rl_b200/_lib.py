@@ -7,7 +7,7 @@ import os
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get('MPE_B200_LIB', os.path.join(HERE, 'libmpe_b200.so'))  # override: A/B builds
-ABI_VERSION = 3
+ABI_VERSION = 4
 
 MPE_OK, MPE_EINVAL, MPE_ECUDA, MPE_EUNSUPPORTED = 0, -1, -2, -3
 SCENARIO_IDS = {'simple_spread': 0, 'simple_reference': 1, 'simple_speaker_listener': 2, 'fullobs_collect_treasure': 3}
@@ -76,7 +76,6 @@ SIGNATURES = {
     'mpe_observe': (C.c_int, [P, P, P]),
     'mpe_step': (C.c_int, [P, P, P, P, P, P, P, P, P, P]),
     'mpe_step_host': (C.c_int, [P, P, P, P, P, P, P]),
-    'mpe_step_host_async': (C.c_int, [P, P, P, P, P, P, P]),
     'mpe_reset_host_async': (C.c_int, [P, P, P]),
     'mpe_host_wait': (C.c_int, [P]),
     'mpe_host_block_layout': (C.c_int, [P, C.POINTER(MpeHostBlockLayout)]),
@@ -92,8 +91,6 @@ SIGNATURES = {
     'actor_set_impl': (C.c_int, [P, C.c_int32]),
     'actor_forward': (C.c_int, [P, P, C.c_int64, C.c_int32, P, C.c_uint64, C.c_uint64, C.c_int64, P, P, P, P, P, P]),
     'actor_forward_host': (C.c_int, [P, P, C.c_int64, C.c_int32, C.c_uint64, C.c_uint64, C.c_int64, P, P, P, P]),
-    'actor_forward_host_async': (C.c_int, [P, P, C.c_int64, C.c_int32, C.c_uint64, C.c_uint64, C.c_int64, P, P, P,
-                                           C.c_int32, P]),
     'mpe_rollout': (C.c_int, [P, P, C.c_int32, C.c_uint64, P, P, P, P, P]),
     'critic_create': (C.c_int, [C.POINTER(CriticConfig), C.POINTER(P)]),
     'critic_destroy': (C.c_int, [P]),

@@ -18,6 +18,7 @@
 
 #include "actor_launch.h"
 #include "common.cuh"
+#include "launch.h"
 
 namespace mpe {
 
@@ -498,9 +499,10 @@ __global__ void __launch_bounds__(256) k_dense3x2(ActorDev w, const float *__res
 
 cudaError_t launch_dense3(const ActorDev &w, const float *hcat, int64_t rows, float *next_state, cudaStream_t st) {
   if (rows <= 0) return cudaSuccess;
+  const int64_t nsm = sm_count(current_device());
   if (w.D <= 32) {  // every scenario of the reference (D <= 30): two rows per thread
     const int64_t blocks2 = (rows + kD3Rows2 - 1) / kD3Rows2;
-    const unsigned grid2 = (unsigned)(blocks2 < 148 * 5 ? blocks2 : 148 * 5);
+    const unsigned grid2 = (unsigned)(blocks2 < nsm * 5 ? blocks2 : nsm * 5);
     switch ((w.D + 3) / 4) {
 #define D3X(Q) case Q: k_dense3x2<Q><<<grid2, 256, 0, st>>>(w, hcat, rows, next_state); break;
       D3X(1) D3X(2) D3X(3) D3X(4) D3X(5) D3X(6) D3X(7) D3X(8)
@@ -510,7 +512,7 @@ cudaError_t launch_dense3(const ActorDev &w, const float *hcat, int64_t rows, fl
     return cudaGetLastError();
   }
   const int64_t blocks = (rows + kD3Rows - 1) / kD3Rows;
-  const unsigned grid = (unsigned)(blocks < 148 * 8 ? blocks : 148 * 8);
+  const unsigned grid = (unsigned)(blocks < nsm * 8 ? blocks : nsm * 8);
   switch ((w.D + 3) / 4) {
 #define D3(Q) case Q: k_dense3<Q><<<grid, 256, 0, st>>>(w, hcat, rows, next_state); break;
     D3(1) D3(2) D3(3) D3(4) D3(5) D3(6) D3(7) D3(8) D3(9) D3(10) D3(11) D3(12) D3(13) D3(14) D3(15) D3(16)
@@ -526,29 +528,15 @@ cudaError_t launch_dense3(const ActorDev &w, const float *hcat, int64_t rows, fl
 bool actor_supported(int N) { return N >= 1 && N <= 12; }  // any team size make_env(n=...) is asked for, up to 12
 bool rollout_supported(int scenario, int N) { return env_supported(scenario, N); }
 
-static int sm_count() {
-  static int cached[64] = {0};
-  int dev = 0;
-  cudaGetDevice(&dev);
-  if (dev < 0 || dev >= 64) dev = 0;
-  if (cached[dev] == 0) cudaDeviceGetAttribute(&cached[dev], cudaDevAttrMultiProcessorCount, dev);
-  return cached[dev] > 0 ? cached[dev] : 148;
-}
-
 template <int N, int TB, int PAD>
 static cudaError_t launch_actor_t(const ActorDev &w, const ActorIO &io, cudaStream_t st) {
+  const int dev = current_device();
   const size_t smem = ActorSmem<N, TB, PAD>::bytes(w.smem_floats, w.D);
-  static size_t have[64] = {0};  // sticky per (kernel, device): raise the opt-in only when a launch needs more
-  int dev = 0;
-  cudaGetDevice(&dev);
-  if (dev < 0 || dev >= 64) dev = 0;
-  if (have[dev] < smem) {
-    cudaError_t e = cudaFuncSetAttribute(k_actor_forward<N, TB, PAD>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    have[dev] = smem;
-  }
+  cudaError_t e = ensure_smem<k_actor_forward<N, TB, PAD>>(smem, dev);
+  if (e != cudaSuccess) return e;
   const int64_t ntiles = (io.B + TB - 1) / TB;
-  const int grid = (int)(ntiles < sm_count() ? ntiles : sm_count());
+  const int nsm = sm_count(dev);
+  const int grid = (int)(ntiles < nsm ? ntiles : nsm);
   k_actor_forward<N, TB, PAD><<<grid, kActorThreads, smem, st>>>(w, io, ntiles);
   return cudaGetLastError();
 }

@@ -12,6 +12,7 @@
 #include "actor_launch.h"
 #include "critic_launch.h"
 #include "env_launch.h"
+#include "launch.h"
 #include "replay_launch.h"
 
 namespace {
@@ -72,19 +73,16 @@ struct MpeEnv {
   int32_t host_tstep = 0;   // that common episode step
 };
 
-constexpr int kHostSlots = 4;  // independent sets of device mirrors: that many *_host_async calls may be in flight
-
 struct ActorMirror {
-  float *obs = nullptr, *onehot = nullptr;  // device mirrors for actor_forward_host[_async]
+  float *obs = nullptr, *onehot = nullptr;  // device mirrors for actor_forward_host
   int32_t *act_u = nullptr, *act_c = nullptr;
-  float *tc_scratch = nullptr;  // slots > 0: own dense2-share scratch (slot 0 uses the actor's), see MpeEnv::tc_scratch
   int64_t cap = 0;  // capacity in rows (B*N)
 };
 
 struct MpeActor {
   mpe::ActorDev dev;
   int device = 0;
-  ActorMirror mirror[kHostSlots];
+  ActorMirror mirror;
   float *hcat = nullptr;  // [rows][64] relu(BiLSTM output) between the tensor-core forward and the dense3 head
   int64_t hcat_rows = 0;
 };
@@ -105,9 +103,7 @@ struct MpeReplay {
 
 static cudaError_t ensure_tc_scratch(float **p, int device) {
   if (*p != nullptr) return cudaSuccess;
-  int nsm = 0;
-  cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, device);
-  return cudaMalloc(p, mpe::tc_scratch_floats(nsm > 0 ? nsm : 148) * sizeof(float));
+  return cudaMalloc(p, mpe::tc_scratch_floats(mpe::sm_count(device)) * sizeof(float));
 }
 
 // The actor's tensor-core weights for a launch on the caller's stream.  The kernels of large teams (N > 3) and of
@@ -307,12 +303,13 @@ int mpe_step(MpeEnv *env, const int32_t *act_u, const int32_t *act_c, const void
   return MPE_OK;
 }
 
-static int mpe_step_host_impl(MpeEnv *env, const int32_t *act_u_host, const int32_t *act_c_host, void *obs_host,
-                              void *rew_host, uint8_t *done_host, cudaStream_t st, bool sync, const char *who) {
-  if (env == nullptr || act_u_host == nullptr) return fail(MPE_EINVAL, std::string(who) + ": null env or act_u");
+int mpe_step_host(MpeEnv *env, const int32_t *act_u_host, const int32_t *act_c_host, void *obs_host, void *rew_host,
+                  uint8_t *done_host, void *stream) {
+  if (env == nullptr || act_u_host == nullptr) return fail(MPE_EINVAL, "mpe_step_host: null env or act_u");
   if (env->st.scenario == MPE_SIMPLE_REFERENCE && act_c_host == nullptr)
-    return fail(MPE_EINVAL, std::string(who) + ": simple_reference needs act_c");
+    return fail(MPE_EINVAL, "mpe_step_host: simple_reference needs act_c");
   DeviceGuard g(env->device);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
   const mpe::EnvStateAny &s = env->st;
   const size_t rows = (size_t)s.B * s.N, rs = real_size(s.precision);
   CK(ensure_host_mirrors(env));
@@ -326,20 +323,8 @@ static int mpe_step_host_impl(MpeEnv *env, const int32_t *act_u_host, const int3
   if (obs_host != nullptr) CK(cudaMemcpyAsync(obs_host, env->h_obs, rows * s.D * rs, cudaMemcpyDeviceToHost, st));
   if (rew_host != nullptr) CK(cudaMemcpyAsync(rew_host, env->h_rew, rows * rs, cudaMemcpyDeviceToHost, st));
   if (done_host != nullptr) CK(cudaMemcpyAsync(done_host, env->h_done, rows, cudaMemcpyDeviceToHost, st));
-  if (sync) CK(cudaStreamSynchronize(st));
+  CK(cudaStreamSynchronize(st));
   return MPE_OK;
-}
-
-int mpe_step_host(MpeEnv *env, const int32_t *act_u_host, const int32_t *act_c_host, void *obs_host, void *rew_host,
-                  uint8_t *done_host, void *stream) {
-  return mpe_step_host_impl(env, act_u_host, act_c_host, obs_host, rew_host, done_host, static_cast<cudaStream_t>(stream),
-                            true, "mpe_step_host");
-}
-
-int mpe_step_host_async(MpeEnv *env, const int32_t *act_u_host, const int32_t *act_c_host, void *obs_host,
-                        void *rew_host, uint8_t *done_host, void *stream) {
-  return mpe_step_host_impl(env, act_u_host, act_c_host, obs_host, rew_host, done_host, static_cast<cudaStream_t>(stream),
-                            false, "mpe_step_host_async");
 }
 
 int mpe_reset_host_async(MpeEnv *env, void *obs_host, void *stream) {
@@ -416,11 +401,10 @@ int actor_destroy(MpeActor *a) {
   void *ptrs[] = {a->dev.blob, a->dev.tc.blob, a->dev.tc.scratch, a->hcat};
   for (void *p : ptrs)
     if (p != nullptr) cudaFree(p);
-  for (ActorMirror &m : a->mirror) {
-    void *mp[] = {m.obs, m.onehot, m.act_u, m.act_c, m.tc_scratch};
-    for (void *p : mp)
-      if (p != nullptr) cudaFree(p);
-  }
+  const ActorMirror &m = a->mirror;
+  void *mp[] = {m.obs, m.onehot, m.act_u, m.act_c};
+  for (void *p : mp)
+    if (p != nullptr) cudaFree(p);
   delete a;
   return MPE_OK;
 }
@@ -494,27 +478,25 @@ int actor_forward(MpeActor *a, const float *obs, int64_t B, int32_t N, const flo
   return MPE_OK;
 }
 
-// H2D obs -> forward + sample -> D2H actions, all enqueued on `st`; `sync` waits for the stream at the end.
-static int actor_forward_host_impl(MpeActor *a, const float *obs_host, int64_t B, int32_t N, uint64_t seed, uint64_t step,
-                                   int64_t env_id_offset, int32_t *act_u_host, int32_t *act_c_host, float *onehot_host,
-                                   int32_t slot, cudaStream_t st, bool sync, const char *who) {
-  if (a == nullptr || obs_host == nullptr) return fail(MPE_EINVAL, std::string(who) + ": null argument");
-  if (slot < 0 || slot >= kHostSlots) return fail(MPE_EINVAL, std::string(who) + ": slot out of range");
+// H2D obs -> forward + sample -> D2H actions, all enqueued on `stream`, then a stream synchronise.
+int actor_forward_host(MpeActor *a, const float *obs_host, int64_t B, int32_t N, uint64_t seed, uint64_t step,
+                       int64_t env_id_offset, int32_t *act_u_host, int32_t *act_c_host, float *onehot_host,
+                       void *stream) {
+  if (a == nullptr || obs_host == nullptr) return fail(MPE_EINVAL, "actor_forward_host: null argument");
   if (B <= 0) return MPE_OK;
-  if (!mpe::actor_supported(N)) return fail(MPE_EUNSUPPORTED, std::string(who) + ": unsupported agent count");
+  if (!mpe::actor_supported(N)) return fail(MPE_EUNSUPPORTED, "actor_forward_host: unsupported agent count");
   DeviceGuard g(a->device);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
   const int64_t rows = B * N;
   const int A = a->dev.A0 + a->dev.A1;
-  ActorMirror &m = a->mirror[slot];
+  ActorMirror &m = a->mirror;
   if (rows > m.cap) {
-    // growing a mirror frees the old one: wait for whatever the stream still has in flight on it
+    // growing the mirror frees the old one: wait for whatever the stream still has in flight on it
     if (m.cap > 0) CK(cudaStreamSynchronize(st));
     void *old[] = {m.obs, m.onehot, m.act_u, m.act_c};
     for (void *p : old)
       if (p != nullptr) cudaFree(p);
-    float *keep = m.tc_scratch;
     m = ActorMirror();
-    m.tc_scratch = keep;
     CK(cudaMalloc(&m.obs, (size_t)rows * a->dev.D * sizeof(float)));
     CK(cudaMalloc(&m.onehot, (size_t)rows * A * sizeof(float)));
     CK(cudaMalloc(&m.act_u, (size_t)rows * sizeof(int32_t)));
@@ -526,28 +508,14 @@ static int actor_forward_host_impl(MpeActor *a, const float *obs_host, int64_t B
   io.obs = m.obs; io.act_u = m.act_u; io.act_c = a->dev.A1 > 0 ? m.act_c : nullptr;
   io.onehot = onehot_host != nullptr ? m.onehot : nullptr;
   io.B = B; io.N = N; io.seed = seed; io.step = step; io.gid0 = env_id_offset;
-  CK(launch_actor(a, io, slot > 0 ? &m.tc_scratch : nullptr, st));  // slots are in flight on different streams: own scratch each
+  CK(launch_actor(a, io, nullptr, st));
   if (act_u_host != nullptr) CK(cudaMemcpyAsync(act_u_host, m.act_u, (size_t)rows * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
   if (act_c_host != nullptr && a->dev.A1 > 0)
     CK(cudaMemcpyAsync(act_c_host, m.act_c, (size_t)rows * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
   if (onehot_host != nullptr)
     CK(cudaMemcpyAsync(onehot_host, m.onehot, (size_t)rows * A * sizeof(float), cudaMemcpyDeviceToHost, st));
-  if (sync) CK(cudaStreamSynchronize(st));
+  CK(cudaStreamSynchronize(st));
   return MPE_OK;
-}
-
-int actor_forward_host(MpeActor *a, const float *obs_host, int64_t B, int32_t N, uint64_t seed, uint64_t step,
-                       int64_t env_id_offset, int32_t *act_u_host, int32_t *act_c_host, float *onehot_host,
-                       void *stream) {
-  return actor_forward_host_impl(a, obs_host, B, N, seed, step, env_id_offset, act_u_host, act_c_host, onehot_host, 0,
-                                 static_cast<cudaStream_t>(stream), true, "actor_forward_host");
-}
-
-int actor_forward_host_async(MpeActor *a, const float *obs_host, int64_t B, int32_t N, uint64_t seed, uint64_t step,
-                             int64_t env_id_offset, int32_t *act_u_host, int32_t *act_c_host, float *onehot_host,
-                             int32_t slot, void *stream) {
-  return actor_forward_host_impl(a, obs_host, B, N, seed, step, env_id_offset, act_u_host, act_c_host, onehot_host, slot,
-                                 static_cast<cudaStream_t>(stream), false, "actor_forward_host_async");
 }
 
 static MpeHostBlockLayout block_layout(const mpe::EnvStateAny &s) {

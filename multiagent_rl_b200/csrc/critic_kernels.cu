@@ -15,6 +15,7 @@
 
 #include "common.cuh"
 #include "critic_launch.h"
+#include "launch.h"
 
 namespace mpe {
 
@@ -229,17 +230,11 @@ cudaError_t launch_critic_forward(const CriticDev &w, const float *obs, const fl
                                   float *r, cudaStream_t st) {
   if (B <= 0) return cudaSuccess;
   if (N < 1 || N > kCriticMaxAgents) return cudaErrorInvalidValue;
+  const int dev = current_device();
   const size_t smem = w.blob_floats * sizeof(float) + kCriticWarps * sizeof(CriticWarpSmem) + 64;
-  static size_t have[64] = {0};
-  int dev = 0, nsm = 148;
-  cudaGetDevice(&dev);
-  if (dev < 0 || dev >= 64) dev = 0;
-  if (have[dev] < smem) {
-    cudaError_t e = cudaFuncSetAttribute(k_critic_forward, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    have[dev] = smem;
-  }
-  cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, dev);
+  cudaError_t e = ensure_smem<k_critic_forward>(smem, dev);
+  if (e != cudaSuccess) return e;
+  const int nsm = sm_count(dev);
   const int64_t want = ((B + kCriticR - 1) / kCriticR + kCriticWarps - 1) / kCriticWarps;
   const int grid = (int)(want < nsm ? want : nsm);
   k_critic_forward<<<grid, kCriticThreads, smem, st>>>(w, obs, action, B, N, q, r);

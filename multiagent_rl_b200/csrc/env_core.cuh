@@ -17,6 +17,7 @@
 #include <type_traits>
 
 #include "common.cuh"
+#include "env_launch.h"
 
 namespace mpe {
 
@@ -152,6 +153,28 @@ inline void set_thresholds(EnvState<T> &s, int scenario) {
     s.tr_cut[1] = sqrt_gt_threshold<T>((T)cd + Underflow<T>::v);
     s.tr_cut[2] = sqrt_gt_threshold<T>((T)dd + Underflow<T>::v);
   }
+}
+
+// host side: the kernels' EnvState<T> view of a shard's type-erased EnvStateAny (env_launch.h)
+template <typename T>
+inline EnvState<T> typed(const EnvStateAny &a) {
+  EnvState<T> s;
+  s.pv = static_cast<T *>(a.pv);
+  s.lm = static_cast<T *>(a.lm);
+  s.goal = a.goal;
+  s.episode = a.episode;
+  s.tstep = a.tstep;
+  s.ep_ret = static_cast<T *>(a.ep_ret);
+  s.comm = static_cast<T *>(a.comm);
+  s.stats = a.stats;
+  s.B = a.B;
+  s.gid0 = a.gid0;
+  s.seed = a.seed;
+  s.max_speed = (T)a.max_speed;
+  s.accel = (T)a.accel;
+  s.track = a.track;
+  set_thresholds<T>(s, a.scenario);
+  return s;
 }
 
 // get_collision_force for one close pair: (gx, gy) = contact_force * delta / dist * penetration.

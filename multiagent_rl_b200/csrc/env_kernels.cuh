@@ -9,6 +9,7 @@
 #pragma once
 #include "env_core.cuh"
 #include "env_launch.h"
+#include "launch.h"
 
 namespace mpe {
 constexpr int kStepThreads = 128;
@@ -307,27 +308,6 @@ __global__ void k_get_state(EnvState<T> s, int N, int L, T *pos, T *vel, T *lm, 
 // ---------------------------------------------------------------------------------------------
 // host-side dispatch over (scenario, N)
 // ---------------------------------------------------------------------------------------------
-template <typename T>
-inline EnvState<T> typed(const EnvStateAny &a) {
-  EnvState<T> s;
-  s.pv = static_cast<T *>(a.pv);
-  s.lm = static_cast<T *>(a.lm);
-  s.goal = a.goal;
-  s.episode = a.episode;
-  s.tstep = a.tstep;
-  s.ep_ret = static_cast<T *>(a.ep_ret);
-  s.comm = static_cast<T *>(a.comm);
-  s.stats = a.stats;
-  s.B = a.B;
-  s.gid0 = a.gid0;
-  s.seed = a.seed;
-  s.max_speed = (T)a.max_speed;
-  s.accel = (T)a.accel;
-  s.track = a.track;
-  set_thresholds<T>(s, a.scenario);
-  return s;
-}
-
 #define MPE_DISPATCH(a, CALL)                                                       \
   do {                                                                              \
     if ((a).scenario == kSpread) {                                                  \
@@ -363,26 +343,11 @@ inline EnvState<T> typed(const EnvStateAny &a) {
     }                            \
   } while (0)
 
-// kernels that stage more than the default 48 KB opt in once per (kernel, device): the attribute is sticky.  The
-// kernel is a template ARGUMENT so that every kernel gets its own "done" flags.
-template <auto Kernel>
-inline cudaError_t set_smem_once(int bytes) {
-  if (bytes <= 48 * 1024) return cudaSuccess;
-  static bool done[64] = {false};
-  int dev = 0;
-  cudaGetDevice(&dev);
-  if (dev < 0 || dev >= 64) return cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
-  if (done[dev]) return cudaSuccess;
-  cudaError_t e = cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
-  if (e == cudaSuccess) done[dev] = true;
-  return e;
-}
-
 #define MPE_GRP_RESET(NN, GG, DO_RESET)                                                                            \
   {                                                                                                                \
     using GL = GroupLayout<T, NN, GG>;                                                                             \
     constexpr int sm = GL::kBlockBytes;                                                                            \
-    cudaError_t err = set_smem_once<k_reset_grp<T, NN, GG>>(sm);                                                     \
+    cudaError_t err = ensure_smem<k_reset_grp<T, NN, GG>>(sm);                                                       \
     if (err != cudaSuccess) return err;                                                                            \
     const int64_t per_block = (int64_t)GL::EPW * (kStepThreads / 32);                                              \
     k_reset_grp<T, NN, GG><<<(unsigned)((a.B + per_block - 1) / per_block), kStepThreads, sm, st>>>(               \
@@ -395,7 +360,7 @@ template <typename T, int MODE>
 cudaError_t launch_treasure_t(const EnvStateAny &a, const int32_t *act_u, const uint8_t *mask, int auto_len, void *obs,
                               void *rew, uint8_t *done, int32_t *info_i, cudaStream_t st) {
   constexpr int sm = TrLayout<T>::kBlockBytes;
-  cudaError_t err = set_smem_once<k_treasure<T, MODE>>(sm);
+  cudaError_t err = ensure_smem<k_treasure<T, MODE>>(sm);
   if (err != cudaSuccess) return err;
   const int64_t per_block = TrLayout<T>::kEnvsPerBlock;  // 8 lanes per env
   const unsigned grid = (unsigned)((a.B + per_block - 1) / per_block);
@@ -417,7 +382,7 @@ cudaError_t launch_reset_t(const EnvStateAny &a, const uint8_t *mask, void *obs,
 #define CALL(SC, NN)                                                                          \
   {                                                                                           \
     constexpr int sm = StageLayout<T, SC, NN>::kBlockBytes;                                   \
-    cudaError_t err = set_smem_once<k_reset<T, SC, NN>>(sm);                                    \
+    cudaError_t err = ensure_smem<k_reset<T, SC, NN>>(sm);                                      \
     if (err != cudaSuccess) return err;                                                       \
     k_reset<T, SC, NN><<<grid, kStepThreads, sm, st>>>(typed<T>(a), mask, static_cast<T *>(obs), auto_len); \
   }
@@ -441,7 +406,7 @@ cudaError_t launch_observe_t(const EnvStateAny &a, void *obs, cudaStream_t st) {
 #define CALL(SC, NN)                                                                    \
   {                                                                                     \
     constexpr int sm = StageLayout<T, SC, NN>::kBlockBytes;                             \
-    cudaError_t err = set_smem_once<k_observe<T, SC, NN>>(sm);                            \
+    cudaError_t err = ensure_smem<k_observe<T, SC, NN>>(sm);                              \
     if (err != cudaSuccess) return err;                                                 \
     k_observe<T, SC, NN><<<grid, kStepThreads, sm, st>>>(typed<T>(a), static_cast<T *>(obs)); \
   }
@@ -460,7 +425,7 @@ cudaError_t launch_step_t(const EnvStateAny &a, const int32_t *act_u, const int3
   {                                                                                                                \
     using GL = GroupLayout<T, NN, GG>;                                                                             \
     constexpr int sm = GL::kBlockBytes;                                                                            \
-    cudaError_t err = set_smem_once<k_step_grp<T, NN, GG>>(sm);                                                      \
+    cudaError_t err = ensure_smem<k_step_grp<T, NN, GG>>(sm);                                                        \
     if (err != cudaSuccess) return err;                                                                            \
     const int64_t per_block = (int64_t)GL::EPW * (kStepThreads / 32);                                              \
     k_step_grp<T, NN, GG><<<(unsigned)((a.B + per_block - 1) / per_block), kStepThreads, sm, st>>>(                \
@@ -474,7 +439,7 @@ cudaError_t launch_step_t(const EnvStateAny &a, const int32_t *act_u, const int3
 #define CALL(SC, NN)                                                                                         \
   {                                                                                                          \
     constexpr int sm = StageLayout<T, SC, NN>::kBlockBytes;                                                  \
-    cudaError_t err = set_smem_once<k_step<T, SC, NN>>(sm);                                                    \
+    cudaError_t err = ensure_smem<k_step<T, SC, NN>>(sm);                                                      \
     if (err != cudaSuccess) return err;                                                                      \
     k_step<T, SC, NN><<<grid, kStepThreads, sm, st>>>(typed<T>(a), act_u, act_c, static_cast<const T *>(comm_vec), \
                                                       static_cast<T *>(obs), static_cast<T *>(rew), done, info_i, \

@@ -6,6 +6,7 @@
 #include "replay_launch.h"
 
 #include "common.cuh"
+#include "launch.h"
 
 namespace mpe {
 
@@ -173,8 +174,8 @@ __global__ void __launch_bounds__(256) k_replay_gather_tile(ReplayDev r, int64_t
 }
 
 static unsigned grid_for(int64_t total) {
-  const int64_t blocks = (total + 255) / 256;
-  return (unsigned)(blocks < 148 * 32 ? (blocks > 0 ? blocks : 1) : 148 * 32);
+  const int64_t blocks = (total + 255) / 256, cap = (int64_t)sm_count(current_device()) * 32;
+  return (unsigned)(blocks < cap ? (blocks > 0 ? blocks : 1) : cap);
 }
 
 cudaError_t launch_replay_add(const ReplayDev &r, int64_t head, int64_t B, const float *obs, const int32_t *act_u,
@@ -185,12 +186,13 @@ cudaError_t launch_replay_add(const ReplayDev &r, int64_t head, int64_t B, const
   int rpb = 128;  // records per block (32 KB of shared memory at 256 B per record)
   while (rpb > 1 && (int64_t)rpb * r.rec_bytes > 32 * 1024) rpb >>= 1;
   if (r.rec_bytes > kReplayMaxRecordBytes) return cudaErrorInvalidValue;
+  const int64_t cap = (int64_t)sm_count(current_device()) * 16;
   int64_t row0 = 0;
   while (row0 < B) {  // at most capacity rows per segment; a batch larger than the ring wraps more than once
     const int64_t slot0 = (head + row0) % r.capacity;
     const int64_t rows = (B - row0) < (r.capacity - slot0) ? (B - row0) : (r.capacity - slot0);
     const int64_t blocks = (rows + rpb - 1) / rpb;
-    const unsigned grid = (unsigned)(blocks < 148 * 16 ? blocks : 148 * 16);
+    const unsigned grid = (unsigned)(blocks < cap ? blocks : cap);
     const size_t sm = (size_t)rpb * r.rec_bytes;
     const uintptr_t al = reinterpret_cast<uintptr_t>(obs + row0 * R) | reinterpret_cast<uintptr_t>(obs_next + row0 * R);
     if (R % 2 == 0 && (al & 7) == 0)
@@ -221,8 +223,8 @@ cudaError_t launch_replay_gather(const ReplayDev &r, int64_t size, int64_t batch
   int rpb = 64;  // records per block (16 KB of shared memory at 256 B per record; measured 128: 0.67, 64: 0.75, 32: 0.64 of HBM)
   while (rpb > 1 && (int64_t)rpb * r.rec_bytes > 16 * 1024) rpb >>= 1;
   if (r.rec_bytes <= 16 * 1024) {
-    const int64_t blocks = (batch + rpb - 1) / rpb;
-    const unsigned grid = (unsigned)(blocks < 148 * 16 ? blocks : 148 * 16);
+    const int64_t blocks = (batch + rpb - 1) / rpb, cap = (int64_t)sm_count(current_device()) * 16;
+    const unsigned grid = (unsigned)(blocks < cap ? blocks : cap);
     const size_t sm = (size_t)rpb * r.rec_bytes;
     if (v2)
       k_replay_gather_tile<2><<<grid, 256, sm, st>>>(r, size, batch, rpb, idx, obs, act_onehot, rew, obs_next, done);

@@ -18,6 +18,7 @@
 
 #include "actor_launch.h"
 #include "env_core.cuh"
+#include "launch.h"
 #include "tc_common.cuh"
 
 namespace mpe {
@@ -1026,46 +1027,23 @@ __global__ void __launch_bounds__(tc2_threads(N), 1)
 // ------------------------------------------------------------------------------------------------
 // launch
 // ------------------------------------------------------------------------------------------------
-// Per-launch host work is kept to the launch itself (the fused step is a ~60 us kernel): the device ordinal is one
-// cheap runtime call, everything derived from it is cached per device.
-static int current_device() {
-  int dev = 0;
-  cudaGetDevice(&dev);
-  return (dev >= 0 && dev < 64) ? dev : 0;
-}
-static int sm_count_tc(int dev) {
-  static int cached[64] = {0};
-  if (cached[dev] == 0) {
-    int n = 0;
-    cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev);
-    cached[dev] = n > 0 ? n : 148;
-  }
-  return cached[dev];
-}
-// cudaFuncAttributeMaxDynamicSharedMemorySize is sticky per function and device: raise it only when a launch needs more
-template <typename K>
-static cudaError_t ensure_smem(K kernel, size_t bytes, size_t (&have)[64], int dev) {
-  if (have[dev] >= bytes) return cudaSuccess;
-  cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
-  if (e == cudaSuccess) have[dev] = bytes;
-  return e;
-}
 static int tc_debug_flag() {
   static const int dbg = getenv("MPE_TC_TIMELINE") != nullptr ? 1 : 0;
   return dbg;
 }
 
+// Per-launch host work is kept to the launch itself (the fused step is a ~60 us kernel): one cudaGetDevice, everything
+// derived from the device is cached (launch.h).
 template <int SC, int N, bool FUSED, int APAD>
 static cudaError_t launch_tc2_t(const EnvState<float> &s, const TcDev &w, const ActorIO &io, const RolloutIO &ro,
                                 int max_episode_len, int64_t nenvs, cudaStream_t st) {
-  static size_t have[64] = {0};
   const int dev = current_device();
   const size_t smem = tc2_smem_bytes(w.bytes, N, w.Kx, APAD);
   if (smem > 227 * 1024) return cudaErrorInvalidValue;  // tc_*_supported rule these out
-  cudaError_t e = ensure_smem(k_tc2<SC, N, FUSED, APAD>, smem, have, dev);
+  cudaError_t e = ensure_smem<k_tc2<SC, N, FUSED, APAD>>(smem, dev);
   if (e != cudaSuccess) return e;
   const int64_t ntiles = (nenvs + kRows - 1) / kRows;
-  const int nsm = sm_count_tc(dev);
+  const int nsm = sm_count(dev);
   const int64_t pairs = (ntiles + 1) / 2;
   const int grid = (int)(pairs < nsm ? pairs : nsm);
   k_tc2<SC, N, FUSED, APAD><<<grid, tc2_threads(N), smem, st>>>(s, w, io, ro, max_episode_len, ntiles, tc_debug_flag());
@@ -1106,12 +1084,8 @@ cudaError_t launch_actor_forward_tc(const TcDev &w, const ActorIO &io, cudaStrea
 }
 
 cudaError_t launch_rollout_tc(const EnvStateAny &a, const TcDev &w, const RolloutIO &ro, cudaStream_t st) {
-  EnvState<float> s;
-  s.pv = static_cast<float *>(a.pv); s.lm = static_cast<float *>(a.lm); s.goal = a.goal; s.episode = a.episode;
-  s.tstep = a.tstep; s.ep_ret = static_cast<float *>(a.ep_ret); s.comm = static_cast<float *>(a.comm);
-  s.stats = a.stats; s.B = a.B; s.gid0 = a.gid0; s.seed = a.seed; s.max_speed = (float)a.max_speed;
-  s.accel = (float)a.accel; s.track = 1;
-  set_thresholds<float>(s, a.scenario);
+  EnvState<float> s = typed<float>(a);
+  s.track = 1;  // the fused rollout always keeps the episode counters (mpe_track_returns)
   ActorIO io;
   if (a.scenario == kReference) return launch_tc2_t<kReference, 2, true, 16>(s, w, io, ro, a.max_episode_len, a.B, st);
   if (a.scenario == kSpeaker) return launch_tc2_t<kSpeaker, 2, true, 8>(s, w, io, ro, a.max_episode_len, a.B, st);

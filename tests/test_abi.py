@@ -42,7 +42,7 @@ def test_struct_layouts_match_header():
     assert ctypes.sizeof(_lib.MpeHostBlockLayout) == 48
 
 
-def test_argument_errors_do_not_need_a_gpu():
+def test_bad_arguments_are_rejected_before_cuda():
     from multiagent_rl_b200 import _lib
     lib = _lib.load()
     assert lib.mpe_create(None, None) == _lib.MPE_EINVAL
@@ -61,9 +61,9 @@ def test_argument_errors_do_not_need_a_gpu():
     assert lib.mpe_act_step_host_async(None, None, None, 0, None, None) == _lib.MPE_EINVAL
     assert lib.mpe_host_block_layout(None, None) == _lib.MPE_EINVAL
     assert lib.mpe_host_alloc(None, 0) == _lib.MPE_EINVAL and lib.mpe_host_free(None) == _lib.MPE_OK
-    assert lib.mpe_step_host_async(None, None, None, None, None, None, None) == _lib.MPE_EINVAL
+    assert lib.mpe_step_host(None, None, None, None, None, None, None) == _lib.MPE_EINVAL
     assert lib.mpe_reset_host_async(None, None, None) == _lib.MPE_EINVAL
-    assert lib.actor_forward_host_async(None, None, 1, 3, 0, 0, 0, None, None, None, 0, None) == _lib.MPE_EINVAL
+    assert lib.actor_forward_host(None, None, 1, 3, 0, 0, 0, None, None, None, None) == _lib.MPE_EINVAL
     assert lib.critic_create(None, None) == _lib.MPE_EINVAL and lib.critic_destroy(None) == _lib.MPE_OK
     cc = _lib.CriticConfig(obs_dim=60, act_dim=10, out_dim=1)
     assert lib.critic_create(ctypes.byref(cc), ctypes.byref(h)) == _lib.MPE_EUNSUPPORTED

@@ -374,9 +374,9 @@ def test_fused_rollout_equals_stepwise_path_tiny_batches(scenario, n, A, impl):
                                                ('fullobs_collect_treasure', 2, 515),
                                                ('fullobs_collect_treasure', 4, 20_011)])
 def test_host_rollout_shards_match_the_blocking_calls(scenario, shards, B):
-    """HostRollout (non-blocking actor_forward_host_async + mpe_step_host_async per shard and stream) gives, for every
-    shard count, exactly the transitions of the device-tensor calls on one env handle: same Philox keys (global env
-    id, step), same kernels.  Both ends of each transition are on the host: obs_prev -> (act, rew) -> obs."""
+    """HostRollout (non-blocking mpe_act_step_host_async per shard and stream) gives, for every shard count, exactly
+    the transitions of the device-tensor calls on one env handle: same Philox keys (global env id, step), same
+    kernels.  Both ends of each transition are on the host: obs_prev -> (act, rew) -> obs."""
     import multiagent_rl_b200 as m
     L, seed = 4, 31
     n = None
@@ -491,46 +491,3 @@ def test_host_block_layout_and_argument_checks():
         m.HostRollout('simple_spread', 8, actor, n=6)
     blk.free()
 
-
-def test_async_host_calls_with_two_slots_on_two_streams():
-    """actor_forward_host_async / mpe_step_host_async / mpe_host_wait used directly: two halves of a batch in flight on
-    two streams (two mirror slots of one actor handle, two env handles) give the blocking calls' results."""
-    import ctypes as C
-    import multiagent_rl_b200 as m
-    from multiagent_rl_b200 import _lib
-    lib = _lib.load()
-    B, seed = 2000, 13
-    actor = m.FusedActor(actor_ref.init_state_dict(10, 5, 1), seed=seed)
-    whole = m.make_env('simple_spread', num_envs=B, batched=True, seed=seed)
-    obs = whole.reset()
-    want = actor.forward(obs, step=5, want_onehot=True)
-    o2, r2, d2, _ = whole.step(want['act_u'])
-    blk = _lib.HostBlock(8 << 20)
-    halves = []
-    for k in range(2):
-        n = B // 2
-        env = m.make_env('simple_spread', num_envs=n, batched=True, seed=seed, env_id_offset=k * n)
-        env.reset()
-        st = torch.cuda.Stream()
-        h = {'env': env, 'st': st, 'sp': C.c_void_p(st.cuda_stream), 'n': n,
-             'obs': blk.tensor((n, 3, 10), torch.float32), 'act': blk.tensor((n, 3), torch.int32),
-             'onehot': blk.tensor((n, 3, 5), torch.float32), 'obs2': blk.tensor((n, 3, 10), torch.float32),
-             'rew': blk.tensor((n, 3), torch.float32), 'done': blk.tensor((n, 3), torch.uint8)}
-        h['obs'].copy_(obs[k * n:(k + 1) * n].cpu())
-        halves.append(h)
-    for k, h in enumerate(halves):  # both chains are enqueued before anything is waited for
-        _lib.check(lib.actor_forward_host_async(actor._h, _lib.ptr(h['obs']), h['n'], 3, C.c_uint64(seed), C.c_uint64(5),
-                                                k * h['n'], _lib.ptr(h['act']), None, _lib.ptr(h['onehot']), k, h['sp']),
-                   'actor_forward_host_async')
-        _lib.check(lib.mpe_step_host_async(h['env']._h, _lib.ptr(h['act']), None, _lib.ptr(h['obs2']), _lib.ptr(h['rew']),
-                                           _lib.ptr(h['done']), h['sp']), 'mpe_step_host_async')
-    for h in halves:
-        _lib.check(lib.mpe_host_wait(h['sp']), 'mpe_host_wait')
-    assert np.array_equal(np.concatenate([h['act'].numpy() for h in halves]), want['act_u'].cpu().numpy())
-    assert np.array_equal(np.concatenate([h['onehot'].numpy() for h in halves]), want['onehot'].cpu().numpy())
-    assert np.array_equal(np.concatenate([h['obs2'].numpy() for h in halves]), o2.cpu().numpy())
-    assert np.array_equal(np.concatenate([h['rew'].numpy() for h in halves]), r2.cpu().numpy())
-    assert lib.actor_forward_host_async(actor._h, _lib.ptr(halves[0]['obs']), 10, 3, 0, 0, 0, None, None, None, 7,
-                                        halves[0]['sp']) == _lib.MPE_EINVAL  # slot out of range
-    del halves
-    blk.free()
