@@ -374,69 +374,12 @@ __global__ void __launch_bounds__(kActorThreads, 1) k_actor_forward(ActorDev w, 
 // ------------------------------------------------------------------------------------------------
 // dense3 head of the "+model" actor on top of the tensor-core forward: next_state[row][j] = b3[j] + sum_k
 // relu(hcat)[row][k] W3[k][j] (ac_network_model_multi_gumbel.py:49,65).  64 x D MACs per row - HBM-bound on reading
-// hcat (256 B per row), so a plain FFMA kernel: one thread per (row, output), the row's 64 inputs are broadcast loads.
+// hcat (256 B per row), so a plain FFMA kernel.  A CTA stages 128 rows of relu(hcat) (32 KB, coalesced float4 loads)
+// and the head's weights in shared memory; thread (row pair = tid / 4, quarter = tid % 4) then produces outputs
+// quarter, quarter + 4, ... of its two rows: a row's 64 inputs are broadcast reads shared by four threads, the weights
+// are re-laid out so that a thread's DQ weights of one k are contiguous and feed 2 x DQ FMAs.  The tensor-core path
+// only takes D <= 32 (tc_layout), so DQ <= 8.
 // ------------------------------------------------------------------------------------------------
-constexpr int kD3Rows = 64;  // rows per CTA tile
-template <int DQ>  // DQ = ceil(D / 4): outputs per thread
-__global__ void __launch_bounds__(256) k_dense3(ActorDev w, const float *__restrict__ hcat, int64_t rows,
-                                                float *__restrict__ next_state) {
-  // A CTA stages 64 rows of relu(hcat) (16 KB, coalesced float4 loads) and the head's weights in shared memory; thread
-  // (row = tid / 4, quarter = tid % 4) then produces outputs quarter, quarter + 4, ... of its row: a row's 64 inputs are
-  // broadcast reads shared by four threads, the weights are re-laid out so that a thread's DQ weights of one k are
-  // contiguous.
-  __shared__ __align__(16) float sh[kD3Rows][kHid + 4];  // +4: rows start in different banks
-  constexpr int DQP = (DQ + 3) / 4 * 4;                  // a thread's weights of one k: DQP contiguous floats (LDS.128)
-  __shared__ __align__(16) float sw3[kHid * 4 * DQP + 4 * DQP];
-  const int D = w.D, Dpad = w.Dpad;
-  const float *W3 = w.blob + w.off_w3, *b3 = w.blob + w.off_b3;
-  for (int i = threadIdx.x; i < kHid * 4 * DQP; i += 256) {
-    const int k = i / (4 * DQP), rem = i - k * 4 * DQP, q = rem / DQP, jj = rem - q * DQP, j = q + 4 * jj;
-    sw3[i] = (jj < DQ && j < D) ? W3[k * Dpad + j] : 0.0f;
-  }
-  for (int i = threadIdx.x; i < 4 * DQP; i += 256) {
-    const int q = i / DQP, jj = i - q * DQP, j = q + 4 * jj;
-    sw3[kHid * 4 * DQP + i] = (jj < DQ && j < D) ? b3[j] : 0.0f;
-  }
-  const int r = threadIdx.x >> 2, qd = threadIdx.x & 3;
-  for (int64_t row0 = (int64_t)blockIdx.x * kD3Rows; row0 < rows; row0 += (int64_t)gridDim.x * kD3Rows) {
-    __syncthreads();  // weights staged / the previous tile is consumed
-    for (int i = threadIdx.x; i < kD3Rows * (kHid / 4); i += 256) {
-      const int rr = i / (kHid / 4), c4 = i - rr * (kHid / 4);
-      const float4 v = row0 + rr < rows ? reinterpret_cast<const float4 *>(hcat + (row0 + rr) * kHid)[c4]
-                                        : make_float4(0.0f, 0.0f, 0.0f, 0.0f);
-      *reinterpret_cast<float4 *>(&sh[rr][4 * c4]) = v;
-    }
-    __syncthreads();
-    float acc[DQP];
-#pragma unroll
-    for (int jj = 0; jj < DQP; ++jj) acc[jj] = sw3[kHid * 4 * DQP + qd * DQP + jj];
-#pragma unroll 4
-    for (int k0 = 0; k0 < kHid; k0 += 4) {
-      const float4 h4 = *reinterpret_cast<const float4 *>(&sh[r][k0]);
-      const float hk[4] = {h4.x, h4.y, h4.z, h4.w};
-#pragma unroll
-      for (int kk = 0; kk < 4; ++kk) {
-        const float4 *wk = reinterpret_cast<const float4 *>(sw3 + ((k0 + kk) * 4 + qd) * DQP);
-#pragma unroll
-        for (int v = 0; v < DQP / 4; ++v) {
-          const float4 w4 = wk[v];
-          acc[4 * v] = fmaf(hk[kk], w4.x, acc[4 * v]);
-          if (4 * v + 1 < DQ) acc[4 * v + 1] = fmaf(hk[kk], w4.y, acc[4 * v + 1]);
-          if (4 * v + 2 < DQ) acc[4 * v + 2] = fmaf(hk[kk], w4.z, acc[4 * v + 2]);
-          if (4 * v + 3 < DQ) acc[4 * v + 3] = fmaf(hk[kk], w4.w, acc[4 * v + 3]);
-        }
-      }
-    }
-    if (row0 + r < rows) {
-#pragma unroll
-      for (int jj = 0; jj < DQ; ++jj)
-        if (qd + 4 * jj < D) next_state[(row0 + r) * D + qd + 4 * jj] = acc[jj];
-    }
-  }
-}
-
-// The same head with two rows per thread and 128-row tiles (D <= 32): a thread's DQ weights of one k feed 2 x DQ
-// FMAs, and there are half as many barriers per row (80 -> ~50 us for 393,216 rows at D = 16).
 constexpr int kD3Rows2 = 128;
 template <int DQ>
 __global__ void __launch_bounds__(256) k_dense3x2(ActorDev w, const float *__restrict__ hcat, int64_t rows,
@@ -500,24 +443,13 @@ __global__ void __launch_bounds__(256) k_dense3x2(ActorDev w, const float *__res
 cudaError_t launch_dense3(const ActorDev &w, const float *hcat, int64_t rows, float *next_state, cudaStream_t st) {
   if (rows <= 0) return cudaSuccess;
   const int64_t nsm = sm_count(current_device());
-  if (w.D <= 32) {  // every scenario of the reference (D <= 30): two rows per thread
-    const int64_t blocks2 = (rows + kD3Rows2 - 1) / kD3Rows2;
-    const unsigned grid2 = (unsigned)(blocks2 < nsm * 5 ? blocks2 : nsm * 5);
-    switch ((w.D + 3) / 4) {
-#define D3X(Q) case Q: k_dense3x2<Q><<<grid2, 256, 0, st>>>(w, hcat, rows, next_state); break;
-      D3X(1) D3X(2) D3X(3) D3X(4) D3X(5) D3X(6) D3X(7) D3X(8)
-#undef D3X
-      default: return cudaErrorInvalidValue;
-    }
-    return cudaGetLastError();
-  }
-  const int64_t blocks = (rows + kD3Rows - 1) / kD3Rows;
-  const unsigned grid = (unsigned)(blocks < nsm * 8 ? blocks : nsm * 8);
+  const int64_t blocks2 = (rows + kD3Rows2 - 1) / kD3Rows2;
+  const unsigned grid2 = (unsigned)(blocks2 < nsm * 5 ? blocks2 : nsm * 5);
   switch ((w.D + 3) / 4) {
-#define D3(Q) case Q: k_dense3<Q><<<grid, 256, 0, st>>>(w, hcat, rows, next_state); break;
-    D3(1) D3(2) D3(3) D3(4) D3(5) D3(6) D3(7) D3(8) D3(9) D3(10) D3(11) D3(12) D3(13) D3(14) D3(15) D3(16)
-#undef D3
-    default: return cudaErrorInvalidValue;
+#define D3X(Q) case Q: k_dense3x2<Q><<<grid2, 256, 0, st>>>(w, hcat, rows, next_state); break;
+    D3X(1) D3X(2) D3X(3) D3X(4) D3X(5) D3X(6) D3X(7) D3X(8)
+#undef D3X
+    default: return cudaErrorInvalidValue;  // D > 32: no tensor-core forward feeds this head
   }
   return cudaGetLastError();
 }

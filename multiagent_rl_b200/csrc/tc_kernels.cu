@@ -566,13 +566,16 @@ __global__ void __launch_bounds__(tc2_threads(N), 1)
         }
 
         if (!have_w) { mbar_wait(&bars[0], 0); have_w = true; }
-        // dense2 sums of the OWN tile's rows over this thread's 16 units (+ bias), packed pairs of head entries
+        // dense2 sums of the OWN tile's rows over this thread's 16 units, packed pairs of head entries (large teams:
+        // just the bias, the shares come from the scratch rows).  Small teams add the bias after the two warpgroups'
+        // sums: (own + other) + bias rounds the same whichever warpgroup owns the tile, so an env's logits do not depend
+        // on the parity of its tile, i.e. on where it sits in the batch (HostRollout shards start anywhere)
         constexpr int NLG = kJit ? 1 : N;
         f2 lgp[NLG][APAD / 2];
 #pragma unroll
         for (int t = 0; t < NLG; ++t)
 #pragma unroll
-          for (int a = 0; a < APAD / 2; ++a) lgp[t][a] = pk(b2[2 * a], b2[2 * a + 1]);
+          for (int a = 0; a < APAD / 2; ++a) lgp[t][a] = kJit ? pk(b2[2 * a], b2[2 * a + 1]) : 0ull;
 
         // cell state of this thread's 16 units (2 chunks x 4 packed pairs), one set per tile
         f2 cA[2][4], cB[2][4];
@@ -875,7 +878,7 @@ __global__ void __launch_bounds__(tc2_threads(N), 1)
               } else {
                 other = own_xchg2[((size_t)t * (APAD / 2) + a) * kRows + row];
               }
-              upk(add2(lgp[t][a], other), lgt[2 * a], lgt[2 * a + 1]);
+              upk(add2(add2(lgp[t][a], other), pk(b2[2 * a], b2[2 * a + 1])), lgt[2 * a], lgt[2 * a + 1]);
             }
             const int64_t orow = b * N + t;
 #pragma unroll

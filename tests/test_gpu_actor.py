@@ -372,11 +372,16 @@ def test_fused_rollout_equals_stepwise_path_tiny_batches(scenario, n, A, impl):
 @pytest.mark.parametrize('scenario,shards,B', [('simple_spread', 3, 5001), ('simple_spread', 1, 700),
                                                ('simple_reference', 2, 2050), ('simple_spread', 4, 3),
                                                ('fullobs_collect_treasure', 2, 515),
-                                               ('fullobs_collect_treasure', 4, 20_011)])
+                                               ('fullobs_collect_treasure', 4, 20_011),
+                                               ('simple_reference', 2, 113_801),
+                                               ('fullobs_collect_treasure', 2, 113_801)])
 def test_host_rollout_shards_match_the_blocking_calls(scenario, shards, B):
     """HostRollout (non-blocking mpe_act_step_host_async per shard and stream) gives, for every shard count, exactly
     the transitions of the device-tensor calls on one env handle: same Philox keys (global env id, step), same
-    kernels.  Both ends of each transition are on the host: obs_prev -> (act, rew) -> obs."""
+    kernels.  Both ends of each transition are on the host: obs_prev -> (act, rew) -> obs.  The two 113,801-env
+    configurations give each shard 445 tiles of 128 envs, more than one wave of tile pairs on a 148-SM part, so the
+    per-stream dense2-share scratch rows of the two-head and the 8-agent tensor-core actors are reused by CTAs that
+    walk a second pair."""
     import multiagent_rl_b200 as m
     L, seed = 4, 31
     n = None
