@@ -236,8 +236,11 @@ __global__ void __launch_bounds__(kStepThreads)
     if (info_f != nullptr) info_f[b] = md;
   }
   if (done != nullptr) {  // no done_callback (experiments/scenarios.py:186-190): always False
-    if (full) {
-      uint32_t *d32 = reinterpret_cast<uint32_t *>(done + b0 * N);  // 32*N bytes, 16 B aligned
+    // a full warp's span is 32*N bytes at done + b0*N, and b0*N is a multiple of 32: when `done` itself is
+    // 4 B aligned the span can be zeroed with 32-bit stores.  A caller's `done` may sit at any byte offset
+    // (a slice of a [T][B][N] record at odd B*N), so otherwise every env stores its own bytes.
+    if (full && (reinterpret_cast<uintptr_t>(done) & 3) == 0) {
+      uint32_t *d32 = reinterpret_cast<uint32_t *>(done + b0 * N);
       for (int k = lane; k < 8 * N; k += 32) d32[k] = 0u;
     } else if (active) {
 #pragma unroll

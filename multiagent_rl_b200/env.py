@@ -254,11 +254,52 @@ class BatchedMultiAgentEnv(object):
                 self.set_state(None, None, lm, goal)
         self._tr_flags = goal[:, 0].copy()
 
+    def _check_out(self, out, host):
+        """``out`` = (obs[B,N,D], rew[B,N], done[B,N] uint8): each entry None (that output is skipped) or a
+        C-contiguous buffer of exactly that shape and dtype, on the env's device (``host=False``: torch tensors) or
+        in host memory (``host=True``: numpy arrays or CPU tensors).  The kernels write B*N*D / B*N elements through
+        the raw pointer, so anything else would be written out of bounds or misread: refuse it before any launch."""
+        B, N = self.num_envs, self.n
+        if not isinstance(out, (tuple, list)) or len(out) != 3:
+            raise ValueError('out must be a tuple (obs, rew, done)')
+        real = np.float32 if self.precision == 'fp32' else np.float64
+        want = (('obs', (B, N, self.obs_dim), real), ('rew', (B, N), real), ('done', (B, N), np.uint8))
+        for x, (name, shape, dt) in zip(out, want):
+            if x is None:
+                continue
+            if isinstance(x, torch.Tensor):
+                if x.device.type == 'cpu':
+                    where = 'host'
+                elif x.device == self.device:
+                    where = 'device'
+                else:
+                    where = str(x.device)
+                dtype_ok = x.dtype == {np.float32: torch.float32, np.float64: torch.float64, np.uint8: torch.uint8}[dt]
+                contiguous = x.is_contiguous()
+                got = (tuple(x.shape), x.dtype)
+            elif isinstance(x, np.ndarray) and host:
+                where, dtype_ok, contiguous = 'host', x.dtype == dt, bool(x.flags['C_CONTIGUOUS'])
+                got = (x.shape, x.dtype)
+            else:
+                raise ValueError('out %s must be a %s or None, got %s' % (name, 'numpy array / CPU tensor' if host
+                                                                         else 'torch tensor', type(x).__name__))
+            if where != ('host' if host else 'device'):
+                raise ValueError('out %s must be in %s, got a tensor on %s' % (
+                    name, 'host memory' if host else str(self.device), where))
+            if tuple(got[0]) != shape or not dtype_ok:
+                raise ValueError('out %s must be %s %s, got %s %s' % (name, np.dtype(dt).name, shape, got[1], got[0]))
+            if not contiguous:
+                raise ValueError('out %s must be contiguous' % name)
+        return tuple(out)
+
     # ------------------------------------------------------------------ tensor surface
     def step_tensor(self, act_u, act_c=None, comm_vec=None, out=None, info=False):
         """act_u [B,N] int (index of the movement head), act_c [B,N] int (message head) or
-        comm_vec [B,N,dim_c] real.  Returns (obs[B,N,D], rew[B,N], done[B,N] uint8, info dict)."""
+        comm_vec [B,N,dim_c] real.  Returns (obs[B,N,D], rew[B,N], done[B,N] uint8, info dict).
+        ``out`` = (obs, rew, done) writes into the caller's device tensors instead (see ``_check_out``)."""
         B, N = self.num_envs, self.n
+        if out is not None:
+            out = self._check_out(out, host=False)
         if self.discrete_action_input:
             remap = torch.tensor([0, 2, 1, 4, 3], device=self.device, dtype=torch.int32)
             act_u = remap[torch.as_tensor(act_u, device=self.device).long()]
@@ -290,6 +331,8 @@ class BatchedMultiAgentEnv(object):
         if out is None:
             dt = np.float32 if self.precision == 'fp32' else np.float64
             out = (np.empty((B, N, self.obs_dim), dt), np.empty((B, N), dt), np.empty((B, N), np.uint8))
+        else:
+            out = self._check_out(out, host=True)
         obs, rew, done = out
         _lib.check(self._lib.mpe_step_host(self._h, _lib.ptr(act_u), _lib.ptr(act_c), _lib.ptr(obs), _lib.ptr(rew),
                                            _lib.ptr(done), self._stream()), 'mpe_step_host')
