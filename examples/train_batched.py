@@ -1,8 +1,8 @@
 """Batched training loop: thousands of particle envs on the GPU feeding the REFERENCE's own learner.
 
 What runs where:
-  * acting + env stepping: `env.rollout(fused_actor, 25, record=True)` - one fused CUDA kernel per episode
-    (experiments/run.py:36-65 for B envs at once);
+  * acting + env stepping: `env.rollout(fused_actor, 25, record=True, replay=memory)` - one fused CUDA kernel per
+    episode (experiments/run.py:36-65 for B envs at once) and one launch that appends its transitions to the ring;
   * replay: `DeviceReplayBuffer` (the reference ReplayBuffer's surface, rls/replay_buffer.py:9-91) - transitions
     never leave HBM;
   * learning: the reference's `Trainer.optimize()` (rls/agent/multiagent/ddpg_gumbel_fix.py:131-219) UNCHANGED, with the
@@ -57,11 +57,9 @@ def train(num_envs=4096, episodes=20, updates_per_episode=4, scenario='simple_sp
     returns = []
     t0 = time.time()
     for ep in range(episodes):
-        obs0 = env.reset()                                                   # [B,N,D]
-        obs_next, rew, act_u, _ = env.rollout(fused, T, step0=ep * T, record=True)   # [T,B,N,...]
-        obs_t = torch.cat([obs0[None], obs_next[:-1]], 0)
-        for t in range(T):                                                   # ReplayBuffer.add, B transitions per call
-            memory.add(obs_t[t], act_u[t], rew[t], obs_next[t])
+        env.reset()
+        # T * B transitions go straight into the replay ring; rew [T,B,N] is kept for the episode history
+        _, rew, _, _ = env.rollout(fused, T, step0=ep * T, record=True, replay=memory)
         hist.add_rollout(rew)
         returns.append(float(rew.sum((0, 2)).mean()))
         if len(memory) >= batch_size:

@@ -35,7 +35,7 @@
 extern "C" {
 #endif
 
-#define MPE_ABI_VERSION 4
+#define MPE_ABI_VERSION 5
 
 enum { MPE_OK = 0, MPE_EINVAL = -1, MPE_ECUDA = -2, MPE_EUNSUPPORTED = -3 };
 enum { MPE_SIMPLE_SPREAD = 0, MPE_SIMPLE_REFERENCE = 1, MPE_SIMPLE_SPEAKER_LISTENER = 2,
@@ -266,6 +266,18 @@ int replay_add(MpeReplay *replay, const float *obs, const int32_t *act_u, const 
  * [batch][N][D], act_onehot [batch][N][act0+act1], rew [batch], done [batch], idx_out [batch]. */
 int replay_sample(MpeReplay *replay, int64_t batch, const int64_t *idx, uint64_t seed, float *obs, float *act_onehot,
                   float *rew, float *obs_next, float *done, int64_t *idx_out, void *stream);
+
+/* mpe_rollout that also appends every env-step's transition to `replay`: (obs_t, act_u, act_c, sum_n rew,
+ * obs_{t+1}, done = 0), where obs_t is the observation the actor acted on (the post-reset observation at an episode's
+ * first step) and obs_{t+1} the one the step returned (before any reset).  Step-major, then env order: the ring ends
+ * up as after T replay_add calls of B transitions each, wrapping as often as T * B / capacity says.  Recordings,
+ * env state, Philox streams and episode statistics are those of mpe_rollout; the recording pointers may be NULL.
+ * The ring must match the env and actor (num_agents, obs_dim, act0 / act1), sit on their device and hold at least
+ * B transitions; otherwise MPE_EINVAL before anything is launched.  Envs whose episodes are aligned (after an
+ * unmasked reset) run the fused kernel in segments up to each episode end and one ring-writer launch per segment;
+ * others run per-step kernels with one replay_add per step. */
+int mpe_rollout_replay(MpeEnv *env, MpeActor *actor, MpeReplay *replay, int32_t T, uint64_t step0, float *obs_next,
+                       float *rew, int32_t *act_u, int32_t *act_c, void *stream);
 
 #ifdef __cplusplus
 }

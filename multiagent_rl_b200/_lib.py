@@ -7,7 +7,7 @@ import os
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get('MPE_B200_LIB', os.path.join(HERE, 'libmpe_b200.so'))  # override: A/B builds
-ABI_VERSION = 4
+ABI_VERSION = 5
 
 MPE_OK, MPE_EINVAL, MPE_ECUDA, MPE_EUNSUPPORTED = 0, -1, -2, -3
 SCENARIO_IDS = {'simple_spread': 0, 'simple_reference': 1, 'simple_speaker_listener': 2, 'fullobs_collect_treasure': 3}
@@ -103,6 +103,7 @@ SIGNATURES = {
     'replay_next_idx': (C.c_int64, [P]),
     'replay_add': (C.c_int, [P, P, P, P, P, P, P, C.c_int64, P]),
     'replay_sample': (C.c_int, [P, C.c_int64, P, C.c_uint64, P, P, P, P, P, P, P]),
+    'mpe_rollout_replay': (C.c_int, [P, P, P, C.c_int32, C.c_uint64, P, P, P, P, P]),
 }
 
 _lib = None

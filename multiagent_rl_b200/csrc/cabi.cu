@@ -62,6 +62,11 @@ struct MpeEnv {
   // scratch of the per-step rollout (teams of > 3 agents, the FFMA actor): current observations and sampled actions
   float *r_obs = nullptr;
   int32_t *r_act = nullptr;
+  // mpe_rollout_replay: the per-step path's second observation buffer (obs_t and obs_{t+1} of one transition must
+  // both survive the step) and rewards when the caller records none; the fused path's recordings of one segment
+  float *r_obs2 = nullptr, *r_rew = nullptr;
+  unsigned char *rr_scratch = nullptr;
+  size_t rr_bytes = 0;
   // mpe_act_step_host_async: device mirror of the caller's observations and of its transition block
   float *hb_obs_in = nullptr;
   unsigned char *hb_block = nullptr;
@@ -228,7 +233,7 @@ int mpe_destroy(MpeEnv *env) {
   mpe::EnvStateAny &s = env->st;
   void *ptrs[] = {s.pv, s.lm, s.ep_ret, s.comm, s.goal, s.episode, s.tstep, s.stats,
                   env->h_act_u, env->h_act_c, env->h_obs, env->h_rew, env->h_done, env->r_obs, env->r_act,
-                  env->hb_obs_in, env->hb_block, env->tc_scratch};
+                  env->r_obs2, env->r_rew, env->rr_scratch, env->hb_obs_in, env->hb_block, env->tc_scratch};
   for (void *p : ptrs)
     if (p != nullptr) cudaFree(p);
   delete env;
@@ -587,64 +592,190 @@ int mpe_host_wait(void *stream) {
   return MPE_OK;
 }
 
+// The common episode step of a synced env after T fused iterations (every env resets when its step reaches L).
+static void advance_episode_step(MpeEnv *env, int64_t T) {
+  const int L = env->st.max_episode_len;
+  if (!env->synced || L <= 0) return;  // without auto-reset the episode step never decides a launch
+  const int64_t first_end = env->host_tstep >= L ? 1 : L - env->host_tstep;
+  env->host_tstep = T < first_end ? (int32_t)(env->host_tstep + T) : (int32_t)((T - first_end) % L);
+}
+
+static bool use_fused_rollout(const MpeEnv *env, const MpeActor *actor) {
+  return actor->dev.impl != mpe::kImplSimt && mpe::tc_rollout_supported(actor->dev.tc, env->st.N);
+}
+
+static int check_rollout(const MpeEnv *env, const MpeActor *actor, const char *who) {
+  const std::string w(who);
+  if (env->st.precision != MPE_F32) return fail(MPE_EUNSUPPORTED, w + ": fp32 envs only");
+  if (env->device != actor->device) return fail(MPE_EINVAL, w + ": env and actor on different devices");
+  if (actor->dev.D != env->st.D) return fail(MPE_EINVAL, w + ": actor obs_dim does not match the env");
+  if (actor->dev.A0 != 5 || actor->dev.A1 != env->st.act_c)
+    return fail(MPE_EINVAL, w + ": actor heads do not match the env's action space");
+  if (!mpe::rollout_supported(env->st.scenario, env->st.N))
+    return fail(MPE_EUNSUPPORTED, w + ": unsupported scenario / agent count");
+  return MPE_OK;
+}
+
+// Every combination the fused kernel does not cover (teams of > 3 agents, the fp32 FFMA actor, and with a ring envs
+// whose episodes are not aligned): the same loop as kernels per step - actor (tensor cores where the shape is covered,
+// else FFMA), the env step kernel, and a reset kernel on the steps where an episode can end.  Same Philox keys, same
+// arithmetic: bit-identical to the stepwise calls.  With `rep`, each step's B transitions are appended after the step
+// and before the reset overwrites the observations: obs_t is `cur`, obs_{t+1} is `o`.
+static int rollout_stepwise(MpeEnv *env, MpeActor *actor, MpeReplay *rep, int32_t T, uint64_t step0, float *obs_next,
+                            float *rew, int32_t *act_u, int32_t *act_c, cudaStream_t st) {
+  mpe::EnvStateAny s = env->st;
+  s.track = 1;
+  const int64_t rows = s.B * s.N;
+  if (env->r_obs == nullptr) {
+    CK(cudaMalloc(&env->r_obs, (size_t)rows * s.D * sizeof(float)));
+    CK(cudaMalloc(&env->r_act, (size_t)rows * 2 * sizeof(int32_t)));
+  }
+  if (rep != nullptr && obs_next == nullptr && env->r_obs2 == nullptr)
+    CK(cudaMalloc(&env->r_obs2, (size_t)rows * s.D * sizeof(float)));
+  if (rep != nullptr && rew == nullptr && env->r_rew == nullptr) CK(cudaMalloc(&env->r_rew, (size_t)rows * sizeof(float)));
+  CK(mpe::launch_observe(s, env->r_obs, st));
+  const float *cur = env->r_obs;
+  const int L = s.max_episode_len;
+  for (int t = 0; t < T; ++t) {
+    mpe::ActorIO aio;
+    aio.obs = cur; aio.B = s.B; aio.N = s.N; aio.seed = s.seed; aio.step = step0 + (uint64_t)t; aio.gid0 = s.gid0;
+    aio.act_u = act_u != nullptr ? act_u + (int64_t)t * rows : env->r_act;
+    if (s.act_c > 0) aio.act_c = act_c != nullptr ? act_c + (int64_t)t * rows : env->r_act + rows;
+    CK(launch_actor(actor, aio, &env->tc_scratch, st));  // rollouts of several envs may share one actor on different streams
+    float *o = obs_next != nullptr ? obs_next + (int64_t)t * rows * s.D
+                                   : (rep != nullptr && cur == env->r_obs ? env->r_obs2 : env->r_obs);
+    float *r = rew != nullptr ? rew + (int64_t)t * rows : (rep != nullptr ? env->r_rew : nullptr);
+    CK(mpe::launch_step(s, aio.act_u, aio.act_c, nullptr, o, r, nullptr, nullptr, nullptr, st));
+    if (rep != nullptr) {
+      CK(mpe::launch_replay_add(rep->dev, rep->head, s.B, cur, aio.act_u, aio.act_c, r, o, nullptr, st));
+      rep->head = (rep->head + s.B) % rep->dev.capacity;
+      rep->size = rep->size + s.B < rep->dev.capacity ? rep->size + s.B : rep->dev.capacity;
+    }
+    cur = o;
+    env->host_tstep += 1;
+    const bool may_end = L > 0 && (!env->synced || env->host_tstep >= L);
+    if (may_end) {  // experiments/run.py:59-60; also re-emits the observations the next actor call reads
+      CK(mpe::launch_reset(s, nullptr, env->r_obs, L, st));
+      cur = env->r_obs;
+      if (env->synced) env->host_tstep = 0;
+    }
+  }
+  return MPE_OK;
+}
+
 int mpe_rollout(MpeEnv *env, MpeActor *actor, int32_t T, uint64_t step0, float *obs_next, float *rew, int32_t *act_u,
                 int32_t *act_c, void *stream) {
   if (env == nullptr || actor == nullptr) return fail(MPE_EINVAL, "mpe_rollout: null handle");
   if (T <= 0) return MPE_OK;
-  if (env->st.precision != MPE_F32) return fail(MPE_EUNSUPPORTED, "mpe_rollout: fp32 envs only");
-  if (env->device != actor->device) return fail(MPE_EINVAL, "mpe_rollout: env and actor on different devices");
-  if (actor->dev.D != env->st.D) return fail(MPE_EINVAL, "mpe_rollout: actor obs_dim does not match the env");
-  if (actor->dev.A0 != 5 || actor->dev.A1 != env->st.act_c)
-    return fail(MPE_EINVAL, "mpe_rollout: actor heads do not match the env's action space");
-  if (!mpe::rollout_supported(env->st.scenario, env->st.N))
-    return fail(MPE_EUNSUPPORTED, "mpe_rollout: unsupported scenario / agent count");
+  if (int rc = check_rollout(env, actor, "mpe_rollout")) return rc;
   DeviceGuard g(env->device);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   // One kernel for all T steps: teams of 2 / 3 on the tensor cores (the large teams run faster as actor + step kernels
   // per step, DESIGN.md 4.3)
-  if (actor->dev.impl != mpe::kImplSimt && mpe::tc_rollout_supported(actor->dev.tc, env->st.N)) {
+  if (use_fused_rollout(env, actor)) {
     mpe::RolloutIO io;
     io.T = T; io.step0 = step0; io.obs_next = obs_next; io.rew = rew; io.act_u = act_u; io.act_c = act_c;
     mpe::TcDev tcw;
     CK(tc_for_stream(actor, env->st.N, &env->tc_scratch, &tcw));  // rollouts of several envs may share one actor
     CK(mpe::launch_rollout_tc(env->st, tcw, io, st));
-    env->synced = false;
+    advance_episode_step(env, T);
     return MPE_OK;
   }
-  {
-    // Every other combination (teams of > 3 agents, the fp32 FFMA actor): the same loop as kernels per step - actor
-    // (tensor cores where the shape is covered, else FFMA), the env step kernel, and a reset kernel on the steps
-    // where an episode can end.  Same Philox keys, same arithmetic: bit-identical to the stepwise calls.
-    mpe::EnvStateAny s = env->st;
-    s.track = 1;
-    const int64_t rows = s.B * s.N;
-    if (env->r_obs == nullptr) {
-      CK(cudaMalloc(&env->r_obs, (size_t)rows * s.D * sizeof(float)));
-      CK(cudaMalloc(&env->r_act, (size_t)rows * 2 * sizeof(int32_t)));
+  return rollout_stepwise(env, actor, nullptr, T, step0, obs_next, rew, act_u, act_c, st);
+}
+
+// The fused path of mpe_rollout_replay keeps the recordings the caller does not take in an env-owned scratch of at
+// most this many bytes, kept until mpe_destroy so that the calls of a training loop do not allocate; a segment is cut
+// short where the next step's recordings would not fit (one recorded step of simple_spread N = 3 at 1,048,576 envs is
+// 144 MB: 7 steps per segment).
+constexpr size_t kRolloutReplayScratchBytes = size_t(1) << 30;
+
+// Synced envs with the fused kernel: the call runs as segments that end at the common episode end (or where the
+// scratch is full).  k_tc2 runs each segment unchanged and records into the caller's buffers or the scratch; one
+// launch of the multi-step ring writer then builds the segment's records, obs_t of its first step from the
+// observation before the segment (mpe_observe after an episode end: the post-reset observation; else a copy of the
+// last step's obs_next) and of every later step from the previous step's obs_next.
+static int rollout_fused_replay(MpeEnv *env, MpeActor *actor, MpeReplay *rep, int32_t T, uint64_t step0, float *obs_next,
+                                float *rew, int32_t *act_u, int32_t *act_c, cudaStream_t st) {
+  const mpe::EnvStateAny &s = env->st;
+  const int64_t rows = s.B * s.N, obs_step = rows * s.D;
+  auto up = [](size_t x) { return (x + 255) / 256 * 256; };
+  const size_t b_obs = obs_next ? 0 : up(obs_step * 4), b_rew = rew ? 0 : up(rows * 4), b_au = act_u ? 0 : up(rows * 4),
+               b_ac = (act_c || s.act_c == 0) ? 0 : up(rows * 4), per_step = b_obs + b_rew + b_au + b_ac;
+  const int L = s.max_episode_len;
+  int64_t seg_cap = per_step == 0 ? T : (int64_t)(kRolloutReplayScratchBytes / per_step);
+  seg_cap = seg_cap < 1 ? 1 : (seg_cap > T ? T : seg_cap);
+  if (L > 0 && seg_cap > L) seg_cap = L;
+  if (env->r_obs == nullptr) {
+    CK(cudaMalloc(&env->r_obs, (size_t)obs_step * sizeof(float)));
+    CK(cudaMalloc(&env->r_act, (size_t)rows * 2 * sizeof(int32_t)));
+  }
+  const size_t need = per_step * (size_t)seg_cap;
+  if (need > env->rr_bytes) {
+    if (env->rr_scratch != nullptr) {  // a recording of an earlier call may still be read on this stream
+      CK(cudaStreamSynchronize(st));
+      cudaFree(env->rr_scratch);
+      env->rr_scratch = nullptr; env->rr_bytes = 0;
     }
-    CK(mpe::launch_observe(s, env->r_obs, st));
-    const float *cur = env->r_obs;
-    const int L = s.max_episode_len;
-    for (int t = 0; t < T; ++t) {
-      mpe::ActorIO aio;
-      aio.obs = cur; aio.B = s.B; aio.N = s.N; aio.seed = s.seed; aio.step = step0 + (uint64_t)t; aio.gid0 = s.gid0;
-      aio.act_u = act_u != nullptr ? act_u + (int64_t)t * rows : env->r_act;
-      if (s.act_c > 0) aio.act_c = act_c != nullptr ? act_c + (int64_t)t * rows : env->r_act + rows;
-      CK(launch_actor(actor, aio, &env->tc_scratch, st));  // rollouts of several envs may share one actor on different streams
-      float *o = obs_next != nullptr ? obs_next + (int64_t)t * rows * s.D : env->r_obs;
-      CK(mpe::launch_step(s, aio.act_u, aio.act_c, nullptr, o, rew != nullptr ? rew + (int64_t)t * rows : nullptr, nullptr,
-                          nullptr, nullptr, st));
-      cur = o;
-      env->host_tstep += 1;
-      const bool may_end = L > 0 && (!env->synced || env->host_tstep >= L);
-      if (may_end) {  // experiments/run.py:59-60; also re-emits the observations the next actor call reads
-        CK(mpe::launch_reset(s, nullptr, env->r_obs, L, st));
-        cur = env->r_obs;
-        if (env->synced) env->host_tstep = 0;
-      }
+    CK(cudaMalloc(&env->rr_scratch, need));
+    env->rr_bytes = need;
+  }
+  unsigned char *sc = env->rr_scratch;
+  float *sc_obs = reinterpret_cast<float *>(sc);
+  float *sc_rew = reinterpret_cast<float *>(sc + b_obs * seg_cap);
+  int32_t *sc_au = reinterpret_cast<int32_t *>(sc + (b_obs + b_rew) * seg_cap);
+  int32_t *sc_ac = reinterpret_cast<int32_t *>(sc + (b_obs + b_rew + b_au) * seg_cap);
+  mpe::TcDev tcw;
+  CK(tc_for_stream(actor, s.N, &env->tc_scratch, &tcw));  // rollouts of several envs may share one actor
+  const int64_t keep_from = (int64_t)T * s.B - rep->dev.capacity;  // earlier transitions are overwritten in this call
+  CK(mpe::launch_observe(s, env->r_obs, st));
+  for (int32_t t0 = 0; t0 < T;) {
+    int64_t n = T - t0 < seg_cap ? T - t0 : seg_cap;
+    const int64_t to_end = L > 0 ? (env->host_tstep >= L ? 1 : L - env->host_tstep) : n;
+    if (to_end < n) n = to_end;
+    mpe::RolloutIO io;
+    io.T = (int32_t)n; io.step0 = step0 + (uint64_t)t0;
+    io.obs_next = obs_next ? obs_next + t0 * obs_step : sc_obs;
+    io.rew = rew ? rew + t0 * rows : sc_rew;
+    io.act_u = act_u ? act_u + t0 * rows : sc_au;
+    io.act_c = s.act_c == 0 ? nullptr : (act_c ? act_c + t0 * rows : sc_ac);
+    CK(mpe::launch_rollout_tc(s, tcw, io, st));
+    CK(mpe::launch_replay_add_steps(rep->dev, rep->head, s.B, io.T, (int64_t)t0 * s.B, keep_from, env->r_obs, io.obs_next,
+                                    io.act_u, io.act_c, io.rew, st));
+    const bool ended = n == to_end && L > 0;
+    advance_episode_step(env, n);
+    t0 += (int32_t)n;
+    if (t0 < T) {
+      if (ended) CK(mpe::launch_observe(s, env->r_obs, st));
+      else CK(cudaMemcpyAsync(env->r_obs, io.obs_next + (n - 1) * obs_step, (size_t)obs_step * sizeof(float),
+                              cudaMemcpyDeviceToDevice, st));
     }
   }
+  const int64_t total = (int64_t)T * s.B;
+  rep->head = (rep->head + total) % rep->dev.capacity;
+  rep->size = rep->size + total < rep->dev.capacity ? rep->size + total : rep->dev.capacity;
   return MPE_OK;
+}
+
+int mpe_rollout_replay(MpeEnv *env, MpeActor *actor, MpeReplay *rep, int32_t T, uint64_t step0, float *obs_next,
+                       float *rew, int32_t *act_u, int32_t *act_c, void *stream) {
+  if (env == nullptr || actor == nullptr || rep == nullptr) return fail(MPE_EINVAL, "mpe_rollout_replay: null handle");
+  if (T <= 0) return MPE_OK;
+  if (int rc = check_rollout(env, actor, "mpe_rollout_replay")) return rc;
+  const mpe::ReplayDev &r = rep->dev;
+  if (rep->device != env->device) return fail(MPE_EINVAL, "mpe_rollout_replay: ring and env on different devices");
+  if (r.N != env->st.N || r.D != env->st.D)
+    return fail(MPE_EINVAL, "mpe_rollout_replay: ring agents / obs_dim do not match the env");
+  if (r.A0 != actor->dev.A0 || r.A1 != actor->dev.A1)
+    return fail(MPE_EINVAL, "mpe_rollout_replay: ring action heads do not match the actor");
+  if (env->st.B > r.capacity) return fail(MPE_EINVAL, "mpe_rollout_replay: batch larger than the ring");
+  DeviceGuard g(env->device);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  // the fused kernel needs the episode ends of all envs to coincide: only there can a segment end and the ring
+  // writer find every step's obs_t among the recordings
+  if (use_fused_rollout(env, actor) && env->synced)
+    return rollout_fused_replay(env, actor, rep, T, step0, obs_next, rew, act_u, act_c, st);
+  return rollout_stepwise(env, actor, rep, T, step0, obs_next, rew, act_u, act_c, st);
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -62,6 +62,68 @@ __global__ void __launch_bounds__(256) k_replay_add(ReplayDev r, int64_t slot0, 
   }
 }
 
+// add for T steps of a rollout at once: k_replay_add's record assembly on a (block, step) grid.  Step t's obs_t is
+// obs0 for t = 0 and obs_next[t - 1] after that (within one episode the observation an actor acts on is the one the
+// previous step returned); transition `first + t * B + b` of the call lands in ring slot (head + that) % capacity.
+// Transitions before `keep_from` would be overwritten by a later transition of the same call: they are skipped, so
+// that no two blocks of one launch write the same slot.  A block's records are one ring span apart from one wrap.
+template <int V>
+__global__ void __launch_bounds__(256) k_replay_add_steps(ReplayDev r, int64_t head, int64_t B, int T, int64_t first,
+                                                          int64_t keep_from, int rpb, const float *__restrict__ obs0,
+                                                          const float *__restrict__ obs_next, const int32_t *__restrict__ act_u,
+                                                          const int32_t *__restrict__ act_c, const float *__restrict__ rew) {
+  extern __shared__ __align__(16) unsigned char tile[];
+  const int R = r.N * r.D, RV = R / V, rec = (int)r.rec_bytes, VPR = rec / 16;
+  const int dj = 256 / RV, dc = 256 - dj * RV;
+  for (int t = blockIdx.y; t < T; t += gridDim.y) {
+    const float *so_t = t == 0 ? obs0 : obs_next + (int64_t)(t - 1) * B * R, *sn_t = obs_next + (int64_t)t * B * R;
+    const int64_t g_t = first + (int64_t)t * B;  // call-wide index of env 0's transition of step t
+    for (int64_t bb = (int64_t)blockIdx.x * rpb; bb < B; bb += (int64_t)gridDim.x * rpb) {
+      const int64_t skip = keep_from - (g_t + bb), end = (B - bb) < rpb ? (B - bb) : rpb;
+      if (skip >= end) continue;  // uniform per block
+      const int64_t b0 = skip > 0 ? bb + skip : bb;
+      const int nrows = (int)(bb + end - b0);
+      {
+        int row = threadIdx.x / RV, c = threadIdx.x - row * RV;
+        const float *so = so_t + b0 * R, *sn = sn_t + b0 * R;
+        for (int e = threadIdx.x; e < nrows * RV; e += 256, row += dj, c += dc) {
+          if (c >= RV) { c -= RV; ++row; }
+          unsigned char *rp = tile + row * rec;
+          if (V == 2) {
+            reinterpret_cast<float2 *>(rp)[c] = reinterpret_cast<const float2 *>(so)[e];
+            reinterpret_cast<float2 *>(rp + r.off_next())[c] = reinterpret_cast<const float2 *>(sn)[e];
+          } else {
+            reinterpret_cast<float *>(rp)[c] = so[e];
+            reinterpret_cast<float *>(rp + r.off_next())[c] = sn[e];
+          }
+        }
+      }
+      const int64_t a0 = (int64_t)t * B * r.N + b0 * r.N;
+      for (int e = threadIdx.x; e < nrows * r.N; e += 256) {
+        const int row = e / r.N, n = e - row * r.N;
+        tile[row * rec + r.off_au() + n] = (unsigned char)(int8_t)act_u[a0 + e];
+        tile[row * rec + r.off_ac() + n] = act_c != nullptr ? (unsigned char)(int8_t)act_c[a0 + e] : (unsigned char)0;
+      }
+      for (int row = threadIdx.x; row < nrows; row += 256) {
+        float s = 0.0f;  // rew_shared = np.sum(rew_n) (experiments/run.py:46), agent order
+        for (int n = 0; n < r.N; ++n) s += rew[a0 + (int64_t)row * r.N + n];
+        *reinterpret_cast<float *>(tile + row * rec + r.off_rew()) = s;
+        *reinterpret_cast<float *>(tile + row * rec + r.off_done()) = 0.0f;
+      }
+      __syncthreads();
+      // the first n1 records end at the ring's last slot, the rest continue at slot 0
+      const int64_t s0 = (head + g_t + b0) % r.capacity;
+      const int n1v = (int)((r.capacity - s0) < nrows ? (r.capacity - s0) : nrows) * VPR;
+      uint4 *dst0 = reinterpret_cast<uint4 *>(r.ring + s0 * r.rec_bytes), *dst1 = reinterpret_cast<uint4 *>(r.ring);
+      const uint4 *src = reinterpret_cast<const uint4 *>(tile);
+      for (int v = threadIdx.x; v < nrows * VPR; v += 256) {
+        if (v < n1v) dst0[v] = src[v]; else dst1[v - n1v] = src[v];
+      }
+      __syncthreads();
+    }
+  }
+}
+
 // uniform indices with replacement: random.randint(0, len - 1) per sample (rls/replay_buffer.py:51-52)
 __global__ void __launch_bounds__(256) k_replay_make_index(int64_t size, int64_t batch, uint64_t seed, uint64_t counter,
                                                            int64_t *__restrict__ idx) {
@@ -205,6 +267,25 @@ cudaError_t launch_replay_add(const ReplayDev &r, int64_t head, int64_t B, const
                                              obs_next + row0 * R, done != nullptr ? done + row0 : nullptr);
     row0 += rows;
   }
+  return cudaGetLastError();
+}
+
+cudaError_t launch_replay_add_steps(const ReplayDev &r, int64_t head, int64_t B, int32_t T, int64_t first,
+                                    int64_t keep_from, const float *obs0, const float *obs_next, const int32_t *act_u,
+                                    const int32_t *act_c, const float *rew, cudaStream_t st) {
+  if (B <= 0 || T <= 0) return cudaSuccess;
+  if (r.rec_bytes > kReplayMaxRecordBytes) return cudaErrorInvalidValue;
+  int rpb = 128;  // records per block, as launch_replay_add
+  while (rpb > 1 && (int64_t)rpb * r.rec_bytes > 32 * 1024) rpb >>= 1;
+  const int64_t blocks = (B + rpb - 1) / rpb, cap = (int64_t)sm_count(current_device()) * 16;
+  const dim3 grid((unsigned)(blocks < cap ? blocks : cap), (unsigned)(T < 65535 ? T : 65535));
+  const size_t sm = (size_t)rpb * r.rec_bytes;
+  const bool v2 = (int64_t)r.N * r.D % 2 == 0 &&
+                  ((reinterpret_cast<uintptr_t>(obs0) | reinterpret_cast<uintptr_t>(obs_next)) & 7) == 0;
+  if (v2)
+    k_replay_add_steps<2><<<grid, 256, sm, st>>>(r, head, B, T, first, keep_from, rpb, obs0, obs_next, act_u, act_c, rew);
+  else
+    k_replay_add_steps<1><<<grid, 256, sm, st>>>(r, head, B, T, first, keep_from, rpb, obs0, obs_next, act_u, act_c, rew);
   return cudaGetLastError();
 }
 

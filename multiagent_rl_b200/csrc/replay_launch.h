@@ -26,6 +26,12 @@ constexpr int64_t kReplayMaxRecordBytes = 48 * 1024;
 cudaError_t launch_replay_add(const ReplayDev &r, int64_t head, int64_t B, const float *obs, const int32_t *act_u,
                               const int32_t *act_c, const float *rew, const float *obs_next, const float *done,
                               cudaStream_t st);
+// T steps of a rollout in one launch: step t's transitions are (t == 0 ? obs0 : obs_next[t-1], act_u[t], act_c[t],
+// rew[t], obs_next[t]) with done = 0, [T][B][...] sources; transition first + t*B + b goes to slot (head + that) %
+// capacity, and those before keep_from (overwritten later in the same call) are not written.
+cudaError_t launch_replay_add_steps(const ReplayDev &r, int64_t head, int64_t B, int32_t T, int64_t first,
+                                    int64_t keep_from, const float *obs0, const float *obs_next, const int32_t *act_u,
+                                    const int32_t *act_c, const float *rew, cudaStream_t st);
 cudaError_t launch_replay_make_index(int64_t size, int64_t batch, uint64_t seed, uint64_t counter, int64_t *idx,
                                      cudaStream_t st);
 cudaError_t launch_replay_gather(const ReplayDev &r, int64_t size, int64_t batch, const int64_t *idx, float *obs, float *act_onehot,

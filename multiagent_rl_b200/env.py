@@ -384,12 +384,21 @@ class BatchedMultiAgentEnv(object):
         return np.array(list(out), dtype=np.float64)
 
     # ------------------------------------------------------------------ fused rollout
-    def rollout(self, actor, T, step0=None, record=False):
+    def rollout(self, actor, T, step0=None, record=False, replay=None):
         """T fused iterations of experiments/run.py:36-65 (act -> step -> reward -> auto-reset).
-        ``record`` returns per-step (obs_next[T,B,N,D], rew[T,B,N], act_u[T,B,N], act_c[T,B,N] | None)."""
+        ``record`` returns per-step (obs_next[T,B,N,D], rew[T,B,N], act_u[T,B,N], act_c[T,B,N] | None).
+        ``replay`` (a DeviceReplayBuffer) receives every env-step's transition (obs_t, act, sum of rewards, obs_t+1,
+        done = 0) in step-major, then env order, as ``T`` calls of ``replay.add`` with ``B`` transitions each would:
+        obs_t is the observation the actor acted on, the post-reset one at an episode's first step.
+        Memory: on envs whose episodes are aligned (small teams on the tensor cores), the recordings not requested here
+        go to a scratch buffer the env keeps until it is destroyed - one segment's worth, at most 1 GiB (144 B per env
+        and step for simple_spread N = 3 without ``record``); other envs keep two observation buffers and a reward
+        buffer of one step."""
         if self.precision != 'fp32':
             raise RuntimeError('rollout is fp32 only')
         B, N = self.num_envs, self.n
+        if replay is not None:
+            self._check_replay(replay)
         step0 = self.global_step if step0 is None else int(step0)
         obs = rew = au = ac = None
         if record:
@@ -397,10 +406,31 @@ class BatchedMultiAgentEnv(object):
             rew = self._empty(T, B, N)
             au = self._empty(T, B, N, dtype=torch.int32)
             ac = self._empty(T, B, N, dtype=torch.int32) if self.act_c > 0 else None
-        _lib.check(self._lib.mpe_rollout(self._h, actor._h, int(T), C.c_uint64(step0), _lib.ptr(obs), _lib.ptr(rew),
-                                         _lib.ptr(au), _lib.ptr(ac), self._stream()), 'mpe_rollout')
+        if replay is None:
+            _lib.check(self._lib.mpe_rollout(self._h, actor._h, int(T), C.c_uint64(step0), _lib.ptr(obs), _lib.ptr(rew),
+                                             _lib.ptr(au), _lib.ptr(ac), self._stream()), 'mpe_rollout')
+        else:
+            _lib.check(self._lib.mpe_rollout_replay(self._h, actor._h, replay._h, int(T), C.c_uint64(step0),
+                                                    _lib.ptr(obs), _lib.ptr(rew), _lib.ptr(au), _lib.ptr(ac),
+                                                    self._stream()), 'mpe_rollout_replay')
         self.global_step = step0 + int(T)
         return (obs, rew, au, ac) if record else None
+
+    def _check_replay(self, replay):
+        """The ring stores this env's transitions: same device, agents, observation width and action heads, and room
+        for one step of every env."""
+        from .replay import DeviceReplayBuffer
+        if not isinstance(replay, DeviceReplayBuffer):
+            raise ValueError('replay must be a DeviceReplayBuffer, got %s' % type(replay).__name__)
+        if replay.device != self.device:
+            raise ValueError('replay is on %s, the env on %s' % (replay.device, self.device))
+        if (replay.N, replay.D) != (self.n, self.obs_dim):
+            raise ValueError('replay stores %d agents x %d observations, the env has %d x %d'
+                             % (replay.N, replay.D, self.n, self.obs_dim))
+        if (replay.act_dims[0], replay.A1) != (5, self.act_c):
+            raise ValueError('replay action heads %s do not match the env (5, %d)' % (replay.act_dims, self.act_c))
+        if self.num_envs > replay._maxsize:
+            raise ValueError('replay holds %d transitions, fewer than one step of %d envs' % (replay._maxsize, self.num_envs))
 
 
 def make_env(scenario_name, n=None, local_observation=True, benchmark=False, discrete_action=True, **kw):

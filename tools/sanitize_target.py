@@ -79,5 +79,18 @@ for n, D, cap, B in ((3, 7, 331, 203), (3, 10, 331, 203), (31, 67, 53, 37)):
     assert int(idx.min()) >= 0 and int(idx.max()) < len(rb)
     rb.sample_index(torch.tensor([-1, 0, cap - 1, cap, -10 * cap, 7], device='cuda'))
     rb.collect()
+# rollouts into the ring at ragged sizes: the multi-step writer (synced envs, fused kernel) with and without
+# recordings, the per-step path after a masked reset, and calls that wrap the ring
+for scen, n, B, cap in (('simple_spread', None, 129, 300), ('simple_reference', None, 33, 1000), ('simple_spread', 6, 65, 100)):
+    env = m.make_env(scen, n=n, num_envs=B, batched=True, seed=3, max_episode_len=3)
+    A = [5, env.act_c] if env.act_c else 5
+    actor = m.FusedActor(random_state_dict(env.obs_dim, A, 1), seed=3)
+    rb = m.DeviceReplayBuffer(cap, env.n, env.obs_dim, A)
+    env.reset()
+    env.rollout(actor, 7, record=True, replay=rb)
+    env.rollout(actor, 5, replay=rb)
+    env.reset(mask=(torch.arange(B, device='cuda') % 2).to(torch.uint8))
+    env.rollout(actor, 4, replay=rb)
+    rb.collect()
 torch.cuda.synchronize()
 print('sanitize target done')
