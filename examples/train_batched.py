@@ -65,7 +65,7 @@ def train(num_envs=4096, episodes=20, updates_per_episode=4, scenario='simple_sp
         if len(memory) >= batch_size:
             for _ in range(updates_per_episode):
                 learner.optimize()                                           # reference code, device replay
-            fused.load_state_dict(learner.actor.state_dict())
+            fused.load_state_dict(learner.actor.state_dict())  # CUDA parameters: packed on the device, in stream order
         log('episode %d: mean return %.2f over %d envs, %d transitions in replay, %.1f s'
             % (ep, returns[-1], num_envs, len(memory), time.time() - t0))
     return returns, learner, hist

@@ -15,8 +15,8 @@
  *   - buffers are borrowed: the caller allocates and keeps them alive until the
  *     work enqueued on `stream` (a cudaStream_t passed as void*) has finished.
  *     Handles own only their persistent state and free it in *_destroy.
- *   - nothing synchronises the host except the *_host entry points, *_destroy
- *     and mpe_stats_read.
+ *   - nothing synchronises the host except the *_host entry points, *_destroy,
+ *     mpe_stats_read, actor_load and critic_load.
  *   - a handle is not thread-safe; handles on different devices are independent.
  *     One MpeActor may serve several MpeEnv handles on DIFFERENT streams at the same time through mpe_rollout and
  *     mpe_act_step_host_async (scratch per env handle); actor_forward and actor_forward_host calls on one actor must
@@ -35,7 +35,7 @@
 extern "C" {
 #endif
 
-#define MPE_ABI_VERSION 5
+#define MPE_ABI_VERSION 6
 
 enum { MPE_OK = 0, MPE_EINVAL = -1, MPE_ECUDA = -2, MPE_EUNSUPPORTED = -3 };
 enum { MPE_SIMPLE_SPREAD = 0, MPE_SIMPLE_REFERENCE = 1, MPE_SIMPLE_SPEAKER_LISTENER = 2,
@@ -168,7 +168,8 @@ typedef struct {
   int32_t reserved0;
 } ActorConfig;
 
-/* HOST pointers to fp32 tensors in the reference's state_dict layout (row-major [out][in]). */
+/* Pointers to fp32 tensors in the reference's state_dict layout (row-major [out][in], contiguous, 4 B alignment
+ * suffices): HOST pointers for actor_load, DEVICE pointers for actor_load_device. */
 typedef struct {
   const float *dense1_w, *dense1_b;               /* [64][D], [64]    */
   const float *w_ih, *w_hh, *b_ih, *b_hh;         /* [128][64], [128][32], [128], [128] */
@@ -180,8 +181,18 @@ typedef struct {
 
 int actor_create(const ActorConfig *cfg, MpeActor **out);
 int actor_destroy(MpeActor *actor);
-/* actor.load_state_dict(...) - rls/agent/multiagent/ddpg_gumbel_fix.py:231-241 */
+/* actor.load_state_dict(...) - rls/agent/multiagent/ddpg_gumbel_fix.py:231-241 - from HOST arrays: copies them to
+ * the device, packs the weight images on `stream` and synchronises it; the arrays may be reused when it returns. */
 int actor_load(MpeActor *actor, const ActorWeights *w, void *stream);
+/* The same load from DEVICE tensors (a learner's parameters), enqueued on `stream` as one pack kernel: no host
+ * synchronisation and no allocation, so it can be captured in a CUDA graph.  The tensors are read when the kernel
+ * runs, not when the call returns: they must stay allocated until then, and a change made to them earlier on `stream`
+ * is what gets loaded.  Ordering: actor launches on `stream` after this call see the new weights, launches enqueued
+ * before it the old ones.  The weights are overwritten in place, so launches on OTHER streams (HostRollout shards
+ * sharing this actor, for example) must be ordered against the load by the caller with events.  MPE_EINVAL before
+ * anything is launched for a missing tensor (the rules of actor_load) or a pointer that is not device or managed
+ * memory on the actor's device. */
+int actor_load_device(MpeActor *actor, const ActorWeights *w, void *stream);
 
 /* Implementation of the actor GEMMs: 0 = auto (tensor cores where supported), 1 = fp32 SIMT (FFMA),
  * 2 = tcgen05 tensor cores with fp16 hi/lo split operands (fp32-level accuracy; 2/3/4/6/8/9/12 agents).
@@ -224,7 +235,8 @@ typedef struct {
   int32_t relu_attention;   /* 1: relu on the attention output (ac_network_multi_gumbel.py:141), 0: "+model" critic */
   int32_t device;
 } CriticConfig;
-/* HOST pointers to fp32 tensors in the reference's state_dict layout (row-major [out][in]). */
+/* Pointers to fp32 tensors in the reference's state_dict layout (row-major [out][in], contiguous, 4 B alignment
+ * suffices): HOST pointers for critic_load, DEVICE pointers for critic_load_device. */
 typedef struct {
   const float *dense1_w, *dense1_b;        /* [64][D + act_dim], [64]                    */
   const float *w_ih, *w_hh, *b_ih, *b_hh;  /* lstm.*_l0: [256][64], [256][64], [256], [256] */
@@ -233,7 +245,12 @@ typedef struct {
 } CriticWeights;
 int critic_create(const CriticConfig *cfg, MpeCritic **out);
 int critic_destroy(MpeCritic *critic);
+/* From HOST arrays, like actor_load: copy, pack on `stream`, synchronise. */
 int critic_load(MpeCritic *critic, const CriticWeights *w, void *stream);
+/* From DEVICE tensors, like actor_load_device: one pack kernel on `stream`, no host synchronisation, no allocation;
+ * critic launches on `stream` after the call see the new weights, launches on other streams are ordered by the caller.
+ * MPE_EINVAL before any launch for a missing tensor or a pointer that is not device memory on the critic's device. */
+int critic_load_device(MpeCritic *critic, const CriticWeights *w, void *stream);
 /* critic.forward(obs, action): obs [B][N][D], action [B][N][act_dim] fp32 (one-hot or soft; two heads concatenated
  * like ac_network_multi_gumbel.py:131-132) -> q [B][out_dim] and, for the "+model" critic, r [B][out_dim] (or NULL). */
 int critic_forward(MpeCritic *critic, const float *obs, const float *action, int64_t B, int32_t N, float *q, float *r,

@@ -7,7 +7,7 @@ import os
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get('MPE_B200_LIB', os.path.join(HERE, 'libmpe_b200.so'))  # override: A/B builds
-ABI_VERSION = 5
+ABI_VERSION = 6
 
 MPE_OK, MPE_EINVAL, MPE_ECUDA, MPE_EUNSUPPORTED = 0, -1, -2, -3
 SCENARIO_IDS = {'simple_spread': 0, 'simple_reference': 1, 'simple_speaker_listener': 2, 'fullobs_collect_treasure': 3}
@@ -88,6 +88,7 @@ SIGNATURES = {
     'actor_create': (C.c_int, [C.POINTER(ActorConfig), C.POINTER(P)]),
     'actor_destroy': (C.c_int, [P]),
     'actor_load': (C.c_int, [P, C.POINTER(ActorWeights), P]),
+    'actor_load_device': (C.c_int, [P, C.POINTER(ActorWeights), P]),
     'actor_set_impl': (C.c_int, [P, C.c_int32]),
     'actor_forward': (C.c_int, [P, P, C.c_int64, C.c_int32, P, C.c_uint64, C.c_uint64, C.c_int64, P, P, P, P, P, P]),
     'actor_forward_host': (C.c_int, [P, P, C.c_int64, C.c_int32, C.c_uint64, C.c_uint64, C.c_int64, P, P, P, P]),
@@ -95,6 +96,7 @@ SIGNATURES = {
     'critic_create': (C.c_int, [C.POINTER(CriticConfig), C.POINTER(P)]),
     'critic_destroy': (C.c_int, [P]),
     'critic_load': (C.c_int, [P, C.POINTER(CriticWeights), P]),
+    'critic_load_device': (C.c_int, [P, C.POINTER(CriticWeights), P]),
     'critic_forward': (C.c_int, [P, P, P, C.c_int64, C.c_int32, P, P, P]),
     'replay_create': (C.c_int, [C.POINTER(ReplayConfig), C.POINTER(P)]),
     'replay_destroy': (C.c_int, [P]),
@@ -143,6 +145,38 @@ def ptr(t):
     if hasattr(t, 'data_ptr'):
         return C.c_void_p(t.data_ptr())
     return C.c_void_p(t.ctypes.data)
+
+
+def np32(v):
+    """A C-contiguous float32 numpy copy (or view) of a torch tensor, numpy array or nested list."""
+    import numpy as np
+    import torch
+    if isinstance(v, torch.Tensor):
+        v = v.detach().to('cpu', torch.float32).numpy()
+    return np.ascontiguousarray(np.asarray(v, dtype=np.float32))
+
+
+def weights(cls, sd, names, shapes, device):
+    """Fill a weight struct (``ActorWeights`` / ``CriticWeights``) from the state_dict ``sd``.
+
+    ``names``: (struct field, state_dict key) pairs; ``shapes``: field -> the shape the handle's layout expects.
+    When every entry is a CUDA tensor on ``device`` the struct holds device pointers for ``*_load_device``
+    (``.to(float32).contiguous()``, a no-op for a learner's parameters); otherwise host pointers to float32 copies for
+    ``*_load``.  Returns ``(struct, keep, on_device)``, where ``keep`` owns the memory the pointers refer to.
+    KeyError for a missing key and ValueError for a wrong shape, both before anything is launched."""
+    import torch
+    for _, key in names:
+        if key not in sd:
+            raise KeyError('state_dict is missing %r' % key)
+    vals = [sd[key] for _, key in names]
+    on_device = all(isinstance(v, torch.Tensor) and v.device == device for v in vals)
+    keep = [v.detach().to(torch.float32).contiguous() if on_device else np32(v) for v in vals]
+    w = cls()
+    for (field, key), a in zip(names, keep):
+        if tuple(a.shape) != tuple(shapes[field]):
+            raise ValueError('%r has shape %s, expected %s' % (key, tuple(a.shape), tuple(shapes[field])))
+        setattr(w, field, a.data_ptr() if on_device else a.ctypes.data)
+    return w, keep, on_device
 
 
 def current_stream(device):

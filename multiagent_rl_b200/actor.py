@@ -21,12 +21,6 @@ _KEYS = [('dense1_w', 'dense1.module.weight'), ('dense1_b', 'dense1.module.bias'
          ('b_ih_r', 'bilstm.bias_ih_l0_reverse'), ('b_hh_r', 'bilstm.bias_hh_l0_reverse')]
 
 
-def _np32(v):
-    if isinstance(v, torch.Tensor):
-        v = v.detach().to('cpu', torch.float32).numpy()
-    return np.ascontiguousarray(np.asarray(v, dtype=np.float32))
-
-
 class FusedActor(object):
     """Device-resident copy of an ActorNetwork's weights + the fused forward/sample kernel.
 
@@ -43,7 +37,7 @@ class FusedActor(object):
         if self.device.index is None:
             self.device = torch.device('cuda', torch.cuda.current_device())
         sd = dict(state_dict)
-        self.obs_dim = int(_np32(sd['dense1.module.weight']).shape[1])
+        self.obs_dim = int(_lib.np32(sd['dense1.module.weight']).shape[1])
         self.multi = 'dense2_1.module.weight' in sd
         if self.multi:
             self.act_dims = [int(sd['dense2_1.module.weight'].shape[0]), int(sd['dense2_2.module.weight'].shape[0])]
@@ -73,24 +67,33 @@ class FusedActor(object):
         self.impl = impl
 
     def load_state_dict(self, sd):
-        """``actor.load_state_dict`` (rls/agent/multiagent/ddpg_gumbel_fix.py:231-241)."""
-        keep = []
-        w = _lib.ActorWeights()
+        """``actor.load_state_dict`` (rls/agent/multiagent/ddpg_gumbel_fix.py:231-241).
+
+        CUDA tensors on the actor's device - a learner's ``state_dict()`` - are packed by one kernel on torch's current
+        stream, without a host synchronisation: forwards and rollouts enqueued on that stream afterwards see the new
+        weights, and in-place changes made to the tensors earlier on it are what gets loaded.  The weights are
+        overwritten in place, so work on other streams that uses this actor must be ordered with events.  Anything
+        else (numpy arrays, CPU tensors, another device) is read on the host; the call returns when it has been
+        loaded.  KeyError for a missing key, ValueError for a tensor of the wrong shape."""
+        H = 64
         names = list(_KEYS)
+        shapes = {'dense1_w': (H, self.obs_dim), 'dense1_b': (H,)}
+        for d in ('', '_r'):
+            shapes.update({'w_ih' + d: (4 * 32, H), 'w_hh' + d: (4 * 32, 32), 'b_ih' + d: (4 * 32,), 'b_hh' + d: (4 * 32,)})
         if self.multi:
             names += [('dense2_w', 'dense2_1.module.weight'), ('dense2_b', 'dense2_1.module.bias'),
                       ('dense2b_w', 'dense2_2.module.weight'), ('dense2b_b', 'dense2_2.module.bias')]
+            shapes.update({'dense2b_w': (self.act_dims[1], H), 'dense2b_b': (self.act_dims[1],)})
         else:
             names += [('dense2_w', 'dense2.module.weight'), ('dense2_b', 'dense2.module.bias')]
+        shapes.update({'dense2_w': (self.act_dims[0], H), 'dense2_b': (self.act_dims[0],)})
         if self.has_model:
             names += [('dense3_w', 'dense3.module.weight'), ('dense3_b', 'dense3.module.bias')]
-        for field, key in names:
-            if key not in sd:
-                raise KeyError('state_dict is missing %r' % key)
-            arr = _np32(sd[key])
-            keep.append(arr)
-            setattr(w, field, arr.ctypes.data)
-        _lib.check(self._lib.actor_load(self._h, C.byref(w), _lib.current_stream(self.device)), 'actor_load')
+            shapes.update({'dense3_w': (self.obs_dim, H), 'dense3_b': (self.obs_dim,)})
+        w, keep, on_device = _lib.weights(_lib.ActorWeights, sd, names, shapes, self.device)
+        fn = 'actor_load_device' if on_device else 'actor_load'
+        _lib.check(getattr(self._lib, fn)(self._h, C.byref(w), _lib.current_stream(self.device)), fn)
+        del keep  # the host path has copied the arrays; device tensors are released in stream order by torch
 
     # ------------------------------------------------------------------ device tensors
     def forward(self, obs, gumbel=None, step=0, env_id_offset=0, want_logits=False, want_onehot=False,
@@ -149,6 +152,7 @@ class FusedActingMixin(object):
             self._fused = FusedActor(self.actor.state_dict(), device=dev if dev.type == 'cuda' else None,
                                      seed=getattr(self, 'sample_seed', torch.initial_seed() & (2 ** 63 - 1)))
         elif v != self._fused_version:  # optimize() stepped the actor (ddpg_gumbel_fix.py:196-199)
+            # a CUDA actor reloads on the device, in stream order after the update (no host round trip)
             self._fused.load_state_dict(self.actor.state_dict())
         self._fused_version = v
         return self._fused

@@ -7,7 +7,6 @@ as is).  Acting never calls the critic; ``Trainer.optimize()`` (autograd, out of
 """
 import ctypes as C
 
-import numpy as np
 import torch
 
 from . import _lib
@@ -15,12 +14,6 @@ from . import _lib
 _KEYS = [('dense1_w', 'dense1.module.weight'), ('dense1_b', 'dense1.module.bias'),
          ('w_ih', 'lstm.weight_ih_l0'), ('w_hh', 'lstm.weight_hh_l0'), ('b_ih', 'lstm.bias_ih_l0'),
          ('b_hh', 'lstm.bias_hh_l0'), ('dense2_w', 'dense2.weight'), ('dense2_b', 'dense2.bias')]
-
-
-def _np32(v):
-    if isinstance(v, torch.Tensor):
-        v = v.detach().to('cpu', torch.float32).numpy()
-    return np.ascontiguousarray(np.asarray(v, dtype=np.float32))
 
 
 class FusedCritic(object):
@@ -35,9 +28,9 @@ class FusedCritic(object):
         if self.device.index is None:
             self.device = torch.device('cuda', torch.cuda.current_device())
         sd = dict(state_dict)
-        din = int(_np32(sd['dense1.module.weight']).shape[1])
+        din = int(_lib.np32(sd['dense1.module.weight']).shape[1])
         self.obs_dim, self.act_dim = int(obs_dim), din - int(obs_dim)
-        self.out_dim = int(_np32(sd['dense2.weight']).shape[0])
+        self.out_dim = int(_lib.np32(sd['dense2.weight']).shape[0])
         self.model = 'dense3.weight' in sd
         cfg = _lib.CriticConfig(obs_dim=self.obs_dim, act_dim=self.act_dim, out_dim=self.out_dim,
                                 has_reward_head=1 if self.model else 0, relu_attention=0 if self.model else 1,
@@ -54,15 +47,19 @@ class FusedCritic(object):
             self._h = None
 
     def load_state_dict(self, sd):
-        keep, w = [], _lib.CriticWeights()
+        """``critic.load_state_dict``.  CUDA tensors on the critic's device are packed by one kernel on torch's current
+        stream without a host synchronisation (critic forwards enqueued on that stream afterwards see the new weights;
+        other streams are ordered by the caller); anything else is read on the host.  KeyError for a missing key,
+        ValueError for a tensor of the wrong shape."""
+        H, G = 64, 256
         names = list(_KEYS) + ([('dense3_w', 'dense3.weight'), ('dense3_b', 'dense3.bias')] if self.model else [])
-        for field, key in names:
-            if key not in sd:
-                raise KeyError('state_dict is missing %r' % key)
-            arr = _np32(sd[key])
-            keep.append(arr)
-            setattr(w, field, arr.ctypes.data)
-        _lib.check(self._lib.critic_load(self._h, C.byref(w), _lib.current_stream(self.device)), 'critic_load')
+        shapes = {'dense1_w': (H, self.obs_dim + self.act_dim), 'dense1_b': (H,), 'w_ih': (G, H), 'w_hh': (G, H),
+                  'b_ih': (G,), 'b_hh': (G,), 'dense2_w': (self.out_dim, H), 'dense2_b': (self.out_dim,),
+                  'dense3_w': (self.out_dim, H), 'dense3_b': (self.out_dim,)}
+        w, keep, on_device = _lib.weights(_lib.CriticWeights, sd, names, shapes, self.device)
+        fn = 'critic_load_device' if on_device else 'critic_load'
+        _lib.check(getattr(self._lib, fn)(self._h, C.byref(w), _lib.current_stream(self.device)), fn)
+        del keep
 
     def forward(self, obs, action):
         obs = torch.as_tensor(obs, dtype=torch.float32, device=self.device).contiguous()

@@ -14,7 +14,6 @@
 // 16 unit-groups x 8 row-groups; a thread owns RT rows x (4 gates x 2 units) = RT x 8 accumulators and
 // the cell state of those (row, unit) pairs for the whole sequence, so c never leaves registers.
 #include <cmath>
-#include <cstring>
 
 #include "actor_launch.h"
 #include "common.cuh"
@@ -25,7 +24,7 @@ namespace mpe {
 constexpr int kActorThreads = 256;
 
 // ------------------------------------------------------------------------------------------------
-// host: blob layout + packing
+// host: blob layout (packed by pack_kernels.cu)
 // ------------------------------------------------------------------------------------------------
 static int round_up(int x, int m) { return (x + m - 1) / m * m; }
 
@@ -47,43 +46,6 @@ void actor_layout(int D, int A0, int A1, bool has_model, ActorDev *o) {
   o->off_w3 = off; off += has_model ? kHid * o->Dpad : 0;
   o->off_b3 = off; off += has_model ? o->Dpad : 0;
   o->blob_floats = (size_t)round_up(off, 32);
-}
-
-// reference gate row (gate*32 + unit) -> packed column; unit = ug + 16*uu
-static int packed_col(int gate, int unit) {
-  const int ug = unit & 15, uu = unit >> 4;
-  return ug * 8 + gate * 2 + uu;
-}
-
-void actor_pack(const ActorDev &d, const ActorHostWeights &w, float *blob) {
-  std::memset(blob, 0, d.blob_floats * sizeof(float));
-  const float *wih[2] = {w.w_ih, w.w_ih_r}, *whh[2] = {w.w_hh, w.w_hh_r};
-  const float *bih[2] = {w.b_ih, w.b_ih_r}, *bhh[2] = {w.b_hh, w.b_hh_r};
-  for (int dir = 0; dir < 2; ++dir) {
-    float *wg = blob + d.off_wg[dir];
-    for (int gate = 0; gate < 4; ++gate)
-      for (int unit = 0; unit < kH; ++unit) {
-        const int row = gate * kH + unit, col = packed_col(gate, unit);
-        for (int k = 0; k < kHid; ++k) wg[k * kGateN + col] = wih[dir][row * kHid + k];
-        for (int k = 0; k < kH; ++k) wg[(kHid + k) * kGateN + col] = whh[dir][row * kH + k];
-        blob[d.off_bg + dir * kGateN + col] = bih[dir][row] + bhh[dir][row];
-      }
-  }
-  for (int j = 0; j < kHid; ++j) {
-    for (int k = 0; k < d.D; ++k) blob[d.off_w1 + k * kHid + j] = w.dense1_w[j * d.D + k];
-    blob[d.off_b1 + j] = w.dense1_b[j];
-  }
-  for (int a = 0; a < d.A; ++a) {
-    const float *src = a < d.A0 ? w.dense2_w + a * kHid : w.dense2b_w + (a - d.A0) * kHid;
-    for (int k = 0; k < kHid; ++k) blob[d.off_w2 + k * d.Apad + a] = src[k];
-    blob[d.off_b2 + a] = a < d.A0 ? w.dense2_b[a] : w.dense2b_b[a - d.A0];
-  }
-  if (d.has_model) {
-    for (int j = 0; j < d.D; ++j) {
-      for (int k = 0; k < kHid; ++k) blob[d.off_w3 + k * d.Dpad + j] = w.dense3_w[j * kHid + k];
-      blob[d.off_b3 + j] = w.dense3_b[j];
-    }
-  }
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "../../include/mpe_b200.h"
 #include "env_launch.h"
 
 namespace mpe {
@@ -46,11 +47,6 @@ struct ActorDev {
   int off_b3 = 0;          // [Dpad]
 };
 
-struct ActorHostWeights {
-  const float *dense1_w, *dense1_b, *w_ih, *w_hh, *b_ih, *b_hh, *w_ih_r, *w_hh_r, *b_ih_r, *b_hh_r;
-  const float *dense2_w, *dense2_b, *dense2b_w, *dense2b_b, *dense3_w, *dense3_b;
-};
-
 struct ActorIO {
   const float *obs = nullptr;     // [B][N][D]
   const float *gumbel = nullptr;  // [B][N][A] or null (Philox)
@@ -73,18 +69,19 @@ struct RolloutIO {
 };
 
 void actor_layout(int D, int A0, int A1, bool has_model, ActorDev *out);
-void actor_pack(const ActorDev &d, const ActorHostWeights &w, float *host_blob);
 bool actor_supported(int N);
 bool rollout_supported(int scenario, int N);
 cudaError_t launch_actor_forward(const ActorDev &w, const ActorIO &io, cudaStream_t st);
 // tensor-core path (tc_kernels.cu)
 void tc_layout(int D, int A0, int A1, TcDev *out);
-void tc_pack(const TcDev &t, const ActorHostWeights &w, unsigned char *host_image);
 bool tc_actor_supported(const TcDev &w, int N);
 bool tc_rollout_supported(const TcDev &w, int N);
 size_t tc_scratch_floats(int sm_count);
 cudaError_t launch_actor_forward_tc(const TcDev &w, const ActorIO &io, cudaStream_t st);
 cudaError_t launch_rollout_tc(const EnvStateAny &env, const TcDev &w, const RolloutIO &io, cudaStream_t st);
+// Packs the actor's images from DEVICE pointers to the reference's tensors (pack_kernels.cu): d.blob always, d.tc.blob
+// when d.tc.Kx > 0.  dense2b_* are read only when A1 > 0, dense3_* only with the model head.
+cudaError_t launch_actor_pack(const ActorDev &d, const ActorWeights &src, cudaStream_t st);
 // next_state = dense3(hcat): the "+model" head (ac_network_model_multi_gumbel.py:49,65) on top of the tensor-core forward
 cudaError_t launch_dense3(const ActorDev &w, const float *hcat, int64_t rows, float *next_state, cudaStream_t st);
 

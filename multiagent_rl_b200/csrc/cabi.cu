@@ -87,6 +87,7 @@ struct ActorMirror {
 struct MpeActor {
   mpe::ActorDev dev;
   int device = 0;
+  float *stage = nullptr;  // actor_load: device copy of the caller's host tensors, read by the pack kernel
   ActorMirror mirror;
   float *hcat = nullptr;  // [rows][64] relu(BiLSTM output) between the tensor-core forward and the dense3 head
   int64_t hcat_rows = 0;
@@ -95,6 +96,7 @@ struct MpeActor {
 struct MpeCritic {
   mpe::CriticDev dev;
   int device = 0;
+  float *stage = nullptr;  // critic_load: device copy of the caller's host tensors, read by the pack kernel
 };
 
 struct MpeReplay {
@@ -133,6 +135,47 @@ static cudaError_t launch_actor(const MpeActor *a, const mpe::ActorIO &io, float
   mpe::TcDev tc;
   cudaError_t e = tc_for_stream(a, io.N, stream_scratch, &tc);
   return e != cudaSuccess ? e : mpe::launch_actor_forward_tc(tc, io, st);
+}
+
+// The weight structs field by field, with the element count of the reference tensor behind each field for a handle
+// (0: the handle does not read that field).
+constexpr int kActorFields = 16, kCriticFields = 10;
+static const float *ActorWeights::*const kActorField[kActorFields] = {
+    &ActorWeights::dense1_w, &ActorWeights::dense1_b, &ActorWeights::w_ih,     &ActorWeights::w_hh,
+    &ActorWeights::b_ih,     &ActorWeights::b_hh,     &ActorWeights::w_ih_r,   &ActorWeights::w_hh_r,
+    &ActorWeights::b_ih_r,   &ActorWeights::b_hh_r,   &ActorWeights::dense2_w, &ActorWeights::dense2_b,
+    &ActorWeights::dense2b_w, &ActorWeights::dense2b_b, &ActorWeights::dense3_w, &ActorWeights::dense3_b};
+static const float *CriticWeights::*const kCriticField[kCriticFields] = {
+    &CriticWeights::dense1_w, &CriticWeights::dense1_b, &CriticWeights::w_ih,     &CriticWeights::w_hh,
+    &CriticWeights::b_ih,     &CriticWeights::b_hh,     &CriticWeights::dense2_w, &CriticWeights::dense2_b,
+    &CriticWeights::dense3_w, &CriticWeights::dense3_b};
+
+static void actor_counts(const mpe::ActorDev &d, size_t (&n)[kActorFields]) {
+  const size_t H = mpe::kHid, G = mpe::kGateN, D = d.D, A0 = d.A0, A1 = d.A1, M = d.has_model ? 1 : 0;
+  const size_t c[kActorFields] = {H * D, H, G * H, G * mpe::kH, G, G, G * H, G * mpe::kH, G, G,
+                                  A0 * H, A0, A1 * H, A1, M * D * H, M * D};
+  for (int f = 0; f < kActorFields; ++f) n[f] = c[f];
+}
+static void critic_counts(const mpe::CriticDev &d, size_t (&n)[kCriticFields]) {
+  const size_t H = mpe::kCriticH, G = 4 * mpe::kCriticH, Din = d.Din, O = d.out, R = d.has_r ? 1 : 0;
+  const size_t c[kCriticFields] = {H * Din, H, G * H, G * H, G, G, O * H, O, R * O * H, R * O};
+  for (int f = 0; f < kCriticFields; ++f) n[f] = c[f];
+}
+template <int F>
+static size_t total(const size_t (&n)[F]) {
+  size_t t = 0;
+  for (int f = 0; f < F; ++f) t += n[f];
+  return t;
+}
+
+// Device or managed memory of `device`.  A host pointer - pageable, pinned or registered - is refused.
+static bool device_memory(const void *p, int device) {
+  cudaPointerAttributes at;
+  if (cudaPointerGetAttributes(&at, p) != cudaSuccess) {
+    cudaGetLastError();  // not a pointer the runtime knows: do not leave the error for the caller's next check
+    return false;
+  }
+  return (at.type == cudaMemoryTypeDevice || at.type == cudaMemoryTypeManaged) && at.device == device;
 }
 
 // device mirrors of the mpe_*_host entry points, allocated on first use
@@ -391,6 +434,9 @@ int actor_create(const ActorConfig *cfg, MpeActor **out) {
   if (e == cudaSuccess) e = cudaMalloc(&a->dev.tc.blob, a->dev.tc.bytes);
   if (e == cudaSuccess) e = cudaMemset(a->dev.tc.blob, 0, a->dev.tc.bytes);
   if (e == cudaSuccess) e = ensure_tc_scratch(&a->dev.tc.scratch, cfg->device);
+  size_t n[kActorFields];
+  actor_counts(a->dev, n);
+  if (e == cudaSuccess) e = cudaMalloc(&a->stage, total(n) * sizeof(float));
   if (e != cudaSuccess) {
     actor_destroy(a);  // frees whatever was allocated before the failure
     return fail_cuda(e, "actor_create: cudaMalloc");
@@ -403,7 +449,7 @@ int actor_destroy(MpeActor *a) {
   if (a == nullptr) return MPE_OK;
   DeviceGuard g(a->device);
   cudaDeviceSynchronize();
-  void *ptrs[] = {a->dev.blob, a->dev.tc.blob, a->dev.tc.scratch, a->hcat};
+  void *ptrs[] = {a->dev.blob, a->dev.tc.blob, a->dev.tc.scratch, a->hcat, a->stage};
   for (void *p : ptrs)
     if (p != nullptr) cudaFree(p);
   const ActorMirror &m = a->mirror;
@@ -414,35 +460,51 @@ int actor_destroy(MpeActor *a) {
   return MPE_OK;
 }
 
-int actor_load(MpeActor *a, const ActorWeights *w, void *stream) {
-  if (a == nullptr || w == nullptr) return fail(MPE_EINVAL, "actor_load: null argument");
+static int check_actor_weights(const MpeActor *a, const ActorWeights *w, const char *who) {
+  const std::string n(who);
+  if (a == nullptr || w == nullptr) return fail(MPE_EINVAL, n + ": null argument");
   if (!w->dense1_w || !w->dense1_b || !w->w_ih || !w->w_hh || !w->b_ih || !w->b_hh || !w->w_ih_r || !w->w_hh_r ||
       !w->b_ih_r || !w->b_hh_r || !w->dense2_w || !w->dense2_b)
-    return fail(MPE_EINVAL, "actor_load: missing tensor");
-  if (a->dev.A1 > 0 && (!w->dense2b_w || !w->dense2b_b)) return fail(MPE_EINVAL, "actor_load: missing dense2_2");
-  if (a->dev.has_model && (!w->dense3_w || !w->dense3_b)) return fail(MPE_EINVAL, "actor_load: missing dense3");
+    return fail(MPE_EINVAL, n + ": missing tensor");
+  if (a->dev.A1 > 0 && (!w->dense2b_w || !w->dense2b_b)) return fail(MPE_EINVAL, n + ": missing dense2_2");
+  if (a->dev.has_model && (!w->dense3_w || !w->dense3_b)) return fail(MPE_EINVAL, n + ": missing dense3");
+  return MPE_OK;
+}
+
+// The host tensors are copied into the handle's staging buffer and packed by the same kernel as actor_load_device;
+// the synchronise frees both the caller's arrays and the staging buffer.
+int actor_load(MpeActor *a, const ActorWeights *w, void *stream) {
+  if (int rc = check_actor_weights(a, w, "actor_load")) return rc;
   DeviceGuard g(a->device);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  float *host = nullptr;
-  CK(cudaMallocHost(&host, a->dev.blob_floats * sizeof(float)));
-  mpe::ActorHostWeights hw = {w->dense1_w, w->dense1_b, w->w_ih,     w->w_hh,     w->b_ih,      w->b_hh,
-                              w->w_ih_r,   w->w_hh_r,   w->b_ih_r,   w->b_hh_r,   w->dense2_w,  w->dense2_b,
-                              w->dense2b_w, w->dense2b_b, w->dense3_w, w->dense3_b};
-  mpe::actor_pack(a->dev, hw, host);
-  cudaError_t e = cudaMemcpyAsync(a->dev.blob, host, a->dev.blob_floats * sizeof(float), cudaMemcpyHostToDevice, st);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(st);  // the pinned staging buffer is freed below
-  cudaFreeHost(host);
-  if (e == cudaSuccess) {  // fp16 hi/lo image of the tensor-core path
-    unsigned char *img = nullptr;
-    e = cudaMallocHost(&img, a->dev.tc.bytes);
-    if (e == cudaSuccess) {
-      mpe::tc_pack(a->dev.tc, hw, img);
-      e = cudaMemcpyAsync(a->dev.tc.blob, img, a->dev.tc.bytes, cudaMemcpyHostToDevice, st);
-      if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-      cudaFreeHost(img);
-    }
+  size_t n[kActorFields];
+  actor_counts(a->dev, n);
+  ActorWeights staged = {};
+  float *p = a->stage;
+  for (int f = 0; f < kActorFields; ++f) {
+    if (n[f] == 0) continue;
+    CK(cudaMemcpyAsync(p, w->*kActorField[f], n[f] * sizeof(float), cudaMemcpyHostToDevice, st));
+    staged.*kActorField[f] = p;
+    p += n[f];
   }
-  if (e != cudaSuccess) return fail_cuda(e, "actor_load: upload");
+  CK(mpe::launch_actor_pack(a->dev, staged, st));
+  CK(cudaStreamSynchronize(st));
+  return MPE_OK;
+}
+
+int actor_load_device(MpeActor *a, const ActorWeights *w, void *stream) {
+  if (int rc = check_actor_weights(a, w, "actor_load_device")) return rc;
+  size_t n[kActorFields];
+  actor_counts(a->dev, n);
+  ActorWeights src = {};  // the fields this actor reads; the rest stay NULL
+  for (int f = 0; f < kActorFields; ++f) {
+    if (n[f] == 0) continue;
+    if (!device_memory(w->*kActorField[f], a->device))
+      return fail(MPE_EINVAL, "actor_load_device: a weight pointer is not device memory on the actor's device");
+    src.*kActorField[f] = w->*kActorField[f];
+  }
+  DeviceGuard g(a->device);
+  CK(mpe::launch_actor_pack(a->dev, src, static_cast<cudaStream_t>(stream)));
   return MPE_OK;
 }
 
@@ -797,6 +859,9 @@ int critic_create(const CriticConfig *cfg, MpeCritic **out) {
   mpe::critic_layout(cfg->obs_dim, cfg->act_dim, cfg->out_dim, cfg->has_reward_head != 0, cfg->relu_attention != 0, &c->dev);
   cudaError_t e = cudaMalloc(&c->dev.blob, c->dev.blob_floats * sizeof(float));
   if (e == cudaSuccess) e = cudaMemset(c->dev.blob, 0, c->dev.blob_floats * sizeof(float));
+  size_t n[kCriticFields];
+  critic_counts(c->dev, n);
+  if (e == cudaSuccess) e = cudaMalloc(&c->stage, total(n) * sizeof(float));
   if (e != cudaSuccess) {
     critic_destroy(c);
     return fail_cuda(e, "critic_create: cudaMalloc");
@@ -810,26 +875,53 @@ int critic_destroy(MpeCritic *c) {
   DeviceGuard g(c->device);
   cudaDeviceSynchronize();
   if (c->dev.blob != nullptr) cudaFree(c->dev.blob);
+  if (c->stage != nullptr) cudaFree(c->stage);
   delete c;
   return MPE_OK;
 }
 
-int critic_load(MpeCritic *c, const CriticWeights *w, void *stream) {
-  if (c == nullptr || w == nullptr) return fail(MPE_EINVAL, "critic_load: null argument");
+static int check_critic_weights(const MpeCritic *c, const CriticWeights *w, const char *who) {
+  const std::string n(who);
+  if (c == nullptr || w == nullptr) return fail(MPE_EINVAL, n + ": null argument");
   if (!w->dense1_w || !w->dense1_b || !w->w_ih || !w->w_hh || !w->b_ih || !w->b_hh || !w->dense2_w || !w->dense2_b)
-    return fail(MPE_EINVAL, "critic_load: missing tensor");
-  if (c->dev.has_r && (!w->dense3_w || !w->dense3_b)) return fail(MPE_EINVAL, "critic_load: missing dense3");
+    return fail(MPE_EINVAL, n + ": missing tensor");
+  if (c->dev.has_r && (!w->dense3_w || !w->dense3_b)) return fail(MPE_EINVAL, n + ": missing dense3");
+  return MPE_OK;
+}
+
+// Same scheme as actor_load: staged copy of the host tensors, the pack kernel, one synchronise.
+int critic_load(MpeCritic *c, const CriticWeights *w, void *stream) {
+  if (int rc = check_critic_weights(c, w, "critic_load")) return rc;
   DeviceGuard g(c->device);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  float *host = nullptr;
-  CK(cudaMallocHost(&host, c->dev.blob_floats * sizeof(float)));
-  mpe::CriticHostWeights hw = {w->dense1_w, w->dense1_b, w->w_ih, w->w_hh, w->b_ih, w->b_hh,
-                               w->dense2_w, w->dense2_b, w->dense3_w, w->dense3_b};
-  mpe::critic_pack(c->dev, hw, host);
-  cudaError_t e = cudaMemcpyAsync(c->dev.blob, host, c->dev.blob_floats * sizeof(float), cudaMemcpyHostToDevice, st);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(st);  // the pinned staging buffer is freed below
-  cudaFreeHost(host);
-  if (e != cudaSuccess) return fail_cuda(e, "critic_load: upload");
+  size_t n[kCriticFields];
+  critic_counts(c->dev, n);
+  CriticWeights staged = {};
+  float *p = c->stage;
+  for (int f = 0; f < kCriticFields; ++f) {
+    if (n[f] == 0) continue;
+    CK(cudaMemcpyAsync(p, w->*kCriticField[f], n[f] * sizeof(float), cudaMemcpyHostToDevice, st));
+    staged.*kCriticField[f] = p;
+    p += n[f];
+  }
+  CK(mpe::launch_critic_pack(c->dev, staged, st));
+  CK(cudaStreamSynchronize(st));
+  return MPE_OK;
+}
+
+int critic_load_device(MpeCritic *c, const CriticWeights *w, void *stream) {
+  if (int rc = check_critic_weights(c, w, "critic_load_device")) return rc;
+  size_t n[kCriticFields];
+  critic_counts(c->dev, n);
+  CriticWeights src = {};
+  for (int f = 0; f < kCriticFields; ++f) {
+    if (n[f] == 0) continue;
+    if (!device_memory(w->*kCriticField[f], c->device))
+      return fail(MPE_EINVAL, "critic_load_device: a weight pointer is not device memory on the critic's device");
+    src.*kCriticField[f] = w->*kCriticField[f];
+  }
+  DeviceGuard g(c->device);
+  CK(mpe::launch_critic_pack(c->dev, src, static_cast<cudaStream_t>(stream)));
   return MPE_OK;
 }
 

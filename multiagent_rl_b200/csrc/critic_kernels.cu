@@ -11,7 +11,6 @@
 // l + 32: its 8 gate pre-activations per step are one 32 B slice of a k-major weight row, x_t / h_{t-1} are broadcast
 // reads of the warp's staging row.  All arithmetic fp32 (FFMA), exp / tanh by the accurate libdevice forms.
 #include <cmath>
-#include <cstring>
 
 #include "common.cuh"
 #include "critic_launch.h"
@@ -38,34 +37,6 @@ void critic_layout(int D, int A, int out, bool has_r, bool relu_attn, CriticDev 
   o->off_w3 = off; off += kCriticH * kCriticMaxOut;
   o->off_b3 = off; off += kCriticMaxOut;
   o->blob_floats = (size_t)((off + 31) / 32 * 32);
-}
-
-// reference gate row (gate * 64 + unit) -> packed column: lane = unit & 31 owns [i0 i1 f0 f1 g0 g1 o0 o1], units (lane, lane + 32)
-static int packed_col(int gate, int unit) { return (unit & 31) * 8 + gate * 2 + (unit >> 5); }
-
-void critic_pack(const CriticDev &d, const CriticHostWeights &w, float *blob) {
-  std::memset(blob, 0, d.blob_floats * sizeof(float));
-  for (int gate = 0; gate < 4; ++gate)
-    for (int unit = 0; unit < kCriticH; ++unit) {
-      const int row = gate * kCriticH + unit, col = packed_col(gate, unit);
-      for (int k = 0; k < kCriticH; ++k) {
-        blob[d.off_wih + k * kGates + col] = w.w_ih[row * kCriticH + k];
-        blob[d.off_whh + k * kGates + col] = w.w_hh[row * kCriticH + k];
-      }
-      blob[d.off_bg + col] = w.b_ih[row] + w.b_hh[row];
-    }
-  for (int j = 0; j < kCriticH; ++j) {
-    for (int k = 0; k < d.Din; ++k) blob[d.off_w1 + k * kCriticH + j] = w.dense1_w[j * d.Din + k];
-    blob[d.off_b1 + j] = w.dense1_b[j];
-  }
-  for (int o = 0; o < d.out; ++o) {
-    for (int k = 0; k < kCriticH; ++k) {
-      blob[d.off_w2 + k * kCriticMaxOut + o] = w.dense2_w[o * kCriticH + k];
-      if (d.has_r) blob[d.off_w3 + k * kCriticMaxOut + o] = w.dense3_w[o * kCriticH + k];
-    }
-    blob[d.off_b2 + o] = w.dense2_b[o];
-    if (d.has_r) blob[d.off_b3 + o] = w.dense3_b[o];
-  }
 }
 
 __device__ __forceinline__ float sigmoid_acc(float x) { return 1.0f / (1.0f + expf(-x)); }

@@ -3,19 +3,14 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "../../include/mpe_b200.h"
+
 namespace mpe {
 
 constexpr int kCriticH = 64;        // dense1 width = LSTM input = LSTM hidden (ac_network_multi_gumbel.py:86-92)
 constexpr int kCriticMaxIn = 64;    // obs_dim + sum(action widths)
 constexpr int kCriticMaxAgents = 16;
 constexpr int kCriticMaxOut = 4;
-
-struct CriticHostWeights {
-  const float *dense1_w, *dense1_b;          // [64][Din], [64]
-  const float *w_ih, *w_hh, *b_ih, *b_hh;    // [256][64], [256][64], [256], [256]  (rows: i, f, g, o)
-  const float *dense2_w, *dense2_b;          // [out][64], [out]
-  const float *dense3_w, *dense3_b;          // [out][64], [out] or NULL
-};
 
 // Packed fp32 blob in device memory (what a CTA stages into shared memory with one bulk copy)
 struct CriticDev {
@@ -26,7 +21,8 @@ struct CriticDev {
 };
 
 void critic_layout(int D, int A, int out, bool has_r, bool relu_attn, CriticDev *o);
-void critic_pack(const CriticDev &d, const CriticHostWeights &w, float *host_blob);
+// Packs the blob from DEVICE pointers to the reference's tensors (pack_kernels.cu); dense3_* are read only when has_r.
+cudaError_t launch_critic_pack(const CriticDev &d, const CriticWeights &src, cudaStream_t st);
 // obs [B][N][D], action [B][N][A] (one-hot or soft), q / r [B][out]
 cudaError_t launch_critic_forward(const CriticDev &w, const float *obs, const float *action, int64_t B, int N, float *q,
                                   float *r, cudaStream_t st);

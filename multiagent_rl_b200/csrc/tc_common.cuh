@@ -15,6 +15,10 @@
 
 namespace mpe {
 
+// Weights are stored as 16 w (kWScale) so that the lo halves of the split stay normal fp16 values; the gate biases
+// are stored pre-multiplied by -log2(e) (-2 log2(e) for the cell gate): the argument form of ex2.
+constexpr float kWScale = 16.0f, kWInv = 0.0625f, kLog2e = 1.4426950408889634f;
+
 // ---- TMEM allocation (one full warp executes these) ----
 __device__ __forceinline__ void tmem_alloc(uint32_t *smem_slot, uint32_t ncols) {
   asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(smem_slot)),

@@ -10,11 +10,10 @@
 // logits to ~1e-6 so that the sampled index is bit-exact under identical noise; every fp32 operand x is
 // split as x = hi + lo (two fp16 values, 22 significant bits) and each product is three kind::f16 MMAs
 // (hi*hi + lo*hi + hi*lo) accumulated in fp32 in TMEM.  Weights are pre-split (and pre-scaled by 16 so
-// that the lo halves stay normal) on the host; activations are split by the epilogue that produces them.
+// that the lo halves stay normal) when they are loaded (pack_kernels.cu); activations are split by the epilogue that produces them.
 #include <cuda_fp16.h>
 
 #include <cstdlib>
-#include <cstring>
 
 #include "actor_launch.h"
 #include "env_core.cuh"
@@ -24,11 +23,10 @@
 namespace mpe {
 
 constexpr int kRows = 128;
-constexpr float kWScale = 16.0f, kWInv = 0.0625f, kLog2e = 1.4426950408889634f;
 constexpr uint32_t kChunkA = kRows * 16;  // bytes of one K-chunk (8 halves) of a 128-row A operand
 
 // ------------------------------------------------------------------------------------------------
-// host: fp16 hi/lo weight image
+// host: layout of the fp16 hi/lo weight image (packed by pack_kernels.cu)
 // ------------------------------------------------------------------------------------------------
 void tc_layout(int D, int A0, int A1, TcDev *o) {
   o->D = D; o->A0 = A0; o->A1 = A1; o->A = A0 + A1;
@@ -47,41 +45,6 @@ void tc_layout(int D, int A0, int A1, TcDev *o) {
 }
 
 bool tc_supported(const TcDev &t) { return t.Kx > 0 && t.A <= 16; }
-
-static void put_split(unsigned char *img, uint32_t off_hi, uint32_t off_lo, int rows, int n, int k, float v) {
-  const float x = v * kWScale;
-  const __half hi = __float2half_rn(x);
-  const __half lo = __float2half_rn(x - __half2float(hi));
-  const size_t idx = ((size_t)(k / 8) * rows + n) * 8 + (k % 8);
-  reinterpret_cast<__half *>(img + off_hi)[idx] = hi;
-  reinterpret_cast<__half *>(img + off_lo)[idx] = lo;
-}
-
-void tc_pack(const TcDev &t, const ActorHostWeights &w, unsigned char *img) {
-  std::memset(img, 0, t.bytes);
-  const float *wih[2] = {w.w_ih, w.w_ih_r}, *whh[2] = {w.w_hh, w.w_hh_r};
-  const float *bih[2] = {w.b_ih, w.b_ih_r}, *bhh[2] = {w.b_hh, w.b_hh_r};
-  float *bg = reinterpret_cast<float *>(img + t.off_bg);
-  for (int d = 0; d < 2; ++d)
-    for (int g = 0; g < 4; ++g)
-      for (int u = 0; u < kH; ++u) {
-        // packed gate column: per pair of units (a, b): [i_a i_b f_a f_b g_a g_b o_a o_b]
-        const int row = g * kH + u, n = (u >> 1) * 8 + g * 2 + (u & 1);
-        for (int k = 0; k < kHid; ++k) put_split(img, t.off_wih[d][0], t.off_wih[d][1], kGateN, n, k, wih[d][row * kHid + k]);
-        for (int k = 0; k < kH; ++k) put_split(img, t.off_whh[d][0], t.off_whh[d][1], kGateN, n, k, whh[d][row * kH + k]);
-        bg[d * kGateN + n] = (bih[d][row] + bhh[d][row]) * (g == 2 ? -2.0f : -1.0f) * kLog2e;  // ex2 argument form
-      }
-  float *b1 = reinterpret_cast<float *>(img + t.off_b1), *b2 = reinterpret_cast<float *>(img + t.off_b2);
-  for (int j = 0; j < kHid; ++j) {
-    for (int k = 0; k < t.D; ++k) put_split(img, t.off_w1[0], t.off_w1[1], kHid, j, k, w.dense1_w[j * t.D + k]);
-    b1[j] = w.dense1_b[j];
-  }
-  for (int a = 0; a < t.A; ++a) {
-    const float *src = a < t.A0 ? w.dense2_w + a * kHid : w.dense2b_w + (a - t.A0) * kHid;
-    for (int k = 0; k < kHid; ++k) reinterpret_cast<float *>(img + t.off_w2f)[k * 16 + a] = src[k];
-    b2[a] = a < t.A0 ? w.dense2_b[a] : w.dense2b_b[a - t.A0];
-  }
-}
 
 // ------------------------------------------------------------------------------------------------
 // device helpers

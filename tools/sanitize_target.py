@@ -92,5 +92,29 @@ for scen, n, B, cap in (('simple_spread', None, 129, 300), ('simple_reference', 
     env.reset(mask=(torch.arange(B, device='cuda') % 2).to(torch.uint8))
     env.rollout(actor, 4, replay=rb)
     rb.collect()
+# weight loads from CUDA tensors: every actor image layout (tensor-core image written, D > 32 where it is not, the
+# dense3 region past the staged blob), sources at 4 B-aligned offsets of one flat buffer; the critic with both heads
+for D, A, model in ((10, 5, False), (21, [5, 10], False), (28, 5, True), (57, 5, True)):
+    sd = random_state_dict(D, A, 4, model_head=model)
+    flat = torch.empty(1 + sum(v.size for v in sd.values()), device='cuda')
+    dev, off = {}, 1
+    for k, v in sd.items():
+        dev[k] = flat[off:off + v.size].view(v.shape)
+        dev[k].copy_(torch.from_numpy(v))
+        off += v.size
+    actor = m.FusedActor(random_state_dict(D, A, 5, model_head=model))
+    actor.load_state_dict(dev)
+    actor.forward(torch.zeros((33, 1 if D > 32 else 2, D), device='cuda'), want_next_state=model)
+for model in (False, True):
+    rng = np.random.RandomState(1)
+    csd = {'dense1.module.weight': rng.randn(64, 15), 'dense1.module.bias': rng.randn(64),
+           'lstm.weight_ih_l0': rng.randn(256, 64), 'lstm.weight_hh_l0': rng.randn(256, 64),
+           'lstm.bias_ih_l0': rng.randn(256), 'lstm.bias_hh_l0': rng.randn(256),
+           'dense2.weight': rng.randn(1, 64), 'dense2.bias': rng.randn(1)}
+    if model:
+        csd['dense3.weight'], csd['dense3.bias'] = rng.randn(1, 64), rng.randn(1)
+    critic = m.FusedCritic(csd, obs_dim=10)
+    critic.load_state_dict({k: torch.from_numpy(v).float().cuda() for k, v in csd.items()})
+    critic.forward(torch.zeros((17, 3, 10), device='cuda'), torch.zeros((17, 3, 5), device='cuda'))
 torch.cuda.synchronize()
 print('sanitize target done')
