@@ -35,7 +35,7 @@
 extern "C" {
 #endif
 
-#define MPE_ABI_VERSION 6
+#define MPE_ABI_VERSION 7
 
 enum { MPE_OK = 0, MPE_EINVAL = -1, MPE_ECUDA = -2, MPE_EUNSUPPORTED = -3 };
 enum { MPE_SIMPLE_SPREAD = 0, MPE_SIMPLE_REFERENCE = 1, MPE_SIMPLE_SPEAKER_LISTENER = 2,
@@ -255,6 +255,32 @@ int critic_load_device(MpeCritic *critic, const CriticWeights *w, void *stream);
  * like ac_network_multi_gumbel.py:131-132) -> q [B][out_dim] and, for the "+model" critic, r [B][out_dim] (or NULL). */
 int critic_forward(MpeCritic *critic, const float *obs, const float *action, int64_t B, int32_t N, float *q, float *r,
                    void *stream);
+/* Gradients of critic.forward for Trainer.optimize() (ddpg_gumbel_fix.py:131-219): the TD loss through the weights,
+ * the actor loss through the action.  Output tensors are fp32 in the reference's state_dict layout ([out][in]); a
+ * NULL field is not computed.  lstm.bias_ih_l0 and lstm.bias_hh_l0 get the same gradient. */
+typedef struct {
+  float *dense1_w, *dense1_b;        /* [64][D + act_dim], [64]                    */
+  float *w_ih, *w_hh, *b_ih, *b_hh;  /* lstm.*_l0: [256][64], [256][64], [256], [256] */
+  float *dense2_w, *dense2_b;        /* [out_dim][64], [out_dim]                   */
+  float *dense3_w, *dense3_b;        /* [out_dim][64], [out_dim]; reward head only */
+} CriticGrads;
+/* Bytes of device workspace critic_backward needs for B samples of N agents (0 for B = 0); < 0 (MPE_E*) on error. */
+int64_t critic_backward_workspace(MpeCritic *critic, int64_t B, int32_t N);
+/* Backward of critic_forward on the same obs [B][N][D] and action [B][N][act_dim], with the weights of the last
+ * critic_load* enqueued on `stream` (the forward is recomputed; nothing is kept from an earlier critic_forward).
+ * dq [B][out_dim] is the gradient of the loss with respect to q; dr [B][out_dim] that with respect to r, for the
+ * "+model" critic only, NULL meaning zero.  Outputs, each optional (NULL: not computed) and overwritten, never
+ * accumulated: dobs [B][N][D], daction [B][N][act_dim] and the fields of `grads` (which may itself be NULL).
+ * `workspace` is device memory of at least critic_backward_workspace(critic, B, N) bytes, borrowed like every buffer;
+ * calls on different streams need different workspaces.  Enqueued on `stream`: no host synchronisation, no
+ * allocation.  Deterministic: no floating-point atomics, every sum in an order that depends on B and N alone, and a
+ * sample's dobs / daction do not depend on where it sits in the batch.  MPE_EINVAL before any launch for a null
+ * critic / obs / action / dq / workspace, dr or dense3 gradients on a critic without a reward head, a workspace that is
+ * too small, B < 0, or a pointer that is not device memory on the critic's device; MPE_EUNSUPPORTED for N outside
+ * 1..16. */
+int critic_backward(MpeCritic *critic, const float *obs, const float *action, int64_t B, int32_t N, const float *dq,
+                    const float *dr, float *dobs, float *daction, const CriticGrads *grads, void *workspace,
+                    int64_t workspace_bytes, void *stream);
 
 /* ---- device-resident replay ring: rls/replay_buffer.py:9-91 (ReplayBuffer), fed with the tuple of
  * experiments/run.py:46,52 (obs_n, action_n_env, rew_shared = sum(rew_n), new_obs_n, float(done)) ---- */

@@ -12,11 +12,11 @@ Gumbel sampling) runs as hand-written sm_100a CUDA kernels in ``libmpe_b200.so``
 from .env import BatchedMultiAgentEnv, make_env  # noqa: F401
 from .actor import ActingTrainer, FusedActingMixin, FusedActor  # noqa: F401
 from .networks import ActorNetwork  # noqa: F401
-from .critic import FusedCritic  # noqa: F401
+from .critic import FusedCritic, FusedCriticNetwork  # noqa: F401
 from .replay import DeviceReplayBuffer  # noqa: F401
 from .history import EpisodeHistory  # noqa: F401
 from .hostpipe import HostRollout  # noqa: F401
 from . import distributed  # noqa: F401
 
 __all__ = ['make_env', 'BatchedMultiAgentEnv', 'FusedActor', 'FusedActingMixin', 'ActingTrainer',
-           'ActorNetwork', 'FusedCritic', 'DeviceReplayBuffer', 'EpisodeHistory', 'HostRollout', 'distributed']
+           'ActorNetwork', 'FusedCritic', 'FusedCriticNetwork', 'DeviceReplayBuffer', 'EpisodeHistory', 'HostRollout', 'distributed']

@@ -7,7 +7,7 @@ import os
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get('MPE_B200_LIB', os.path.join(HERE, 'libmpe_b200.so'))  # override: A/B builds
-ABI_VERSION = 6
+ABI_VERSION = 7
 
 MPE_OK, MPE_EINVAL, MPE_ECUDA, MPE_EUNSUPPORTED = 0, -1, -2, -3
 SCENARIO_IDS = {'simple_spread': 0, 'simple_reference': 1, 'simple_speaker_listener': 2, 'fullobs_collect_treasure': 3}
@@ -49,6 +49,11 @@ class CriticConfig(C.Structure):
 
 
 class CriticWeights(C.Structure):
+    _fields_ = [(n, C.c_void_p) for n in ('dense1_w', 'dense1_b', 'w_ih', 'w_hh', 'b_ih', 'b_hh', 'dense2_w', 'dense2_b',
+                                          'dense3_w', 'dense3_b')]
+
+
+class CriticGrads(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in ('dense1_w', 'dense1_b', 'w_ih', 'w_hh', 'b_ih', 'b_hh', 'dense2_w', 'dense2_b',
                                           'dense3_w', 'dense3_b')]
 
@@ -98,6 +103,8 @@ SIGNATURES = {
     'critic_load': (C.c_int, [P, C.POINTER(CriticWeights), P]),
     'critic_load_device': (C.c_int, [P, C.POINTER(CriticWeights), P]),
     'critic_forward': (C.c_int, [P, P, P, C.c_int64, C.c_int32, P, P, P]),
+    'critic_backward_workspace': (C.c_int64, [P, C.c_int64, C.c_int32]),
+    'critic_backward': (C.c_int, [P, P, P, C.c_int64, C.c_int32, P, P, P, P, C.POINTER(CriticGrads), P, C.c_int64, P]),
     'replay_create': (C.c_int, [C.POINTER(ReplayConfig), C.POINTER(P)]),
     'replay_destroy': (C.c_int, [P]),
     'replay_clear': (C.c_int, [P]),

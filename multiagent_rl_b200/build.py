@@ -27,6 +27,7 @@ UNITS = [
     ('tc_kernels.cu', []),
     ('replay_kernels.cu', []),
     ('critic_kernels.cu', []),
+    ('critic_grad_kernels.cu', []),
     ('pack_kernels.cu', []),
     ('cabi.cu', ['-Xcompiler', '-fvisibility=default']),
 ]

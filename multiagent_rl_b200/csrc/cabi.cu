@@ -936,6 +936,40 @@ int critic_forward(MpeCritic *c, const float *obs, const float *action, int64_t 
   return MPE_OK;
 }
 
+int64_t critic_backward_workspace(MpeCritic *c, int64_t B, int32_t N) {
+  if (c == nullptr) return fail(MPE_EINVAL, "critic_backward_workspace: null critic");
+  if (B < 0) return fail(MPE_EINVAL, "critic_backward_workspace: B < 0");
+  if (N < 1 || N > mpe::kCriticMaxAgents) return fail(MPE_EUNSUPPORTED, "critic_backward_workspace: 1..16 agents");
+  return mpe::critic_backward_bytes(c->dev, B, N);
+}
+
+int critic_backward(MpeCritic *c, const float *obs, const float *action, int64_t B, int32_t N, const float *dq,
+                    const float *dr, float *dobs, float *daction, const CriticGrads *grads, void *workspace,
+                    int64_t workspace_bytes, void *stream) {
+  if (c == nullptr || obs == nullptr || action == nullptr || dq == nullptr || workspace == nullptr)
+    return fail(MPE_EINVAL, "critic_backward: null argument");
+  if (B < 0) return fail(MPE_EINVAL, "critic_backward: B < 0");
+  if (N < 1 || N > mpe::kCriticMaxAgents) return fail(MPE_EUNSUPPORTED, "critic_backward: 1..16 agents");
+  const CriticGrads none = {};
+  const CriticGrads &g = grads != nullptr ? *grads : none;
+  if (!c->dev.has_r && (dr != nullptr || g.dense3_w != nullptr || g.dense3_b != nullptr))
+    return fail(MPE_EINVAL, "critic_backward: dr / dense3 gradients on a critic without a reward head");
+  const int64_t need = mpe::critic_backward_bytes(c->dev, B, N);
+  if (workspace_bytes < need)
+    return fail(MPE_EINVAL, "critic_backward: workspace of " + std::to_string(workspace_bytes) + " bytes, " +
+                                std::to_string(need) + " needed");
+  if (B == 0) return MPE_OK;
+  const void *ptrs[] = {obs, action, dq, dr, dobs, daction, workspace, g.dense1_w, g.dense1_b, g.w_ih, g.w_hh,
+                        g.b_ih, g.b_hh, g.dense2_w, g.dense2_b, g.dense3_w, g.dense3_b};
+  for (const void *p : ptrs)
+    if (p != nullptr && !device_memory(p, c->device))
+      return fail(MPE_EINVAL, "critic_backward: a pointer is not device memory on the critic's device");
+  DeviceGuard dg(c->device);
+  CK(mpe::launch_critic_backward(c->dev, obs, action, B, N, dq, dr, dobs, daction, g, workspace,
+                                 static_cast<cudaStream_t>(stream)));
+  return MPE_OK;
+}
+
 // ------------------------------------------------------------------------------------------------
 // replay ring
 // ------------------------------------------------------------------------------------------------

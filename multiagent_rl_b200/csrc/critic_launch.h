@@ -1,4 +1,5 @@
-// Host-side interface of the critic forward kernel (critic_kernels.cu) used by cabi.cu.
+// Host-side interface of the critic kernels (critic_kernels.cu: forward, critic_grad_kernels.cu: backward) used by
+// cabi.cu.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -11,6 +12,7 @@ constexpr int kCriticH = 64;        // dense1 width = LSTM input = LSTM hidden (
 constexpr int kCriticMaxIn = 64;    // obs_dim + sum(action widths)
 constexpr int kCriticMaxAgents = 16;
 constexpr int kCriticMaxOut = 4;
+constexpr int kCriticGradFields = 10;  // the pointers of CriticGrads
 
 // Packed fp32 blob in device memory (what a CTA stages into shared memory with one bulk copy)
 struct CriticDev {
@@ -26,5 +28,13 @@ cudaError_t launch_critic_pack(const CriticDev &d, const CriticWeights &src, cud
 // obs [B][N][D], action [B][N][A] (one-hot or soft), q / r [B][out]
 cudaError_t launch_critic_forward(const CriticDev &w, const float *obs, const float *action, int64_t B, int N, float *q,
                                   float *r, cudaStream_t st);
+// Bytes of the workspace launch_critic_backward needs for B samples of N agents (0 for B <= 0).
+int64_t critic_backward_bytes(const CriticDev &w, int64_t B, int N);
+// Gradients of launch_critic_forward's function: dq / dr [B][out] upstream (dr may be NULL), dobs [B][N][D],
+// daction [B][N][A] and the non-NULL fields of `g` ([out][in] layout) overwritten.  `workspace` holds
+// critic_backward_bytes(w, B, N) bytes of device memory.
+cudaError_t launch_critic_backward(const CriticDev &w, const float *obs, const float *action, int64_t B, int N,
+                                   const float *dq, const float *dr, float *dobs, float *daction,
+                                   const CriticGrads &g, void *workspace, cudaStream_t st);
 
 }  // namespace mpe

@@ -116,5 +116,14 @@ for model in (False, True):
     critic = m.FusedCritic(csd, obs_dim=10)
     critic.load_state_dict({k: torch.from_numpy(v).float().cuda() for k, v in csd.items()})
     critic.forward(torch.zeros((17, 3, 10), device='cuda'), torch.zeros((17, 3, 5), device='cuda'))
+    # the backward kernel and both gradient reductions at ragged sizes: one sample, a partial last CTA, 16 agents
+    for B, N in ((1, 1), (17, 3), (1031, 16)):
+        o = torch.randn((B, N, 10), device='cuda')
+        a = torch.randn((B, N, 5), device='cuda')
+        dq = torch.randn((B, 1), device='cuda')
+        critic.backward(o, a, dq, torch.randn((B, 1), device='cuda') if model else None, want_obs=True)
+    net = m.FusedCriticNetwork(15, 1, model=model).cuda()
+    out = net(torch.randn((33, 3, 10), device='cuda'), torch.randn((33, 3, 5), device='cuda'))
+    (out[0].sum() + out[1].sum() if model else out.sum()).backward()
 torch.cuda.synchronize()
 print('sanitize target done')
