@@ -7,7 +7,8 @@ What runs where:
     never leave HBM;
   * learning: the reference's `Trainer.optimize()` (rls/agent/multiagent/ddpg_gumbel_fix.py:131-219) UNCHANGED, with the
     device replay as its `memory`; after every update the fused actor reloads the weights.  With `--fused-critic` the
-    learner's critic is `FusedCriticNetwork`, whose forward and backward are the critic kernels.
+    learner's critic is `FusedCriticNetwork`, whose forward and backward are the critic kernels; with `--fused-actor`
+    the learner's actor is `FusedActorNetwork`, whose forward and backward are the actor kernels.
 
 Needs the reference on the import path (PYTHONPATH=/path/to/multiagent_rl, or the compiled copy `python -m
 oracle.build_ref` leaves in oracle/_ref).  Example:
@@ -40,7 +41,7 @@ def import_reference():
 
 
 def train(num_envs=4096, episodes=20, updates_per_episode=4, scenario='simple_spread', n=None, seed=12345678,
-          batch_size=1024, lr=1e-2, log=print, fused_critic=False):
+          batch_size=1024, lr=1e-2, log=print, fused_critic=False, fused_actor=False):
     arglist, Trainer, ActorNetwork, CriticNetwork = import_reference()
     arglist.actor_learning_rate = arglist.critic_learning_rate = lr   # main.py:34-35
     arglist.batch_size = batch_size
@@ -50,7 +51,7 @@ def train(num_envs=4096, episodes=20, updates_per_episode=4, scenario='simple_sp
     env = m.make_env(scenario, n=n, num_envs=num_envs, batched=True, seed=seed, max_episode_len=T)
     N, D = env.n, env.obs_dim
     A = 5
-    actor = ActorNetwork(input_dim=D, out_dim=A)
+    actor = (m.FusedActorNetwork if fused_actor else ActorNetwork)(D, A)
     critic = (m.FusedCriticNetwork if fused_critic else CriticNetwork)(D + A, 1)
     memory = m.DeviceReplayBuffer(max(1_000_000, 2 * num_envs * T), N, D, A, seed=seed)
     learner = Trainer(actor, critic, memory, action_type='Discrete')        # the reference's class, cuda:0
@@ -80,5 +81,6 @@ if __name__ == '__main__':
     ap.add_argument('--scenario', default='simple_spread')
     ap.add_argument('--n', type=int, default=None)
     ap.add_argument('--fused-critic', action='store_true', help='train the critic through the CUDA kernels')
+    ap.add_argument('--fused-actor', action='store_true', help='train the actor through the CUDA kernels')
     a = ap.parse_args()
-    train(a.envs, a.episodes, scenario=a.scenario, n=a.n, fused_critic=a.fused_critic)
+    train(a.envs, a.episodes, scenario=a.scenario, n=a.n, fused_critic=a.fused_critic, fused_actor=a.fused_actor)

@@ -35,7 +35,7 @@
 extern "C" {
 #endif
 
-#define MPE_ABI_VERSION 7
+#define MPE_ABI_VERSION 8
 
 enum { MPE_OK = 0, MPE_EINVAL = -1, MPE_ECUDA = -2, MPE_EUNSUPPORTED = -3 };
 enum { MPE_SIMPLE_SPREAD = 0, MPE_SIMPLE_REFERENCE = 1, MPE_SIMPLE_SPEAKER_LISTENER = 2,
@@ -214,6 +214,35 @@ int actor_forward(MpeActor *actor, const float *obs, int64_t B, int32_t N, const
 int actor_forward_host(MpeActor *actor, const float *obs_host, int64_t B, int32_t N, uint64_t seed,
                        uint64_t step, int64_t env_id_offset, int32_t *act_u_host, int32_t *act_c_host,
                        float *onehot_host, void *stream);
+
+/* Gradients of the actor forward for Trainer.optimize() (ddpg_gumbel_fix.py:131-219): the actor loss through the
+ * weights.  Output tensors are fp32 in the reference's state_dict layout ([out][in]), mirroring ActorWeights; a NULL
+ * field is not computed.  bias_ih* and bias_hh* of a direction get the same gradient. */
+typedef struct {
+  float *dense1_w, *dense1_b;               /* [64][D], [64]    */
+  float *w_ih, *w_hh, *b_ih, *b_hh;         /* [128][64], [128][32], [128], [128] */
+  float *w_ih_r, *w_hh_r, *b_ih_r, *b_hh_r; /* *_reverse        */
+  float *dense2_w, *dense2_b;               /* [act0][64], [act0]  (dense2 or dense2_1) */
+  float *dense2b_w, *dense2b_b;             /* [act1][64], [act1]  (dense2_2); two-head actors only */
+  float *dense3_w, *dense3_b;               /* [D][64], [D]; "+model" actors only       */
+} ActorGrads;
+/* Bytes of device workspace actor_backward needs for B samples of N agents (0 for B = 0); < 0 (MPE_E*) on error. */
+int64_t actor_backward_workspace(MpeActor *actor, int64_t B, int32_t N);
+/* Backward of the fp32 FFMA actor forward (actor_set_impl 1) on obs [B][N][D], with the weights of the last
+ * actor_load* enqueued on `stream` (the forward is recomputed; nothing is kept from an earlier actor_forward).
+ * dlogits [B][N][act0+act1] is the gradient of the loss with respect to the logits (both heads concatenated);
+ * dnext_state [B][N][D] that with respect to next_state, for the "+model" actor only, NULL meaning zero.  Outputs,
+ * each optional (NULL: not computed) and overwritten, never accumulated: dobs [B][N][D] and the fields of `grads`
+ * (which may itself be NULL).  `workspace` is device memory of at least actor_backward_workspace(actor, B, N) bytes,
+ * borrowed like every buffer; calls on different streams need different workspaces.  Enqueued on `stream`: no host
+ * synchronisation, no allocation.  Deterministic: no floating-point atomics, every sum in an order that depends on B
+ * and N alone, and a sample's dobs does not depend on where it sits in the batch.  MPE_EINVAL before any launch for a
+ * null actor / obs / dlogits / workspace, dnext_state or dense3 gradients on an actor without a model head, dense2b
+ * gradients on a single-head actor, a workspace that is too small, B < 0, or a pointer that is not device memory on
+ * the actor's device; MPE_EUNSUPPORTED for N outside 1..12. */
+int actor_backward(MpeActor *actor, const float *obs, int64_t B, int32_t N, const float *dlogits,
+                   const float *dnext_state, float *dobs, const ActorGrads *grads, void *workspace,
+                   int64_t workspace_bytes, void *stream);
 
 /* The loop body of experiments/run.py:36-65 fused: for t in [0, T): observe -> actor -> sample ->
  * step -> reward -> (episode_step == max_episode_len ? reset), state never leaving the SM between

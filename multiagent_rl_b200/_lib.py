@@ -7,7 +7,7 @@ import os
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get('MPE_B200_LIB', os.path.join(HERE, 'libmpe_b200.so'))  # override: A/B builds
-ABI_VERSION = 7
+ABI_VERSION = 8
 
 MPE_OK, MPE_EINVAL, MPE_ECUDA, MPE_EUNSUPPORTED = 0, -1, -2, -3
 SCENARIO_IDS = {'simple_spread': 0, 'simple_reference': 1, 'simple_speaker_listener': 2, 'fullobs_collect_treasure': 3}
@@ -66,6 +66,10 @@ class ActorWeights(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in _WEIGHT_FIELDS]
 
 
+class ActorGrads(C.Structure):
+    _fields_ = [(n, C.c_void_p) for n in _WEIGHT_FIELDS]
+
+
 P = C.c_void_p
 # name -> (restype, argtypes); must list EVERY symbol include/mpe_b200.h declares
 SIGNATURES = {
@@ -97,6 +101,8 @@ SIGNATURES = {
     'actor_set_impl': (C.c_int, [P, C.c_int32]),
     'actor_forward': (C.c_int, [P, P, C.c_int64, C.c_int32, P, C.c_uint64, C.c_uint64, C.c_int64, P, P, P, P, P, P]),
     'actor_forward_host': (C.c_int, [P, P, C.c_int64, C.c_int32, C.c_uint64, C.c_uint64, C.c_int64, P, P, P, P]),
+    'actor_backward_workspace': (C.c_int64, [P, C.c_int64, C.c_int32]),
+    'actor_backward': (C.c_int, [P, P, C.c_int64, C.c_int32, P, P, P, C.POINTER(ActorGrads), P, C.c_int64, P]),
     'mpe_rollout': (C.c_int, [P, P, C.c_int32, C.c_uint64, P, P, P, P, P]),
     'critic_create': (C.c_int, [C.POINTER(CriticConfig), C.POINTER(P)]),
     'critic_destroy': (C.c_int, [P]),
@@ -189,6 +195,22 @@ def weights(cls, sd, names, shapes, device):
 def current_stream(device):
     import torch
     return C.c_void_p(torch.cuda.current_stream(device).cuda_stream)
+
+
+class ModuleHandle(object):
+    """The device handle of one fused network module (``FusedCriticNetwork``, ``FusedActorNetwork``), kept in the
+    attribute named ``slot`` (None until the module's first forward creates it).  A deep copy (how learners build
+    target networks) or a pickle starts without one, so copies never share or double-free a handle."""
+
+    def __init__(self, slot):
+        self._slot = slot
+        setattr(self, slot, None)
+
+    def __deepcopy__(self, memo):
+        return ModuleHandle(self._slot)
+
+    def __getstate__(self):
+        return {'_slot': self._slot, self._slot: None}
 
 
 class HostBlock(object):

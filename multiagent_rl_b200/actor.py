@@ -1,5 +1,6 @@
 """Acting surface: the reference's ``ActorNetwork`` forward + hard Gumbel-softmax sampling as one
-CUDA kernel, behind the names the reference uses.
+CUDA kernel, behind the names the reference uses; and the actor's backward, so that ``Trainer.optimize()`` can train
+the actor through the kernels (``FusedActorNetwork``).
 
 Mirrors
   * ``rls/model/ac_network_multi_gumbel.py:24-67`` (ActorNetwork; state_dict key names are kept so a
@@ -11,8 +12,11 @@ import ctypes as C
 
 import numpy as np
 import torch
+import torch.nn as nn
+from torch.autograd.function import once_differentiable
 
 from . import _lib
+from .networks import _PerAgent
 
 _KEYS = [('dense1_w', 'dense1.module.weight'), ('dense1_b', 'dense1.module.bias'),
          ('w_ih', 'bilstm.weight_ih_l0'), ('w_hh', 'bilstm.weight_hh_l0'),
@@ -66,6 +70,30 @@ class FusedActor(object):
         _lib.check(self._lib.actor_set_impl(self._h, self.IMPLS[impl]), 'actor_set_impl')
         self.impl = impl
 
+    def _names(self):
+        """(ActorWeights field, state_dict key) of every tensor this actor has."""
+        names = list(_KEYS)
+        if self.multi:
+            names += [('dense2_w', 'dense2_1.module.weight'), ('dense2_b', 'dense2_1.module.bias'),
+                      ('dense2b_w', 'dense2_2.module.weight'), ('dense2b_b', 'dense2_2.module.bias')]
+        else:
+            names += [('dense2_w', 'dense2.module.weight'), ('dense2_b', 'dense2.module.bias')]
+        if self.has_model:
+            names += [('dense3_w', 'dense3.module.weight'), ('dense3_b', 'dense3.module.bias')]
+        return names
+
+    def _shapes(self):
+        H = 64
+        shapes = {'dense1_w': (H, self.obs_dim), 'dense1_b': (H,)}
+        for d in ('', '_r'):
+            shapes.update({'w_ih' + d: (4 * 32, H), 'w_hh' + d: (4 * 32, 32), 'b_ih' + d: (4 * 32,), 'b_hh' + d: (4 * 32,)})
+        shapes.update({'dense2_w': (self.act_dims[0], H), 'dense2_b': (self.act_dims[0],)})
+        if self.multi:
+            shapes.update({'dense2b_w': (self.act_dims[1], H), 'dense2b_b': (self.act_dims[1],)})
+        if self.has_model:
+            shapes.update({'dense3_w': (self.obs_dim, H), 'dense3_b': (self.obs_dim,)})
+        return shapes
+
     def load_state_dict(self, sd):
         """``actor.load_state_dict`` (rls/agent/multiagent/ddpg_gumbel_fix.py:231-241).
 
@@ -75,22 +103,7 @@ class FusedActor(object):
         overwritten in place, so work on other streams that uses this actor must be ordered with events.  Anything
         else (numpy arrays, CPU tensors, another device) is read on the host; the call returns when it has been
         loaded.  KeyError for a missing key, ValueError for a tensor of the wrong shape."""
-        H = 64
-        names = list(_KEYS)
-        shapes = {'dense1_w': (H, self.obs_dim), 'dense1_b': (H,)}
-        for d in ('', '_r'):
-            shapes.update({'w_ih' + d: (4 * 32, H), 'w_hh' + d: (4 * 32, 32), 'b_ih' + d: (4 * 32,), 'b_hh' + d: (4 * 32,)})
-        if self.multi:
-            names += [('dense2_w', 'dense2_1.module.weight'), ('dense2_b', 'dense2_1.module.bias'),
-                      ('dense2b_w', 'dense2_2.module.weight'), ('dense2b_b', 'dense2_2.module.bias')]
-            shapes.update({'dense2b_w': (self.act_dims[1], H), 'dense2b_b': (self.act_dims[1],)})
-        else:
-            names += [('dense2_w', 'dense2.module.weight'), ('dense2_b', 'dense2.module.bias')]
-        shapes.update({'dense2_w': (self.act_dims[0], H), 'dense2_b': (self.act_dims[0],)})
-        if self.has_model:
-            names += [('dense3_w', 'dense3.module.weight'), ('dense3_b', 'dense3.module.bias')]
-            shapes.update({'dense3_w': (self.obs_dim, H), 'dense3_b': (self.obs_dim,)})
-        w, keep, on_device = _lib.weights(_lib.ActorWeights, sd, names, shapes, self.device)
+        w, keep, on_device = _lib.weights(_lib.ActorWeights, sd, self._names(), self._shapes(), self.device)
         fn = 'actor_load_device' if on_device else 'actor_load'
         _lib.check(getattr(self._lib, fn)(self._h, C.byref(w), _lib.current_stream(self.device)), fn)
         del keep  # the host path has copied the arrays; device tensors are released in stream order by torch
@@ -120,6 +133,41 @@ class FusedActor(object):
             _lib.ptr(out['act_u']), _lib.ptr(out['act_c']), _lib.ptr(out['onehot']),
             _lib.current_stream(dev)), 'actor_forward')
         return out
+
+    def backward(self, obs, dlogits, dnext_state=None, want_obs=False, want_weights=True):
+        """Gradients of the fp32 FFMA forward (``impl='simt'``) of ``obs`` [B,N,D] with the loaded weights, for
+        upstream gradients ``dlogits`` [B,N,A] (both heads concatenated) and, for the "+model" actor, ``dnext_state``
+        [B,N,D] (None: zero).  Returns ``{'obs': [B,N,D] | None, 'weights': {state_dict key: gradient} (empty unless
+        want_weights)}``; ``bias_ih*`` and ``bias_hh*`` of a direction get the same gradient.  Outputs and workspace
+        come from torch's allocator; the kernels run on torch's current stream without a host synchronisation."""
+        obs = torch.as_tensor(obs, dtype=torch.float32, device=self.device).contiguous()
+        B, N, D = obs.shape
+        if D != self.obs_dim:
+            raise ValueError('obs has D=%d, actor expects %d' % (D, self.obs_dim))
+        dlogits = torch.as_tensor(dlogits, dtype=torch.float32, device=self.device).contiguous()
+        if tuple(dlogits.shape) != (B, N, self.A):
+            raise ValueError('expected dlogits [%d,%d,%d]' % (B, N, self.A))
+        if dnext_state is not None:
+            if not self.has_model:
+                raise ValueError('dnext_state is the gradient of the dense3 head, which this actor does not have')
+            dnext_state = torch.as_tensor(dnext_state, dtype=torch.float32, device=self.device).contiguous()
+            if tuple(dnext_state.shape) != (B, N, D):
+                raise ValueError('expected dnext_state [%d,%d,%d]' % (B, N, D))
+        dobs = torch.empty_like(obs) if want_obs else None
+        grads, g = {}, _lib.ActorGrads()
+        if want_weights:
+            shapes = self._shapes()
+            for field, key in self._names():
+                grads[key] = torch.empty(shapes[field], dtype=torch.float32, device=self.device)
+                setattr(g, field, grads[key].data_ptr())
+        nbytes = self._lib.actor_backward_workspace(self._h, B, N)
+        if nbytes < 0:
+            _lib.check(nbytes, 'actor_backward_workspace')
+        ws = torch.empty(max(nbytes, 1), dtype=torch.uint8, device=self.device)
+        _lib.check(self._lib.actor_backward(self._h, _lib.ptr(obs), B, N, _lib.ptr(dlogits), _lib.ptr(dnext_state),
+                                            _lib.ptr(dobs), C.byref(g), _lib.ptr(ws), nbytes,
+                                            _lib.current_stream(self.device)), 'actor_backward')
+        return {'obs': dobs, 'weights': grads}
 
     # ------------------------------------------------------------------ host buffers
     def act_host(self, obs_host, step=0, env_id_offset=0, act_u=None, act_c=None, onehot=None, seed=None):
@@ -199,3 +247,97 @@ class ActingTrainer(FusedActingMixin):
     def save_models(self, fname):
         """rls/agent/multiagent/ddpg_gumbel_fix.py:221-229 (actor only; this stand-in has no target network)."""
         torch.save(self.actor.state_dict(), './Models/' + str(fname) + '_actor.pt')
+
+
+class _ActorFunction(torch.autograd.Function):
+    """logits (, next_state) = actor(obs) with the weights ``params``: the FFMA forward kernel after a repack of
+    ``params``; the backward repacks the saved ``params`` and runs actor_backward for the gradients autograd asks for."""
+
+    @staticmethod
+    def forward(ctx, actor, keys, obs, *params):
+        actor.load_state_dict(dict(zip(keys, params)))
+        out = actor.forward(obs, want_logits=True, want_next_state=actor.has_model)
+        ctx.actor, ctx.keys = actor, keys
+        ctx.save_for_backward(obs, *params)
+        ctx.set_materialize_grads(False)
+        return (out['logits'], out['next_state']) if actor.has_model else out['logits']
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, dlogits, dnext_state=None):
+        obs, params = ctx.saved_tensors[0], ctx.saved_tensors[1:]
+        need = ctx.needs_input_grad
+        want_w = any(need[3:])
+        if not (need[2] or want_w) or (dlogits is None and dnext_state is None):
+            return (None,) * len(need)
+        actor = ctx.actor
+        unused = set()  # an output the loss does not use gets no gradient, as under autograd
+        if dlogits is None:
+            dlogits = torch.zeros(tuple(obs.shape[:2]) + (actor.A,), dtype=torch.float32, device=obs.device)
+            unused = {k for k in ctx.keys if k.startswith('dense2')}
+        elif actor.has_model and dnext_state is None:
+            unused = {'dense3.module.weight', 'dense3.module.bias'}
+        actor.load_state_dict(dict(zip(ctx.keys, params)))
+        g = actor.backward(obs, dlogits, dnext_state, want_obs=need[2], want_weights=want_w)
+        wg = [g['weights'][k] if n and k not in unused else None for k, n in zip(ctx.keys, need[3:])]
+        return (None, None, g['obs']) + tuple(wg)
+
+
+class FusedActorNetwork(nn.Module):
+    """Drop-in for the reference ``ActorNetwork(input_dim, out_dim)`` (rls/model/ac_network_multi_gumbel.py:24-67;
+    ``out_dim`` an int or a list of two head widths), or with ``model_head=True`` for the actor of
+    ac_network_model_multi_gumbel.py (dense3 head), that runs forward and backward as CUDA kernels.
+
+    Parameters are plain ``nn.Parameter`` s under the reference's names and created in its order (``dense1.module``,
+    ``bilstm`` - an ``nn.LSTM(64, 32, bidirectional=True)`` that only holds the parameters and is never called -
+    ``dense2`` or ``dense2_1`` / ``dense2_2``, ``dense3``), so a seed gives the reference's initial weights, and
+    state_dict / load_state_dict / optimizers work as for the reference.  ``forward(obs [B,N,D])`` returns what the
+    reference returns: logits [B,N,A] (a list of two for two heads; ``(policy, next_state)`` with the model head).
+    Every forward repacks the parameters into the kernel's weight image on the current stream (a soft update written
+    through ``.data`` is seen by the next call) and runs the fp32 FFMA forward, which the backward differentiates; the
+    backward repacks the parameters it saved.  Parameters must be float32 on a CUDA device; there is no CPU path."""
+
+    def __init__(self, input_dim, out_dim, model_head=False):
+        super().__init__()
+        input_dim = int(input_dim)
+        heads = [int(a) for a in out_dim] if isinstance(out_dim, (list, tuple)) else [int(out_dim)]
+        if not 1 <= input_dim <= 64:
+            raise ValueError('FusedActorNetwork: input_dim must be 1..64 (the kernel stages one observation row per '
+                             'lane pair), got %d' % input_dim)
+        if len(heads) not in (1, 2) or min(heads) < 1 or sum(heads) > 16:
+            raise ValueError('FusedActorNetwork: one or two heads of at least one entry and at most 16 in total, '
+                             'got %s' % (out_dim,))
+        self.input_dim, self.out_dim, self.model_head = input_dim, out_dim, bool(model_head)
+        self.dense1 = _PerAgent(nn.Linear(input_dim, 64))
+        self.bilstm = nn.LSTM(64, 32, num_layers=1, batch_first=True, bidirectional=True)
+        if len(heads) == 2:
+            self.dense2_1 = _PerAgent(nn.Linear(64, heads[0]))
+            self.dense2_2 = _PerAgent(nn.Linear(64, heads[1]))
+        else:
+            self.dense2 = _PerAgent(nn.Linear(64, heads[0]))
+        if self.model_head:
+            self.dense3 = _PerAgent(nn.Linear(64, input_dim))
+        self._heads = heads
+        self._handle = _lib.ModuleHandle('actor')
+
+    def forward(self, obs):
+        sd = dict(self.named_parameters())
+        keys = list(sd)
+        params = [sd[k] for k in keys]
+        dev = params[0].device
+        if dev.type != 'cuda' or any(p.device != dev or p.dtype != torch.float32 for p in params):
+            raise RuntimeError('FusedActorNetwork runs only as a CUDA kernel: its parameters must be float32 tensors '
+                               'on one CUDA device (call .cuda()); got %s %s' % (params[0].dtype, dev))
+        obs = torch.as_tensor(obs, device=dev).float()
+        if obs.dim() != 3 or obs.shape[2] != self.input_dim:
+            raise ValueError('expected obs [B,N,%d], got %s' % (self.input_dim, tuple(obs.shape)))
+        if not 1 <= obs.shape[1] <= 12:
+            raise ValueError('FusedActorNetwork: 1..12 agents (the kernel unrolls the agent axis), got %d'
+                             % obs.shape[1])
+        h = self._handle
+        if h.actor is None or h.actor.device != dev:
+            h.actor = FusedActor({k: p.detach() for k, p in zip(keys, params)}, device=dev, impl='simt')
+        out = _ActorFunction.apply(h.actor, keys, obs.contiguous(), *params)
+        logits, next_state = out if self.model_head else (out, None)
+        policy = [logits[..., :self._heads[0]], logits[..., self._heads[0]:]] if len(self._heads) == 2 else logits
+        return (policy, next_state) if self.model_head else policy

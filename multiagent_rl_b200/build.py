@@ -28,6 +28,8 @@ UNITS = [
     ('replay_kernels.cu', []),
     ('critic_kernels.cu', []),
     ('critic_grad_kernels.cu', []),
+    ('actor_grad_kernels.cu', []),
+    ('grad_reduce.cu', []),
     ('pack_kernels.cu', []),
     ('cabi.cu', ['-Xcompiler', '-fvisibility=default']),
 ]

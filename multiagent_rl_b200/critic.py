@@ -125,20 +125,6 @@ class FusedCritic(object):
         return {'obs': dobs, 'action': dact, 'weights': grads}
 
 
-class _Handle(object):
-    """The device handle of one FusedCriticNetwork.  A deep copy (how learners build target networks) or a pickle
-    starts without one, so copies never share or double-free a handle."""
-
-    def __init__(self):
-        self.critic = None
-
-    def __deepcopy__(self, memo):
-        return _Handle()
-
-    def __getstate__(self):
-        return {'critic': None}
-
-
 class _CriticFunction(torch.autograd.Function):
     """q (, r) = critic(obs, action) with the weights ``params``: the forward kernel after a repack of ``params``; the
     backward repacks the saved ``params`` and runs critic_backward for the gradients autograd asks for."""
@@ -202,7 +188,7 @@ class FusedCriticNetwork(nn.Module):
         self.dense2 = nn.Linear(_H, out_dim)
         if self.model:
             self.dense3 = nn.Linear(_H, out_dim)
-        self._handle = _Handle()
+        self._handle = _lib.ModuleHandle('critic')
 
     def _keys(self):
         return [k for _, k in _KEYS] + ([k for _, k in _KEYS3] if self.model else [])

@@ -15,6 +15,7 @@
 // the cell state of those (row, unit) pairs for the whole sequence, so c never leaves registers.
 #include <cmath>
 
+#include "actor_cell.cuh"
 #include "actor_launch.h"
 #include "common.cuh"
 #include "launch.h"
@@ -51,8 +52,7 @@ void actor_layout(int D, int A0, int A1, bool has_model, ActorDev *o) {
 // ------------------------------------------------------------------------------------------------
 // device helpers
 // ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ float sigmoid_f(float x) { return __fdividef(1.0f, 1.0f + __expf(-x)); }
-__device__ __forceinline__ float tanh_f(float x) { return 1.0f - __fdividef(2.0f, 1.0f + __expf(2.0f * x)); }
+// sigmoid_f / tanh_f: actor_cell.cuh
 
 template <int RT>
 __device__ __forceinline__ void load_rows(const float *p, float (&a)[RT]) {

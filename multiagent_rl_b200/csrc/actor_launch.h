@@ -1,4 +1,5 @@
-// Host-side interface of the actor kernels (actor_kernels.cu, tc_kernels.cu) used by cabi.cu.
+// Host-side interface of the actor kernels (actor_kernels.cu, tc_kernels.cu; backward: actor_grad_kernels.cu) used
+// by cabi.cu.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -84,5 +85,13 @@ cudaError_t launch_rollout_tc(const EnvStateAny &env, const TcDev &w, const Roll
 cudaError_t launch_actor_pack(const ActorDev &d, const ActorWeights &src, cudaStream_t st);
 // next_state = dense3(hcat): the "+model" head (ac_network_model_multi_gumbel.py:49,65) on top of the tensor-core forward
 cudaError_t launch_dense3(const ActorDev &w, const float *hcat, int64_t rows, float *next_state, cudaStream_t st);
+// Bytes of the workspace launch_actor_backward needs for B samples of N agents (0 for B <= 0).
+int64_t actor_backward_bytes(const ActorDev &w, int64_t B, int N);
+// Gradients of the FFMA forward's logits / next_state: dlogits [B][N][A] upstream, dnext_state [B][N][D] (NULL: zero),
+// dobs [B][N][D] and the non-NULL fields of `g` ([out][in] layout) overwritten.  `workspace` holds
+// actor_backward_bytes(w, B, N) bytes of device memory.
+cudaError_t launch_actor_backward(const ActorDev &w, const float *obs, int64_t B, int N, const float *dlogits,
+                                  const float *dnext_state, float *dobs, const ActorGrads &g, void *workspace,
+                                  cudaStream_t st);
 
 }  // namespace mpe

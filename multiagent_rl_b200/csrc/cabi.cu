@@ -585,6 +585,42 @@ int actor_forward_host(MpeActor *a, const float *obs_host, int64_t B, int32_t N,
   return MPE_OK;
 }
 
+int64_t actor_backward_workspace(MpeActor *a, int64_t B, int32_t N) {
+  if (a == nullptr) return fail(MPE_EINVAL, "actor_backward_workspace: null actor");
+  if (B < 0) return fail(MPE_EINVAL, "actor_backward_workspace: B < 0");
+  if (!mpe::actor_supported(N)) return fail(MPE_EUNSUPPORTED, "actor_backward_workspace: 1..12 agents");
+  return mpe::actor_backward_bytes(a->dev, B, N);
+}
+
+int actor_backward(MpeActor *a, const float *obs, int64_t B, int32_t N, const float *dlogits, const float *dnext_state,
+                   float *dobs, const ActorGrads *grads, void *workspace, int64_t workspace_bytes, void *stream) {
+  if (a == nullptr || obs == nullptr || dlogits == nullptr || workspace == nullptr)
+    return fail(MPE_EINVAL, "actor_backward: null argument");
+  if (B < 0) return fail(MPE_EINVAL, "actor_backward: B < 0");
+  if (!mpe::actor_supported(N)) return fail(MPE_EUNSUPPORTED, "actor_backward: 1..12 agents");
+  const ActorGrads none = {};
+  const ActorGrads &g = grads != nullptr ? *grads : none;
+  if (!a->dev.has_model && (dnext_state != nullptr || g.dense3_w != nullptr || g.dense3_b != nullptr))
+    return fail(MPE_EINVAL, "actor_backward: dnext_state / dense3 gradients on an actor without a model head");
+  if (a->dev.A1 == 0 && (g.dense2b_w != nullptr || g.dense2b_b != nullptr))
+    return fail(MPE_EINVAL, "actor_backward: dense2_2 gradients on a single-head actor");
+  const int64_t need = mpe::actor_backward_bytes(a->dev, B, N);
+  if (workspace_bytes < need)
+    return fail(MPE_EINVAL, "actor_backward: workspace of " + std::to_string(workspace_bytes) + " bytes, " +
+                                std::to_string(need) + " needed");
+  if (B == 0) return MPE_OK;
+  const void *ptrs[] = {obs, dlogits, dnext_state, dobs, workspace, g.dense1_w, g.dense1_b, g.w_ih, g.w_hh, g.b_ih,
+                        g.b_hh, g.w_ih_r, g.w_hh_r, g.b_ih_r, g.b_hh_r, g.dense2_w, g.dense2_b, g.dense2b_w,
+                        g.dense2b_b, g.dense3_w, g.dense3_b};
+  for (const void *p : ptrs)
+    if (p != nullptr && !device_memory(p, a->device))
+      return fail(MPE_EINVAL, "actor_backward: a pointer is not device memory on the actor's device");
+  DeviceGuard dg(a->device);
+  CK(mpe::launch_actor_backward(a->dev, obs, B, N, dlogits, dnext_state, dobs, g, workspace,
+                                static_cast<cudaStream_t>(stream)));
+  return MPE_OK;
+}
+
 static MpeHostBlockLayout block_layout(const mpe::EnvStateAny &s) {
   const uint64_t rows = (uint64_t)s.B * s.N, rs = real_size(s.precision);
   auto up = [](uint64_t x) { return (x + 255) / 256 * 256; };

@@ -12,9 +12,10 @@
 //      softmax backward and BPTT over the agent axis.  Writes dobs / daction and, per (sample, agent) row, what the
 //      weight gradients are sums of: dgates [256], dz1 [64], x [64], h_{t-1} [64], in [Din]; per sample the heads'
 //      input n [64].
-//   2. k_critic_grad_partial - the weight gradients as sums over rows (dW_ih = sum dgates^T x, ...), each row range
-//      of a fixed chunking summed by one CTA into its own slot of the workspace.
-//   3. k_critic_grad_sum - the chunk partials summed in chunk order into the caller's tensors.
+//   2. k_grad_partial - the weight gradients as sums over rows (dW_ih = sum dgates^T x, ...), each row range
+//      of a fixed chunking summed by one CTA into its own slot of the workspace (grad_reduce.cu, shared with the
+//      actor's backward).
+//   3. k_grad_sum - the chunk partials summed in chunk order into the caller's tensors.
 // Weight gradients cannot be accumulated next to the 151 KB weight image in shared memory, and a warp's registers do
 // not hold them either: hence the workspace and the reductions.  One sample per warp (the forward runs four): the
 // backward's register arrays leave no room for more, and 148 x 8 warps take B = 1,024 samples in one wave.
@@ -22,6 +23,7 @@
 
 #include "common.cuh"
 #include "critic_launch.h"
+#include "grad_reduce.h"
 #include "launch.h"
 
 namespace mpe {
@@ -34,7 +36,6 @@ constexpr int kG = 4 * kCriticH;  // 256 gate rows
 // per-row record of the workspace (floats): gate activations, overwritten by dgates (reference row order
 // gate * 64 + unit); c_t, overwritten by dz1; x_t = relu(dense1); h_{t-1}; the input row cat(obs, action)
 constexpr int kRec = 512, kRecC = 256, kRecX = 320, kRecHp = 384, kRecIn = 448;
-constexpr int kMaxChunks = 64, kChunkRows = 64;
 
 __device__ __forceinline__ float sigmoid_acc(float x) { return 1.0f / (1.0f + expf(-x)); }
 __device__ __forceinline__ float warp_sum(float v) {
@@ -269,81 +270,6 @@ __global__ void __launch_bounds__(kGradThreads, 1)
   }
 }
 
-// One sum over rows: out[m][k] = sum_r A[r][m] B[r][k] (k < kk), bias[m] = sum_r A[r][m], m < mm <= 64, kk <= 64.
-struct GradTile {
-  const float *a, *b;
-  int64_t rows;
-  int a_stride, b_stride, mm, kk;
-  int out, ldo, bias;  // offsets into one chunk's partial vector; bias < 0: none
-};
-constexpr int kMaxTiles = 12;
-struct GradTiles {
-  GradTile t[kMaxTiles];
-  int nchunk, nout;
-};
-struct GradSeg {
-  float *dst;
-  int src, n;  // src < 0: zeros (dense3 with no upstream dr)
-};
-struct GradSegs {
-  GradSeg s[kCriticGradFields];
-  int nseg, nchunk, nout;
-};
-
-// CTA (tile, chunk): 256 threads, thread (ty, tx) owns out[ty + 16 i][tx + 16 j]; rows are staged 32 at a time
-__global__ void __launch_bounds__(256) k_critic_grad_partial(GradTiles p, float *__restrict__ partial) {
-  __shared__ float As[32][64], Bs[32][64];
-  const GradTile &T = p.t[blockIdx.x];
-  const int tid = threadIdx.x, ty = tid >> 4, tx = tid & 15;
-  const int64_t cs = (T.rows + p.nchunk - 1) / p.nchunk, r0 = (int64_t)blockIdx.y * cs;
-  const int64_t r1 = r0 + cs < T.rows ? r0 + cs : T.rows;
-  float acc[4][4] = {}, bacc = 0.0f;
-  for (int64_t rb = r0; rb < r1; rb += 32) {
-    __syncthreads();
-    for (int i = tid; i < 32 * 64; i += 256) {
-      const int rr = i >> 6, cc = i & 63;
-      const int64_t row = rb + rr;
-      As[rr][cc] = row < r1 && cc < T.mm ? T.a[row * T.a_stride + cc] : 0.0f;
-      Bs[rr][cc] = row < r1 && cc < T.kk ? T.b[row * T.b_stride + cc] : 0.0f;
-    }
-    __syncthreads();
-    const int nr = r1 - rb < 32 ? (int)(r1 - rb) : 32;
-    for (int rr = 0; rr < nr; ++rr) {
-      float av[4], bv[4];
-#pragma unroll
-      for (int i = 0; i < 4; ++i) { av[i] = As[rr][ty + 16 * i]; bv[i] = Bs[rr][tx + 16 * i]; }
-#pragma unroll
-      for (int i = 0; i < 4; ++i)
-#pragma unroll
-        for (int j = 0; j < 4; ++j) acc[i][j] = fmaf(av[i], bv[j], acc[i][j]);
-      if (tid < 64) bacc += As[rr][tid];
-    }
-  }
-  float *P = partial + (int64_t)blockIdx.y * p.nout;
-#pragma unroll
-  for (int i = 0; i < 4; ++i)
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      const int m = ty + 16 * i, k = tx + 16 * j;
-      if (m < T.mm && k < T.kk) P[T.out + m * T.ldo + k] = acc[i][j];
-    }
-  if (T.bias >= 0 && tid < T.mm) P[T.bias + tid] = bacc;
-}
-
-__global__ void __launch_bounds__(256) k_critic_grad_sum(GradSegs p, const float *__restrict__ partial) {
-  int i = blockIdx.x * blockDim.x + threadIdx.x;
-  for (int g = 0; g < p.nseg; ++g) {
-    if (i < p.s[g].n) {
-      float v = 0.0f;
-      if (p.s[g].src >= 0)
-        for (int c = 0; c < p.nchunk; ++c) v += partial[(int64_t)c * p.nout + p.s[g].src + i];
-      p.s[g].dst[i] = v;
-      return;
-    }
-    i -= p.s[g].n;
-  }
-}
-
 namespace {
 
 // Where everything lives: the workspace is [rows][kRec] records, [B][64] heads' inputs, [nchunk][nout] partials;
@@ -357,8 +283,7 @@ struct GradPlan {
 GradPlan grad_plan(const CriticDev &w, int64_t B, int N) {
   GradPlan p;
   p.rows = B * N;
-  p.nchunk = (int)(p.rows < (int64_t)kMaxChunks * kChunkRows ? (p.rows + kChunkRows - 1) / kChunkRows : kMaxChunks);
-  if (p.nchunk < 1) p.nchunk = 1;
+  p.nchunk = grad_chunks(p.rows);
   int off = 0;
   p.o_wih = off; off += kG * kCriticH;
   p.o_whh = off; off += kG * kCriticH;
@@ -428,15 +353,7 @@ cudaError_t launch_critic_backward(const CriticDev &w, const float *obs, const f
   if (dr != nullptr) tiles.t[nt++] = GradTile{dr, ws + p.off_n, B, O, H, O, H, p.o_w3, H, p.o_b3};       // dense3
   tiles.nchunk = p.nchunk;
   tiles.nout = p.nout;
-  k_critic_grad_partial<<<dim3(nt, p.nchunk), 256, 0, st>>>(tiles, ws + p.off_part);
-  if ((e = cudaGetLastError()) != cudaSuccess) return e;
-
-  segs.nchunk = p.nchunk;
-  segs.nout = p.nout;
-  int total = 0;
-  for (int i = 0; i < segs.nseg; ++i) total += segs.s[i].n;
-  k_critic_grad_sum<<<(total + 255) / 256, 256, 0, st>>>(segs, ws + p.off_part);
-  return cudaGetLastError();
+  return launch_grad_reduce(tiles, nt, segs, ws + p.off_part, st);
 }
 
 }  // namespace mpe

@@ -12,7 +12,6 @@ constexpr int kCriticH = 64;        // dense1 width = LSTM input = LSTM hidden (
 constexpr int kCriticMaxIn = 64;    // obs_dim + sum(action widths)
 constexpr int kCriticMaxAgents = 16;
 constexpr int kCriticMaxOut = 4;
-constexpr int kCriticGradFields = 10;  // the pointers of CriticGrads
 
 // Packed fp32 blob in device memory (what a CTA stages into shared memory with one bulk copy)
 struct CriticDev {

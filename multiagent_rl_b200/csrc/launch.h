@@ -36,6 +36,7 @@ inline cudaError_t ensure_smem(size_t bytes, int dev) {
   if (cache && granted[dev] >= bytes) return cudaSuccess;
   cudaError_t e = cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
   if (e == cudaSuccess && cache) granted[dev] = bytes;
+  if (e != cudaSuccess) cudaGetLastError();  // returned here: not left for the next launch's cudaGetLastError
   return e;
 }
 

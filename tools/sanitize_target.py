@@ -125,5 +125,18 @@ for model in (False, True):
     net = m.FusedCriticNetwork(15, 1, model=model).cuda()
     out = net(torch.randn((33, 3, 10), device='cuda'), torch.randn((33, 3, 5), device='cuda'))
     (out[0].sum() + out[1].sum() if model else out.sum()).backward()
+# the actor backward and its reductions at ragged sizes for every head layout: one head, two heads, the model head
+# with and without dnext_state, D = 64; one sample, a partial last CTA, 12 agents
+for D, A, model in ((10, 5, False), (21, [5, 10], False), (16, 5, True), (64, [6, 10], True)):
+    actor = m.FusedActor(random_state_dict(D, A, 7, model_head=model), impl='simt')
+    width = sum(A) if isinstance(A, list) else A
+    for B, N in ((1, 1), (17, 3), (1031, 12)):
+        o = torch.randn((B, N, D), device='cuda')
+        actor.backward(o, torch.randn((B, N, width), device='cuda'),
+                       torch.randn((B, N, D), device='cuda') if model else None, want_obs=True)
+        if model:
+            actor.backward(o, torch.randn((B, N, width), device='cuda'), None, want_obs=True)
+net = m.FusedActorNetwork(10, 5).cuda()
+net(torch.randn((33, 3, 10), device='cuda')).sum().backward()
 torch.cuda.synchronize()
 print('sanitize target done')
