@@ -20,11 +20,15 @@ constexpr int kGateN = 128;     // i, f, g, o gates x 32 units
 // output columns are contiguous:  Wg[dir][k][col'] with col' = ug*8 + gate*2 + uu holding the
 // reference row gate*32 + (ug + 16*uu) of [weight_ih | weight_hh]; biases b_ih + b_hh pre-summed.
 // fp16 hi/lo weight image of the tensor-core path (byte offsets; see tc_kernels.cu)
+// dense2 heads of one direction as a B operand [K = 32 units][24 rows]: head entry a < 8 in row 8 + a, rows 0-7 and
+// 16-23 zero, so that the N = 16 operand starting at row 8 / row 0 puts the heads into columns 0-7 / 8-15
+constexpr int kW2Rows = 24;
+constexpr uint32_t kW2Bytes = (kH / 8) * kW2Rows * 16;
 struct TcDev {
   unsigned char *blob = nullptr;
   uint32_t bytes = 0;
   int D = 0, Kx = 0, A0 = 0, A1 = 0, A = 0;
-  uint32_t off_wih[2][2] = {}, off_whh[2][2] = {}, off_w1[2] = {};
+  uint32_t off_wih[2][2] = {}, off_whh[2][2] = {}, off_w1[2] = {}, off_w2[2][2] = {};
   uint32_t off_w2f = 0, off_bg = 0, off_b1 = 0, off_b2 = 0;
   float *scratch = nullptr;  // tc_scratch_floats(SMs): per-CTA dense2 shares (teams of > 3 agents, two-head actors)
 };

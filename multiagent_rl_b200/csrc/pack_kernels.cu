@@ -84,14 +84,22 @@ __device__ uint32_t actor_tc_word(const TcDev &t, const ActorWeights &w, uint32_
     } else if (o < t.off_w1[0]) {
       const uint32_t q = (o - t.off_whh[0][0]) / (kH * kGateN * 2);
       dir = q >> 1; which = q & 1; base = t.off_whh[dir][which]; rows = kGateN; kind = 1;
-    } else {
+    } else if (o < t.off_w2[0][0]) {
       which = o >= t.off_w1[1] ? 1 : 0; base = t.off_w1[which]; rows = kHid; kind = 2;
+    } else {
+      const uint32_t q = (o - t.off_w2[0][0]) / kW2Bytes;
+      dir = q >> 1; which = q & 1; base = t.off_w2[dir][which]; rows = kW2Rows; kind = 3;
     }
     const int h = (int)(o - base) / 2, n = (h / 8) % rows, k = (h / (8 * rows)) * 8 + h % 8;
     float v0, v1;
     if (kind == 2) {  // dense1: row j = n, columns past D are zero
       v0 = k < t.D ? w.dense1_w[n * t.D + k] : 0.0f;
       v1 = k + 1 < t.D ? w.dense1_w[n * t.D + k + 1] : 0.0f;
+    } else if (kind == 3) {  // dense2 heads: row n = 8 + a holds head entry a < min(A, 8), unit k of direction dir
+      const int a = n - 8;
+      const bool on = a >= 0 && a < 8 && a < t.A;
+      v0 = on ? head_w(w, t.A0, a, dir * kH + k) : 0.0f;
+      v1 = on ? head_w(w, t.A0, a, dir * kH + k + 1) : 0.0f;
     } else {  // gate column n = (u >> 1) * 8 + g * 2 + (u & 1) holds the reference row g * 32 + u
       const int row = ((n >> 1) & 3) * kH + ((n >> 3) << 1) + (n & 1);
       const float *src = kind == 0 ? (dir ? w.w_ih_r : w.w_ih) + row * kHid : (dir ? w.w_hh_r : w.w_hh) + row * kH;
@@ -100,7 +108,7 @@ __device__ uint32_t actor_tc_word(const TcDev &t, const ActorWeights &w, uint32_
     return (uint32_t)split_part(v0, which) | ((uint32_t)split_part(v1, which) << 16);
   }
   float v = 0.0f;
-  if (o < t.off_bg) {  // dense2 heads fp32 [k][16]
+  if (o < t.off_bg) {  // dense2 heads fp32 [k][16] (the FFMA heads of large teams and two-head actors)
     const int r = (int)(o - t.off_w2f) / 4, a = r % 16;
     v = a < t.A ? head_w(w, t.A0, a, r / 16) : 0.0f;
   } else if (o < t.off_b1) {  // gate biases in the ex2 argument form: (b_ih + b_hh) * (-2 | -1) * log2(e)

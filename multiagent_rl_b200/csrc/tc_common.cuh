@@ -92,6 +92,17 @@ __device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&v)[16]) {
       : "r"(taddr)
       : "memory");
 }
+__device__ __forceinline__ void tmem_ld8(uint32_t taddr, uint32_t (&v)[8]) {
+  asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
+               : MPE_R8(v, 0)
+               : "r"(taddr)
+               : "memory");
+}
+__device__ __forceinline__ void tmem_st4(uint32_t taddr, const uint32_t (&v)[4]) {
+  asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1,%2,%3,%4};" ::"r"(taddr), "r"(v[0]), "r"(v[1]),
+               "r"(v[2]), "r"(v[3])
+               : "memory");
+}
 __device__ __forceinline__ void tmem_st32(uint32_t taddr, const uint32_t (&v)[32]) {
   asm volatile(
       "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], "

@@ -37,6 +37,8 @@ void tc_layout(int D, int A0, int A1, TcDev *o) {
   for (int d = 0; d < 2; ++d)
     for (int hl = 0; hl < 2; ++hl) { o->off_whh[d][hl] = off; off += kH * kGateN * 2; }
   for (int hl = 0; hl < 2; ++hl) { o->off_w1[hl] = off; off += (o->Kx > 0 ? o->Kx : 16) * kHid * 2; }
+  for (int d = 0; d < 2; ++d)
+    for (int hl = 0; hl < 2; ++hl) { o->off_w2[d][hl] = off; off += kW2Bytes; }
   o->off_w2f = off; off += kHid * 16 * 4;  // dense2 heads, fp32 [k = dir*32 + unit][16]
   o->off_bg = off; off += 2 * kGateN * 4;
   o->off_b1 = off; off += kHid * 4;
@@ -107,8 +109,9 @@ __device__ unsigned long long g_tc_timeline[148 * 128];
 #define TL(role, i)
 #endif
 
-// barriers of one warpgroup's pipeline (indices into its own block of the barrier array)
-enum { B_X = 0, B_D1, B_H1, B_G, B_H, B_PER_WG };
+// barriers of one warpgroup's pipeline (indices into its own block of the barrier array); B_L: the tile's dense2
+// logits are complete in TMEM (heads on the tensor pipe only)
+enum { B_X = 0, B_D1, B_H1, B_G, B_H, B_L, B_PER_WG };
 
 // operand buffers: all agents resident (N <= 3); a ring of 4 (teams of 4 / 6: 16-wide operands, shared memory to
 // spare) or 2 (9 / 12 agents: 32-wide operands) buffers refilled ahead of the dense1 GEMMs
@@ -166,22 +169,17 @@ __device__ __forceinline__ f2 rcp2_newton(f2 d) {
 // LSTM cell math for 8 units of one env row.  v = 32 gate accumulator columns (scaled by 16) in the packed order
 // [i_a i_b f_a f_b g_a g_b o_a o_b] per pair of units (a, b) = (2p, 2p+1), so that the two cells of a pair sit in
 // adjacent registers and every FP32 operation of the cell is one FFMA2/FADD2/FMUL2.  bg = 32 biases in the same
-// order, pre-multiplied by -log2(e) (x2 for the g gate); c = the 4 packed cell-state pairs; pl = packed dense2
-// partial sums.  The MUFU pipe is the floor of this kernel, so the cell is arranged to need 5 MUFU ops (the five
-// ex2) instead of the textbook 10: with e* = exp(-x) (arguments clamped so that no product overflows)
+// order, pre-multiplied by -log2(e) (x2 for the g gate); c = the 4 packed cell-state pairs.  The MUFU pipe is the
+// floor of this kernel, so the cell is arranged to need 5 MUFU ops (the five ex2) instead of the textbook 10: with
+// e* = exp(-x) (arguments clamped so that no product overflows)
 //   c' = sigmoid(f) c + sigmoid(i) tanh(g) = [c (1+ei)(1+eg) + (1-eg)(1+ef)] / [(1+ef)(1+ei)(1+eg)]   one reciprocal
 //   h  = sigmoid(o) tanh(c') = (1 - ec) / ((1+eo)(1+ec))                                              one reciprocal
 // and both reciprocals (denominators >= 1) by a bit-trick seed + 3 Newton steps on the FMA pipe.
-// Writes h as an fp16 hi/lo K-chunk of the recurrent A operand when `store_h`.
-template <int APAD>
-__device__ __forceinline__ void lstm_chunk(const uint32_t (&v)[32], const float *bg, const float *w2rows, f2 (&c)[4],
-                                           f2 (&pl)[APAD / 2], unsigned char *h_chunk, int row, bool store_h,
-                                           float *hcat8 = nullptr) {
+__device__ __forceinline__ void lstm_h8(const uint32_t (&v)[32], const float *bg, f2 (&c)[4], float (&hv)[8]) {
   const f2 ONE = pk(1.0f, 1.0f), NEG1 = pk(-1.0f, -1.0f);
   const f2 S1 = pk(-kWInv * kLog2e, -kWInv * kLog2e), S2 = pk(-2.0f * kWInv * kLog2e, -2.0f * kWInv * kLog2e);
   const f2 S3 = pk(-2.0f * kLog2e, -2.0f * kLog2e);
   constexpr float kClamp = 40.0f;  // e <= 2^40: sigmoid floors at 9e-13, tanh saturates to 1 - 2e-12
-  float hv[8];
   f2 pO[4];
   // stage 1: exponentials of the four gates, then the new cell state with a single reciprocal
 #pragma unroll
@@ -209,7 +207,27 @@ __device__ __forceinline__ void lstm_chunk(const uint32_t (&v)[32], const float 
     const f2 r = rcp2_newton(mul2(pO[p], add2(eC, ONE)));
     upk(mul2(fma2(eC, NEG1, ONE), r), hv[2 * p], hv[2 * p + 1]);
   }
-  // stage 3: dense2 contribution of relu(h): FFMA2 over pairs of head entries, weights broadcast from smem
+}
+
+// The outputs of 8 units' h: h as an fp16 hi/lo K-chunk of the recurrent A operand when `store_h`, relu(h) for the
+// dense3 head when `hcat8` is set.
+__device__ __forceinline__ void h8_outputs(const float (&hv)[8], unsigned char *h_chunk, int row, bool store_h,
+                                           float *hcat8) {
+  if (store_h) store_chunk_split(h_chunk, h_chunk + 8192, row, hv);
+  if (hcat8 != nullptr) {  // relu(h) of these 8 units for the dense3 head (actor_forward with next_state; 32 B aligned)
+    *reinterpret_cast<float4 *>(hcat8) = make_float4(fmaxf(hv[0], 0.0f), fmaxf(hv[1], 0.0f), fmaxf(hv[2], 0.0f), fmaxf(hv[3], 0.0f));
+    *reinterpret_cast<float4 *>(hcat8 + 4) = make_float4(fmaxf(hv[4], 0.0f), fmaxf(hv[5], 0.0f), fmaxf(hv[6], 0.0f), fmaxf(hv[7], 0.0f));
+  }
+}
+
+// Cell math of 8 units with the dense2 heads on the FMA pipe (teams of > 3, two-head actors): pl = packed dense2
+// partial sums, FFMA2 over pairs of head entries with the weights broadcast from smem.
+template <int APAD>
+__device__ __forceinline__ void lstm_chunk(const uint32_t (&v)[32], const float *bg, const float *w2rows, f2 (&c)[4],
+                                           f2 (&pl)[APAD / 2], unsigned char *h_chunk, int row, bool store_h,
+                                           float *hcat8 = nullptr) {
+  float hv[8];
+  lstm_h8(v, bg, c, hv);
 #pragma unroll
   for (int j = 0; j < 8; ++j) {
     const float rj = fmaxf(hv[j], 0.0f);
@@ -221,11 +239,28 @@ __device__ __forceinline__ void lstm_chunk(const uint32_t (&v)[32], const float 
       pl[a / 2 + 1] = fma2(rr, wv.y, pl[a / 2 + 1]);
     }
   }
-  if (store_h) store_chunk_split(h_chunk, h_chunk + 8192, row, hv);
-  if (hcat8 != nullptr) {  // relu(h) of these 8 units for the dense3 head (actor_forward with next_state; 32 B aligned)
-    *reinterpret_cast<float4 *>(hcat8) = make_float4(fmaxf(hv[0], 0.0f), fmaxf(hv[1], 0.0f), fmaxf(hv[2], 0.0f), fmaxf(hv[3], 0.0f));
-    *reinterpret_cast<float4 *>(hcat8 + 4) = make_float4(fmaxf(hv[4], 0.0f), fmaxf(hv[5], 0.0f), fmaxf(hv[6], 0.0f), fmaxf(hv[7], 0.0f));
+  h8_outputs(hv, h_chunk, row, store_h, hcat8);
+}
+
+// Cell math of 8 units with the dense2 heads on the tensor pipe (teams of <= 3 with one head): relu(h) as fp16 hi/lo
+// pairs into the tile's dense2 A operand in TMEM (4 hi columns at taddr, the lo columns 16 further), read by the
+// issuer's dense2 MMAs once the cell is complete.
+__device__ __forceinline__ void lstm_chunk_tc(const uint32_t (&v)[32], const float *bg, f2 (&c)[4], uint32_t taddr,
+                                              unsigned char *h_chunk, int row, bool store_h, float *hcat8) {
+  float hv[8];
+  lstm_h8(v, bg, c, hv);
+  uint32_t hi[4], lo[4];
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    __half h0, l0, h1, l1;
+    split_f16(fmaxf(hv[2 * i], 0.0f), h0, l0);
+    split_f16(fmaxf(hv[2 * i + 1], 0.0f), h1, l1);
+    hi[i] = pack_h2(h0, h1);
+    lo[i] = pack_h2(l0, l1);
   }
+  tmem_st4(taddr, hi);
+  tmem_st4(taddr + 16, lo);
+  h8_outputs(hv, h_chunk, row, store_h, hcat8);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -238,19 +273,25 @@ __device__ __forceinline__ void lstm_chunk(const uint32_t (&v)[32], const float 
 // (E1 = dense1 epilogue -> h1 operand in TMEM, C = LSTM cell math on the gate accumulators).  While all eight warps
 // run the cell math of one tile, the tensor pipe runs the gate GEMM of the other, so no warp ever waits for an MMA
 // in steady state and every SM sub-partition always has two warps in the same MUFU-heavy phase.
-// Warpgroup h owns tile h for everything that is per env (obs operands, sampling, World.step, outputs); the
-// dense2 sums of the units it does not own reach it through a shared-memory exchange buffer.
+// Warpgroup h owns tile h for everything that is per env (obs operands, sampling, World.step, outputs).  Teams of
+// <= 3 with one head of <= 8 entries run the dense2 heads on the tensor pipe: every cell writes relu(h) into a TMEM
+// A operand and the issuer accumulates [128 x 32] x [32 x 16] per cell into the agent's logit columns, which the
+// owner reads after the pipeline.  Large teams and two-head actors keep FFMA2 heads whose per-cell shares travel
+// through global scratch rows (their TMEM has no room for the logit columns / the heads are 16 entries wide).
 // ------------------------------------------------------------------------------------------------
-__host__ __device__ inline size_t tc2_tile_bytes(int N, int Kx, int APAD) {
-  // obs operands, recurrent h operand, action bytes, and (teams of <= 3 with one head) the dense2 exchange buffer;
-  // larger teams and the two-head simple_reference actor keep the dense2 shares in the global scratch instead
-  return tc_x_bytes(N, Kx) + 16384 + (size_t)((kRows * N * 2 + 127) / 128 * 128) + (N <= 3 && APAD <= 8 ? (size_t)N * APAD * kRows * 4 : 0);
+__host__ __device__ constexpr bool tc2_tc_heads(int N, int APAD) { return N <= 3 && APAD <= 8; }
+// TMEM columns of a tile with the heads on the tensor pipe: logits of agent t at kLogitCol + 8t (one M = 128, N = 16
+// accumulator per pair of agents), the relu(h) A operand (K = 32: 16 hi columns, then 16 lo columns) at kReluCol
+constexpr uint32_t kLogitCol = 192, kReluCol = 224;
+__host__ __device__ inline size_t tc2_tile_bytes(int N, int Kx) {
+  // obs operands, recurrent h operand, action bytes
+  return tc_x_bytes(N, Kx) + 16384 + (size_t)((kRows * N * 2 + 127) / 128 * 128);
 }
 // per tile: operand ring buffer q (< 4) ready / free again.  B2_OBS has no waiter; it stays (with its mbar_init)
 // because without it ptxas reschedules the large-team kernels, a change that wants its own measurement.
 enum { B2_XR = 0, B2_XF = 4, B2_OBS = 8, B2_EXTRA = 9 };
-__host__ __device__ inline size_t tc2_smem_bytes(uint32_t wbytes, int N, int Kx, int APAD) {
-  return (size_t)wbytes + 2 * tc2_tile_bytes(N, Kx, APAD) + (1 + 2 * B_PER_WG + 2 * B2_EXTRA) * 8 + 64;
+__host__ __device__ inline size_t tc2_smem_bytes(uint32_t wbytes, int N, int Kx) {
+  return (size_t)wbytes + 2 * tc2_tile_bytes(N, Kx) + (1 + 2 * B_PER_WG + 2 * B2_EXTRA) * 8 + 64;
 }
 // dense2 shares of large teams: [CTA][tile 0/1][warpgroup half][cell 0..2N-1][APAD/2 packed pairs][128 rows] f2
 __host__ __device__ inline size_t tc2_scratch_f2_per_cta(int N, int APAD) { return (size_t)2 * 2 * 2 * N * (APAD / 2) * kRows; }
@@ -268,9 +309,11 @@ __global__ void __launch_bounds__(tc2_threads(N), 1)
   // the earlier two-pipeline kernel; a service warp that also samples one cell behind the pipeline - its ~11 k
   // instructions per tile slow the two sub-partitions it shares and with them the whole barrier-coupled pipeline.)
   constexpr bool kJit = N > 3;
-  // two-head actors of small teams (simple_reference, A = 5 + 10): the exchange buffer does not fit into shared memory
-  // any more, so the OTHER warpgroup's shares travel through the scratch rows as well (the own shares stay in registers)
+  // two-head actors of small teams (simple_reference, A = 5 + 10) keep the FFMA heads too: the OTHER warpgroup's
+  // shares travel through the scratch rows (the own shares stay in registers)
   constexpr bool kXs = !kJit && APAD > 8;
+  // every other small team (one head of <= 8 entries): the heads on the tensor pipe, logits accumulated in TMEM
+  constexpr bool kTcHeads = tc2_tc_heads(N, APAD);
   static_assert(!(kJit && FUSED), "the fused rollout keeps every agent of an env in one thread: N <= 3");
   extern __shared__ __align__(128) unsigned char smem[];
 #ifdef MPE_TC_PHASES
@@ -287,7 +330,7 @@ __global__ void __launch_bounds__(tc2_threads(N), 1)
   const int Kx = w.Kx;
   const int tid = threadIdx.x, warp = tid >> 5;
   const size_t xb = tc_x_bytes(N, Kx);
-  const size_t tile_bytes = tc2_tile_bytes(N, Kx, APAD);
+  const size_t tile_bytes = tc2_tile_bytes(N, Kx);
   unsigned char *sm_w = smem;
   uint64_t *bars = reinterpret_cast<uint64_t *>(smem + w.bytes + 2 * tile_bytes);  // [0] = weights, then 2 x B_PER_WG
   uint64_t *xbars = bars + 1 + 2 * B_PER_WG;  // [tile][B2_XR + buf | B2_XF + buf]
@@ -303,6 +346,7 @@ __global__ void __launch_bounds__(tc2_threads(N), 1)
       mbar_init(&bb[B_H1], 256);  // both warpgroups converted their half of h1
       mbar_init(&bb[B_G], 1);
       mbar_init(&bb[B_H], 256);   // both warpgroups finished their half of the cell
+      mbar_init(&bb[B_L], 1);
       for (int q = 0; q < 4; ++q) {
         mbar_init(&xbars[g * B2_EXTRA + B2_XR + q], 32);  // the service warp filled operand buffer q
         mbar_init(&xbars[g * B2_EXTRA + B2_XF + q], 1);   // the dense1 GEMM reading buffer q has completed
@@ -319,14 +363,17 @@ __global__ void __launch_bounds__(tc2_threads(N), 1)
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
   const int T = FUSED ? ro.T : 1;
-  // TMEM columns of a tile: gate accumulators [0,128) and two 64-column h1 slots at 128 / 192.  A slot first
-  // receives the dense1 accumulators of an agent and is then converted IN PLACE into that agent's h1 operand
-  // (thread half h owns columns [32h, 32h+32) of the slot: fp16 hi pairs in the first 16, lo pairs in the last 16).
-  // Agent t lives in slot t & 1, so the backward pass finds the h1 of agents N-1 and N-2 still resident and only
-  // agents that were overwritten (t + 2 < N) are recomputed: 4 dense1 GEMMs + epilogues per tile instead of 6.
+  // TMEM columns of a tile: gate accumulators [0,128) and 64-column h1 slots from 128 on.  A slot first receives the
+  // dense1 accumulators of an agent and is then converted IN PLACE into that agent's h1 operand (thread half h owns
+  // columns [32h, 32h+32) of the slot: fp16 hi pairs in the first 16, lo pairs in the last 16).  With the heads on
+  // the FMA pipe there are two slots (128 / 192) and agent t lives in slot t & 1, so the backward pass finds the h1 of
+  // agents N-1 and N-2 still resident: 4 dense1 GEMMs + epilogues per 3-agent tile instead of 6.  With the heads on
+  // the tensor pipe [192, 256) holds the logits and the relu(h) operand, one slot remains, and the backward pass
+  // recomputes every agent but N-1: 5 dense1 GEMMs + epilogues per 3-agent tile, 3 per 2-agent tile.
+  constexpr int kSlots = kTcHeads ? 1 : 2;
   auto agent_of = [](int k) { return k < N ? k : 2 * N - 1 - k; };
-  auto need_e1 = [&](int k) { return k < N || agent_of(k) + 2 < N; };
-  auto slot_col = [](int t) { return 128u + 64u * (uint32_t)(t & 1); };
+  auto need_e1 = [&](int k) { return k < N || agent_of(k) + kSlots < N; };
+  auto slot_col = [](int t) { return 128u + 64u * (uint32_t)(t % kSlots); };
   const int64_t npairs = (ntiles + 1) / 2;
   // large teams: index of cell j in the sequence of cells that have a dense1 GEMM (the two resident backward cells
   // N, N+1 are skipped); the operand ring buffer of that GEMM is (index mod ring depth)
@@ -403,7 +450,7 @@ __global__ void __launch_bounds__(tc2_threads(N), 1)
       const uint32_t tmem = tmem_base + X * 256;
       uint32_t ph_x = 0, ph_h1 = 0, ph_h = 0, ph_xr = 0;  // ph_xr: bit q = phase parity of ring buffer q
       uint64_t *xb2 = xbars + X * B2_EXTRA;
-      const uint32_t id_g = make_idesc_f16(128, 128), id_d1 = make_idesc_f16(128, 64);
+      const uint32_t id_g = make_idesc_f16(128, 128), id_d1 = make_idesc_f16(128, 64), id_l = make_idesc_f16(128, 16);
       mbar_wait(&bars[0], 0);
       for (int64_t pair = blockIdx.x; pair < npairs; pair += gridDim.x) {
         for (int it = 0; it < T; ++it) {
@@ -424,11 +471,29 @@ __global__ void __launch_bounds__(tc2_threads(N), 1)
             mma_commit(&bb[B_D1]);
             if constexpr (kJit) mma_commit(&xb2[B2_XF + q]);
           };
+          // dense2 heads of cell j, once both warpgroups have written its relu(h): agent t accumulates into columns
+          // 8t..8t+7 of its pair's N = 16 accumulator (B operand starting at row 8 for even agents, row 0 for odd ones,
+          // the other 8 columns are zero weights).  An even agent's forward cell starts the pair's sums.  Issued
+          // before the tile's next gate GEMM, whose B_G commit the next cell's math (which rewrites relu(h)) waits on.
+          auto dense2_cell = [&](int j) {
+            const int t = agent_of(j), d = j >= N ? 1 : 0;
+            const uint32_t boff = (t & 1) ? 0u : 128u;
+            const unsigned char *w2_hi = sm_w + (d ? w.off_w2[1][0] : w.off_w2[0][0]) + boff;
+            const unsigned char *w2_lo = sm_w + (d ? w.off_w2[1][1] : w.off_w2[0][1]) + boff;
+            mma3_ts(tmem + kLogitCol + 16u * (uint32_t)(t >> 1), tmem + kReluCol, tmem + kReluCol + 16, w2_hi, w2_lo,
+                    kW2Rows * 16, 2, id_l, d == 1 || (t & 1) == 1);
+          };
           dense1_cell(0);
           for (int k = 0; k < 2 * N; ++k) {
             const int d = k >= N ? 1 : 0, st = k - d * N;
+            if (k > 0) {
+              mbar_wait(&bb[B_H], ph_h); ph_h ^= 1;
+              if constexpr (kTcHeads) {
+                tc_fence_after();
+                dense2_cell(k - 1);
+              }
+            }
             if (need_e1(k)) { mbar_wait(&bb[B_H1], ph_h1); ph_h1 ^= 1; }
-            if (k > 0) { mbar_wait(&bb[B_H], ph_h); ph_h ^= 1; }
             tc_fence_after();
             const uint32_t a0 = tmem + slot_col(agent_of(k));  // K blocks 0,1 from half 0 of the slot, 2,3 from half 1
             const unsigned char *wih_hi = sm_w + (d ? w.off_wih[1][0] : w.off_wih[0][0]);
@@ -438,11 +503,17 @@ __global__ void __launch_bounds__(tc2_threads(N), 1)
             if (st > 0) mma3_ss(tmem, sm_h, sm_h + 8192, kChunkA, sm_w + (d ? w.off_whh[1][0] : w.off_whh[0][0]),
                                 sm_w + (d ? w.off_whh[1][1] : w.off_whh[0][1]), kGateN * 16, 2, id_g, true);
             mma_commit(&bb[B_G]);
-            // the next cell's dense1 goes behind this gate GEMM; its slot held agent (next - 2), whose last reader
-            // was issued before this point (the tensor pipe executes in order)
+            // the next cell's dense1 goes behind this gate GEMM; its slot held the agent kSlots cells back, whose
+            // last reader (with one slot: this gate GEMM) was issued before this point (the tensor pipe executes in
+            // order)
             if (k + 1 < 2 * N && need_e1(k + 1)) dense1_cell(k + 1);
           }
           mbar_wait(&bb[B_H], ph_h); ph_h ^= 1;
+          if constexpr (kTcHeads) {
+            tc_fence_after();
+            dense2_cell(2 * N - 1);
+            mma_commit(&bb[B_L]);
+          }
         }
       }
     }
@@ -456,9 +527,8 @@ __global__ void __launch_bounds__(tc2_threads(N), 1)
     const float *w2f = reinterpret_cast<const float *>(sm_w + w.off_w2f);
     unsigned char *own_x = tile_smem(own), *own_h = own_x + xb;
     uint8_t *own_act = own_h + 16384;
-    [[maybe_unused]] const f2 *own_xchg2 = reinterpret_cast<const f2 *>(own_act + (kRows * N * 2 + 127) / 128 * 128);
     float *stage_obs = reinterpret_cast<float *>(own_x), *stage_rew = stage_obs + kRows * R;
-    uint32_t ph_d1[2] = {0, 0}, ph_g[2] = {0, 0};
+    uint32_t ph_d1[2] = {0, 0}, ph_g[2] = {0, 0}, ph_l = 0;
     bool tma_pending = false;  // row 0: a bulk store of the staging buffer (= the obs operand buffer) may still be reading it
     // large teams: this CTA's dense2-share scratch, [tile][half][cell][pair of head entries][row]
     f2 *scr = (kJit || kXs) ? reinterpret_cast<f2 *>(w.scratch) + (size_t)blockIdx.x * tc2_scratch_f2_per_cta(N, APAD) : nullptr;
@@ -525,15 +595,17 @@ __global__ void __launch_bounds__(tc2_threads(N), 1)
         }
         if constexpr (!kJit) {
           fence_proxy_async_smem();
+          if constexpr (kTcHeads) tc_fence_before();  // the previous step's logit loads precede the next MMAs
           mbar_arrive(&bars[1 + own * B_PER_WG + B_X]);
         }
 
         if (!have_w) { mbar_wait(&bars[0], 0); have_w = true; }
-        // dense2 sums of the OWN tile's rows over this thread's 16 units, packed pairs of head entries (large teams:
-        // just the bias, the shares come from the scratch rows).  Small teams add the bias after the two warpgroups'
-        // sums: (own + other) + bias rounds the same whichever warpgroup owns the tile, so an env's logits do not depend
-        // on the parity of its tile, i.e. on where it sits in the batch (HostRollout shards start anywhere)
-        constexpr int NLG = kJit ? 1 : N;
+        // FFMA heads: dense2 sums of the OWN tile's rows over this thread's 16 units, packed pairs of head entries
+        // (large teams: just the bias, the shares come from the scratch rows).  Two-head actors add the bias after the
+        // two warpgroups' sums: (own + other) + bias rounds the same whichever warpgroup owns the tile, so an env's
+        // logits do not depend on the parity of its tile, i.e. on where it sits in the batch (HostRollout shards start
+        // anywhere).  Unused with the heads on the tensor pipe, whose sums are the same MMAs for every tile.
+        constexpr int NLG = kXs ? N : 1;
         f2 lgp[NLG][APAD / 2];
 #pragma unroll
         for (int t = 0; t < NLG; ++t)
@@ -575,7 +647,8 @@ __global__ void __launch_bounds__(tc2_threads(N), 1)
           mbar_arrive(&bb[B_H1]);
           TS(3);
         };
-        // C(X, k): LSTM cell k of tile X on this thread's 16 units; dense2 share to lgp (own tile) or the exchange
+        // C(X, k): LSTM cell k of tile X on this thread's 16 units; relu(h) to the tile's dense2 operand in TMEM, or
+        // (FFMA heads) the dense2 share to lgp (own tile) or the scratch rows
         auto CC = [&](auto XT, int k, f2 (&c)[2][4]) {
           constexpr int X = decltype(XT)::value;
           const int d = k >= N ? 1 : 0, st = k - d * N;
@@ -588,10 +661,12 @@ __global__ void __launch_bounds__(tc2_threads(N), 1)
             for (int q = 0; q < 4; ++q) c[0][q] = c[1][q] = 0ull;
           }
           const float *bg = reinterpret_cast<const float *>(sm_w + w.off_bg) + d * kGateN + half * 64;
-          const float *w2d = w2f + (d * kH + half * 16) * 16;
-          f2 pl[APAD / 2];
+          [[maybe_unused]] const float *w2d = w2f + (d * kH + half * 16) * 16;
+          [[maybe_unused]] f2 pl[APAD / 2];
+          if constexpr (!kTcHeads) {
 #pragma unroll
-          for (int a = 0; a < APAD / 2; ++a) pl[a] = 0ull;
+            for (int a = 0; a < APAD / 2; ++a) pl[a] = 0ull;
+          }
           TS(9);
           mbar_wait(&bb[B_G], ph_g[X]); ph_g[X] ^= 1;
           tc_fence_after();
@@ -611,12 +686,24 @@ __global__ void __launch_bounds__(tc2_threads(N), 1)
             tmem_wait_ld();
             TS(5);
             tmem_ld32(tmem + lane_base + half * 64 + 32, vb);  // in flight during the first chunk's math
-            lstm_chunk<APAD>(va, bg, w2d, c[0], pl, sm_h + (2 * half) * kChunkA, row, st < N - 1, hc);
-            TS(6);
-            tmem_wait_ld();
-            TS(7);
-            lstm_chunk<APAD>(vb, bg + 32, w2d + 8 * 16, c[1], pl, sm_h + (2 * half + 1) * kChunkA, row, st < N - 1,
-                             hc != nullptr ? hc + 8 : nullptr);
+            if constexpr (kTcHeads) {
+              // this thread's 16 units are K rows 16 half .. 16 half + 15 of the operand: hi columns 8 half .. 8 half + 7
+              const uint32_t trelu = tmem + lane_base + kReluCol + half * 8;
+              lstm_chunk_tc(va, bg, c[0], trelu, sm_h + (2 * half) * kChunkA, row, st < N - 1, hc);
+              TS(6);
+              tmem_wait_ld();
+              TS(7);
+              lstm_chunk_tc(vb, bg + 32, c[1], trelu + 4, sm_h + (2 * half + 1) * kChunkA, row, st < N - 1,
+                            hc != nullptr ? hc + 8 : nullptr);
+              tmem_wait_st();
+            } else {
+              lstm_chunk<APAD>(va, bg, w2d, c[0], pl, sm_h + (2 * half) * kChunkA, row, st < N - 1, hc);
+              TS(6);
+              tmem_wait_ld();
+              TS(7);
+              lstm_chunk<APAD>(vb, bg + 32, w2d + 8 * 16, c[1], pl, sm_h + (2 * half + 1) * kChunkA, row, st < N - 1,
+                               hc != nullptr ? hc + 8 : nullptr);
+            }
           }
           fence_proxy_async_smem();
           tc_fence_before();
@@ -628,26 +715,18 @@ __global__ void __launch_bounds__(tc2_threads(N), 1)
             f2 *dst = scr + ((size_t)((X * 2 + half) * 2 * N + k) * (APAD / 2)) * kRows + row;
 #pragma unroll
             for (int a = 0; a < APAD / 2; ++a) dst[a * kRows] = pl[a];
-          } else if (X == own) {
+          } else if constexpr (kXs) {
+            if (X == own) {
 #pragma unroll
-            for (int tt = 0; tt < NLG; ++tt)
-              if (tt == t) {
+              for (int tt = 0; tt < NLG; ++tt)
+                if (tt == t) {
 #pragma unroll
-                for (int a = 0; a < APAD / 2; ++a) lgp[tt][a] = add2(lgp[tt][a], pl[a]);
-              }
-          } else if constexpr (kXs) {  // the other tile's rows: one scratch row per cell, summed by the owner
-            f2 *dst = scr + ((size_t)((X * 2 + half) * 2 * N + k) * (APAD / 2)) * kRows + row;
+                  for (int a = 0; a < APAD / 2; ++a) lgp[tt][a] = add2(lgp[tt][a], pl[a]);
+                }
+            } else {  // the other tile's rows: one scratch row per cell, summed by the owner
+              f2 *dst = scr + ((size_t)((X * 2 + half) * 2 * N + k) * (APAD / 2)) * kRows + row;
 #pragma unroll
-            for (int a = 0; a < APAD / 2; ++a) dst[a * kRows] = pl[a];
-          } else {  // the other tile's rows: park this warpgroup's share for its owner (store, then add)
-            f2 *xr = reinterpret_cast<f2 *>(tile_smem(X) + xb + 16384 + (kRows * N * 2 + 127) / 128 * 128) +
-                     (size_t)t * (APAD / 2) * kRows + row;
-            if (d == 0) {
-#pragma unroll
-              for (int a = 0; a < APAD / 2; ++a) xr[a * kRows] = pl[a];
-            } else {
-#pragma unroll
-              for (int a = 0; a < APAD / 2; ++a) xr[a * kRows] = add2(xr[a * kRows], pl[a]);
+              for (int a = 0; a < APAD / 2; ++a) dst[a * kRows] = pl[a];
             }
           }
         };
@@ -672,7 +751,12 @@ __global__ void __launch_bounds__(tc2_threads(N), 1)
           for (int i = 0; i < 10; ++i) g_tc_timeline[blockIdx.x * 128 + 96 + half * 10 + i] = acc[i];
         }
 #endif
-        bar_sync_n(1, 256);  // the exchange buffers / scratch shares of both warpgroups are complete
+        if constexpr (kTcHeads) {
+          mbar_wait(&bars[1 + own * B_PER_WG + B_L], ph_l); ph_l ^= 1;
+          tc_fence_after();
+        } else {
+          bar_sync_n(1, 256);  // the scratch shares of both warpgroups are complete
+        }
         TL(half, 14);
 
         // ---- own tile: Gumbel-max sampling ----
@@ -773,6 +857,12 @@ __global__ void __launch_bounds__(tc2_threads(N), 1)
           const uint64_t step = FUSED ? ro.step0 + (uint64_t)it : io.step;
           const uint64_t seed = FUSED ? s.seed : io.seed;
           const int64_t gid0 = FUSED ? s.gid0 : io.gid0;
+          // heads on the tensor pipe: the 16-fold logit sums of agent t in columns 8t..8t+7, loaded behind the noise
+          [[maybe_unused]] uint32_t lv[N][8];
+          if constexpr (kTcHeads) {
+#pragma unroll
+            for (int t = 0; t < N; ++t) tmem_ld8(tmem_base + own * 256 + lane_base + kLogitCol + 8 * t, lv[t]);
+          }
           // Gumbel noise of all N agents of this row up front: the N * APAD/4 Philox blocks advance together and
           // the log chains of the values run in lock-step (see bits_to_gumbel_batch)
           float gn[N][APAD];
@@ -826,22 +916,21 @@ __global__ void __launch_bounds__(tc2_threads(N), 1)
               }
             }
           }
+          if constexpr (kTcHeads) tmem_wait_ld();
 #pragma unroll
           for (int t = 0; t < N; ++t) {
             float z[APAD];
             float lgt[APAD];
+            if constexpr (kTcHeads) {
 #pragma unroll
-            for (int a = 0; a < APAD / 2; ++a)
-            {
-              f2 other;
-              if constexpr (kXs) {
+              for (int a = 0; a < APAD; ++a) lgt[a] = fmaf(__uint_as_float(lv[t][a]), kWInv, b2[a]);  // x 1/16: exact
+            } else {
+#pragma unroll
+              for (int a = 0; a < APAD / 2; ++a) {
                 const f2 *sf = scr + ((size_t)((own * 2 + (1 - half)) * 2 * N + t) * (APAD / 2) + a) * kRows + row;
                 const f2 *sb = scr + ((size_t)((own * 2 + (1 - half)) * 2 * N + (2 * N - 1 - t)) * (APAD / 2) + a) * kRows + row;
-                other = add2(*sf, *sb);
-              } else {
-                other = own_xchg2[((size_t)t * (APAD / 2) + a) * kRows + row];
+                upk(add2(add2(lgp[t][a], add2(*sf, *sb)), pk(b2[2 * a], b2[2 * a + 1])), lgt[2 * a], lgt[2 * a + 1]);
               }
-              upk(add2(add2(lgp[t][a], other), pk(b2[2 * a], b2[2 * a + 1])), lgt[2 * a], lgt[2 * a + 1]);
             }
             const int64_t orow = b * N + t;
 #pragma unroll
@@ -971,7 +1060,7 @@ __global__ void __launch_bounds__(tc2_threads(N), 1)
             }
         }
         TL(half, 30);
-        bar_sync_n(1, 256);  // exchange and action buffers of both tiles are free again (staging: see tma_pending)
+        bar_sync_n(1, 256);  // action buffers of both tiles are free again (staging: see tma_pending)
         TL(half, 31);
       }
     }
@@ -1004,7 +1093,7 @@ template <int SC, int N, bool FUSED, int APAD>
 static cudaError_t launch_tc2_t(const EnvState<float> &s, const TcDev &w, const ActorIO &io, const RolloutIO &ro,
                                 int max_episode_len, int64_t nenvs, cudaStream_t st) {
   const int dev = current_device();
-  const size_t smem = tc2_smem_bytes(w.bytes, N, w.Kx, APAD);
+  const size_t smem = tc2_smem_bytes(w.bytes, N, w.Kx);
   if (smem > 227 * 1024) return cudaErrorInvalidValue;  // tc_*_supported rule these out
   cudaError_t e = ensure_smem<k_tc2<SC, N, FUSED, APAD>>(smem, dev);
   if (e != cudaSuccess) return e;
