@@ -35,7 +35,7 @@
 extern "C" {
 #endif
 
-#define MPE_ABI_VERSION 8
+#define MPE_ABI_VERSION 9
 
 enum { MPE_OK = 0, MPE_EINVAL = -1, MPE_ECUDA = -2, MPE_EUNSUPPORTED = -3 };
 enum { MPE_SIMPLE_SPREAD = 0, MPE_SIMPLE_REFERENCE = 1, MPE_SIMPLE_SPEAKER_LISTENER = 2,
@@ -247,10 +247,14 @@ int actor_backward(MpeActor *actor, const float *obs, int64_t B, int32_t N, cons
 /* The loop body of experiments/run.py:36-65 fused: for t in [0, T): observe -> actor -> sample ->
  * step -> reward -> (episode_step == max_episode_len ? reset), state never leaving the SM between
  * the actor and the physics.  F32 envs only.  Per-step outputs (each may be NULL) are written
- * at [t][...]: obs_next [T][B][N][D], rew [T][B][N], act_u [T][B][N], act_c [T][B][N].
+ * at [t][...]: obs_next [T][B][N][D], rew [T][B][N], act_u [T][B][N], act_c [T][B][N],
+ * info_i [T][B][N+1] int32 and info_f [T][B] fp32: benchmark_data, at [t] bit for bit what mpe_step writes to its
+ * info_i / info_f for that step (collisions per agent + occupied landmarks, and min_dists; for
+ * MPE_COLLECT_TREASURE the 0 / 1 flags per agent + a zero, and info_f is not written).  A NULL output changes
+ * nothing else the call writes.
  * `step0` is the global step index of t = 0 (keys the Gumbel stream). */
 int mpe_rollout(MpeEnv *env, MpeActor *actor, int32_t T, uint64_t step0, float *obs_next, float *rew,
-                int32_t *act_u, int32_t *act_c, void *stream);
+                int32_t *act_u, int32_t *act_c, int32_t *info_i, void *info_f, void *stream);
 
 /* ---- critic: rls/model/ac_network_multi_gumbel.py:70-148 (main.py path) and
  * rls/model/ac_network_model_multi_gumbel.py:69-143 ("+model": extra reward head, no relu after the attention).
@@ -343,13 +347,14 @@ int replay_sample(MpeReplay *replay, int64_t batch, const int64_t *idx, uint64_t
  * obs_{t+1}, done = 0), where obs_t is the observation the actor acted on (the post-reset observation at an episode's
  * first step) and obs_{t+1} the one the step returned (before any reset).  Step-major, then env order: the ring ends
  * up as after T replay_add calls of B transitions each, wrapping as often as T * B / capacity says.  Recordings,
- * env state, Philox streams and episode statistics are those of mpe_rollout; the recording pointers may be NULL.
+ * env state, Philox streams, episode statistics and info_i / info_f are those of mpe_rollout; the recording pointers
+ * may be NULL.
  * The ring must match the env and actor (num_agents, obs_dim, act0 / act1), sit on their device and hold at least
  * B transitions; otherwise MPE_EINVAL before anything is launched.  Envs whose episodes are aligned (after an
  * unmasked reset) run the fused kernel in segments up to each episode end and one ring-writer launch per segment;
  * others run per-step kernels with one replay_add per step. */
 int mpe_rollout_replay(MpeEnv *env, MpeActor *actor, MpeReplay *replay, int32_t T, uint64_t step0, float *obs_next,
-                       float *rew, int32_t *act_u, int32_t *act_c, void *stream);
+                       float *rew, int32_t *act_u, int32_t *act_c, int32_t *info_i, void *info_f, void *stream);
 
 #ifdef __cplusplus
 }

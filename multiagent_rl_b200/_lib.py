@@ -7,7 +7,7 @@ import os
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get('MPE_B200_LIB', os.path.join(HERE, 'libmpe_b200.so'))  # override: A/B builds
-ABI_VERSION = 8
+ABI_VERSION = 9
 
 MPE_OK, MPE_EINVAL, MPE_ECUDA, MPE_EUNSUPPORTED = 0, -1, -2, -3
 SCENARIO_IDS = {'simple_spread': 0, 'simple_reference': 1, 'simple_speaker_listener': 2, 'fullobs_collect_treasure': 3}
@@ -103,7 +103,7 @@ SIGNATURES = {
     'actor_forward_host': (C.c_int, [P, P, C.c_int64, C.c_int32, C.c_uint64, C.c_uint64, C.c_int64, P, P, P, P]),
     'actor_backward_workspace': (C.c_int64, [P, C.c_int64, C.c_int32]),
     'actor_backward': (C.c_int, [P, P, C.c_int64, C.c_int32, P, P, P, C.POINTER(ActorGrads), P, C.c_int64, P]),
-    'mpe_rollout': (C.c_int, [P, P, C.c_int32, C.c_uint64, P, P, P, P, P]),
+    'mpe_rollout': (C.c_int, [P, P, C.c_int32, C.c_uint64, P, P, P, P, P, P, P]),
     'critic_create': (C.c_int, [C.POINTER(CriticConfig), C.POINTER(P)]),
     'critic_destroy': (C.c_int, [P]),
     'critic_load': (C.c_int, [P, C.POINTER(CriticWeights), P]),
@@ -118,8 +118,20 @@ SIGNATURES = {
     'replay_next_idx': (C.c_int64, [P]),
     'replay_add': (C.c_int, [P, P, P, P, P, P, P, C.c_int64, P]),
     'replay_sample': (C.c_int, [P, C.c_int64, P, C.c_uint64, P, P, P, P, P, P, P]),
-    'mpe_rollout_replay': (C.c_int, [P, P, P, C.c_int32, C.c_uint64, P, P, P, P, P]),
+    'mpe_rollout_replay': (C.c_int, [P, P, P, C.c_int32, C.c_uint64, P, P, P, P, P, P, P]),
 }
+# ABI version 9 added the info_i / info_f outputs just before the stream; a call from Python may still pass the
+# version-8 argument list without them, which records no benchmark_data
+_INFO_BEFORE_STREAM = ('mpe_rollout', 'mpe_rollout_replay')
+
+
+def _info_optional(fn, nargs):
+    def call(*args):
+        if len(args) == nargs - 2:
+            args = args[:-1] + (None, None) + args[-1:]
+        return fn(*args)
+    call.__name__ = fn.__name__
+    return call
 
 _lib = None
 
@@ -138,6 +150,8 @@ def load():
         fn = getattr(lib, name)  # AttributeError here = header/library mismatch
         fn.restype = res
         fn.argtypes = args
+        if name in _INFO_BEFORE_STREAM:
+            setattr(lib, name, _info_optional(fn, len(args)))
     v = lib.mpe_abi_version()
     if v != ABI_VERSION:
         raise RuntimeError('libmpe_b200.so ABI version %d, python binding expects %d: rebuild' % (v, ABI_VERSION))

@@ -71,6 +71,8 @@ struct RolloutIO {
   float *obs_next = nullptr;  // [T][B][N][D]
   float *rew = nullptr;       // [T][B][N]
   int32_t *act_u = nullptr, *act_c = nullptr;  // [T][B][N]
+  int32_t *info_i = nullptr;  // [T][B][N+1] benchmark_data: collisions per agent, occupied landmarks (mpe_step's info_i)
+  float *info_f = nullptr;    // [T][B] benchmark_data: sum of min distances (mpe_step's info_f)
 };
 
 void actor_layout(int D, int A0, int A1, bool has_model, ActorDev *out);

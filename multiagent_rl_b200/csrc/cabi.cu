@@ -720,7 +720,8 @@ static int check_rollout(const MpeEnv *env, const MpeActor *actor, const char *w
 // arithmetic: bit-identical to the stepwise calls.  With `rep`, each step's B transitions are appended after the step
 // and before the reset overwrites the observations: obs_t is `cur`, obs_{t+1} is `o`.
 static int rollout_stepwise(MpeEnv *env, MpeActor *actor, MpeReplay *rep, int32_t T, uint64_t step0, float *obs_next,
-                            float *rew, int32_t *act_u, int32_t *act_c, cudaStream_t st) {
+                            float *rew, int32_t *act_u, int32_t *act_c, int32_t *info_i, float *info_f,
+                            cudaStream_t st) {
   mpe::EnvStateAny s = env->st;
   s.track = 1;
   const int64_t rows = s.B * s.N;
@@ -743,7 +744,9 @@ static int rollout_stepwise(MpeEnv *env, MpeActor *actor, MpeReplay *rep, int32_
     float *o = obs_next != nullptr ? obs_next + (int64_t)t * rows * s.D
                                    : (rep != nullptr && cur == env->r_obs ? env->r_obs2 : env->r_obs);
     float *r = rew != nullptr ? rew + (int64_t)t * rows : (rep != nullptr ? env->r_rew : nullptr);
-    CK(mpe::launch_step(s, aio.act_u, aio.act_c, nullptr, o, r, nullptr, nullptr, nullptr, st));
+    int32_t *ii = info_i != nullptr ? info_i + (int64_t)t * s.B * (s.N + 1) : nullptr;
+    float *fi = info_f != nullptr ? info_f + (int64_t)t * s.B : nullptr;
+    CK(mpe::launch_step(s, aio.act_u, aio.act_c, nullptr, o, r, nullptr, ii, fi, st));
     if (rep != nullptr) {
       CK(mpe::launch_replay_add(rep->dev, rep->head, s.B, cur, aio.act_u, aio.act_c, r, o, nullptr, st));
       rep->head = (rep->head + s.B) % rep->dev.capacity;
@@ -762,7 +765,7 @@ static int rollout_stepwise(MpeEnv *env, MpeActor *actor, MpeReplay *rep, int32_
 }
 
 int mpe_rollout(MpeEnv *env, MpeActor *actor, int32_t T, uint64_t step0, float *obs_next, float *rew, int32_t *act_u,
-                int32_t *act_c, void *stream) {
+                int32_t *act_c, int32_t *info_i, void *info_f, void *stream) {
   if (env == nullptr || actor == nullptr) return fail(MPE_EINVAL, "mpe_rollout: null handle");
   if (T <= 0) return MPE_OK;
   if (int rc = check_rollout(env, actor, "mpe_rollout")) return rc;
@@ -773,13 +776,15 @@ int mpe_rollout(MpeEnv *env, MpeActor *actor, int32_t T, uint64_t step0, float *
   if (use_fused_rollout(env, actor)) {
     mpe::RolloutIO io;
     io.T = T; io.step0 = step0; io.obs_next = obs_next; io.rew = rew; io.act_u = act_u; io.act_c = act_c;
+    io.info_i = info_i; io.info_f = static_cast<float *>(info_f);
     mpe::TcDev tcw;
     CK(tc_for_stream(actor, env->st.N, &env->tc_scratch, &tcw));  // rollouts of several envs may share one actor
     CK(mpe::launch_rollout_tc(env->st, tcw, io, st));
     advance_episode_step(env, T);
     return MPE_OK;
   }
-  return rollout_stepwise(env, actor, nullptr, T, step0, obs_next, rew, act_u, act_c, st);
+  return rollout_stepwise(env, actor, nullptr, T, step0, obs_next, rew, act_u, act_c, info_i,
+                          static_cast<float *>(info_f), st);
 }
 
 // The fused path of mpe_rollout_replay keeps the recordings the caller does not take in an env-owned scratch of at
@@ -794,7 +799,8 @@ constexpr size_t kRolloutReplayScratchBytes = size_t(1) << 30;
 // observation before the segment (mpe_observe after an episode end: the post-reset observation; else a copy of the
 // last step's obs_next) and of every later step from the previous step's obs_next.
 static int rollout_fused_replay(MpeEnv *env, MpeActor *actor, MpeReplay *rep, int32_t T, uint64_t step0, float *obs_next,
-                                float *rew, int32_t *act_u, int32_t *act_c, cudaStream_t st) {
+                                float *rew, int32_t *act_u, int32_t *act_c, int32_t *info_i, float *info_f,
+                                cudaStream_t st) {
   const mpe::EnvStateAny &s = env->st;
   const int64_t rows = s.B * s.N, obs_step = rows * s.D;
   auto up = [](size_t x) { return (x + 255) / 256 * 256; };
@@ -837,6 +843,8 @@ static int rollout_fused_replay(MpeEnv *env, MpeActor *actor, MpeReplay *rep, in
     io.rew = rew ? rew + t0 * rows : sc_rew;
     io.act_u = act_u ? act_u + t0 * rows : sc_au;
     io.act_c = s.act_c == 0 ? nullptr : (act_c ? act_c + t0 * rows : sc_ac);
+    io.info_i = info_i ? info_i + t0 * s.B * (s.N + 1) : nullptr;  // the ring does not read them: no scratch
+    io.info_f = info_f ? info_f + t0 * s.B : nullptr;
     CK(mpe::launch_rollout_tc(s, tcw, io, st));
     CK(mpe::launch_replay_add_steps(rep->dev, rep->head, s.B, io.T, (int64_t)t0 * s.B, keep_from, env->r_obs, io.obs_next,
                                     io.act_u, io.act_c, io.rew, st));
@@ -856,7 +864,7 @@ static int rollout_fused_replay(MpeEnv *env, MpeActor *actor, MpeReplay *rep, in
 }
 
 int mpe_rollout_replay(MpeEnv *env, MpeActor *actor, MpeReplay *rep, int32_t T, uint64_t step0, float *obs_next,
-                       float *rew, int32_t *act_u, int32_t *act_c, void *stream) {
+                       float *rew, int32_t *act_u, int32_t *act_c, int32_t *info_i, void *info_f, void *stream) {
   if (env == nullptr || actor == nullptr || rep == nullptr) return fail(MPE_EINVAL, "mpe_rollout_replay: null handle");
   if (T <= 0) return MPE_OK;
   if (int rc = check_rollout(env, actor, "mpe_rollout_replay")) return rc;
@@ -872,8 +880,9 @@ int mpe_rollout_replay(MpeEnv *env, MpeActor *actor, MpeReplay *rep, int32_t T, 
   // the fused kernel needs the episode ends of all envs to coincide: only there can a segment end and the ring
   // writer find every step's obs_t among the recordings
   if (use_fused_rollout(env, actor) && env->synced)
-    return rollout_fused_replay(env, actor, rep, T, step0, obs_next, rew, act_u, act_c, st);
-  return rollout_stepwise(env, actor, rep, T, step0, obs_next, rew, act_u, act_c, st);
+    return rollout_fused_replay(env, actor, rep, T, step0, obs_next, rew, act_u, act_c, info_i,
+                                static_cast<float *>(info_f), st);
+  return rollout_stepwise(env, actor, rep, T, step0, obs_next, rew, act_u, act_c, info_i, static_cast<float *>(info_f), st);
 }
 
 // ------------------------------------------------------------------------------------------------

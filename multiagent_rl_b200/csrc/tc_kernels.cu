@@ -297,7 +297,9 @@ __host__ __device__ inline size_t tc2_smem_bytes(uint32_t wbytes, int N, int Kx)
 __host__ __device__ inline size_t tc2_scratch_f2_per_cta(int N, int APAD) { return (size_t)2 * 2 * 2 * N * (APAD / 2) * kRows; }
 __host__ __device__ constexpr int tc2_threads(int N) { return N > 3 ? 384 : 320; }  // + two service warps for large teams
 
-template <int SC, int N, bool FUSED, int APAD>
+// INFO (fused rollouts only): also write the benchmark_data of every env-step to ro.info_i / ro.info_f.  A template
+// flag rather than a test of the pointers, so that the kernel of a rollout without them stays the same code.
+template <int SC, int N, bool FUSED, int APAD, bool INFO = false>
 __global__ void __launch_bounds__(tc2_threads(N), 1)
     k_tc2(EnvState<float> s, TcDev w, ActorIO io, RolloutIO ro, int max_episode_len, int64_t ntiles, int dbg) {
   // Large teams (N > 3, actor only): the obs operands do not fit next to the weights, so a per-tile OPERAND WARP
@@ -315,6 +317,7 @@ __global__ void __launch_bounds__(tc2_threads(N), 1)
   // every other small team (one head of <= 8 entries): the heads on the tensor pipe, logits accumulated in TMEM
   constexpr bool kTcHeads = tc2_tc_heads(N, APAD);
   static_assert(!(kJit && FUSED), "the fused rollout keeps every agent of an env in one thread: N <= 3");
+  static_assert(FUSED || !INFO, "benchmark_data is a rollout output");
   extern __shared__ __align__(128) unsigned char smem[];
 #ifdef MPE_TC_PHASES
   if (dbg && threadIdx.x == 0 && blockIdx.x < 148) {
@@ -981,6 +984,15 @@ __global__ void __launch_bounds__(tc2_threads(N), 1)
             int coll[N], occ;
             float md;
             e.reward(r, coll, occ, md, s);
+            if constexpr (INFO) {  // the values and layout of mpe_step's info_i / info_f, at [it][b]
+              if (ro.info_i != nullptr) {
+                int32_t *ii = ro.info_i + (toff + b) * (N + 1);
+#pragma unroll
+                for (int i = 0; i < N; ++i) ii[i] = coll[i];
+                ii[N] = occ;
+              }
+              if (ro.info_f != nullptr) ro.info_f[toff + b] = md;
+            }
             float sum = 0.0f;
 #pragma unroll
             for (int i = 0; i < N; ++i) { sum += r[i]; stage_rew[row * N + i] = r[i]; }
@@ -1089,19 +1101,19 @@ static int tc_debug_flag() {
 
 // Per-launch host work is kept to the launch itself (the fused step is a ~60 us kernel): one cudaGetDevice, everything
 // derived from the device is cached (launch.h).
-template <int SC, int N, bool FUSED, int APAD>
+template <int SC, int N, bool FUSED, int APAD, bool INFO = false>
 static cudaError_t launch_tc2_t(const EnvState<float> &s, const TcDev &w, const ActorIO &io, const RolloutIO &ro,
                                 int max_episode_len, int64_t nenvs, cudaStream_t st) {
   const int dev = current_device();
   const size_t smem = tc2_smem_bytes(w.bytes, N, w.Kx);
   if (smem > 227 * 1024) return cudaErrorInvalidValue;  // tc_*_supported rule these out
-  cudaError_t e = ensure_smem<k_tc2<SC, N, FUSED, APAD>>(smem, dev);
+  cudaError_t e = ensure_smem<k_tc2<SC, N, FUSED, APAD, INFO>>(smem, dev);
   if (e != cudaSuccess) return e;
   const int64_t ntiles = (nenvs + kRows - 1) / kRows;
   const int nsm = sm_count(dev);
   const int64_t pairs = (ntiles + 1) / 2;
   const int grid = (int)(pairs < nsm ? pairs : nsm);
-  k_tc2<SC, N, FUSED, APAD><<<grid, tc2_threads(N), smem, st>>>(s, w, io, ro, max_episode_len, ntiles, tc_debug_flag());
+  k_tc2<SC, N, FUSED, APAD, INFO><<<grid, tc2_threads(N), smem, st>>>(s, w, io, ro, max_episode_len, ntiles, tc_debug_flag());
   return cudaGetLastError();
 }
 
@@ -1138,14 +1150,23 @@ cudaError_t launch_actor_forward_tc(const TcDev &w, const ActorIO &io, cudaStrea
   }
 }
 
+template <int SC, int N, int APAD>
+static cudaError_t launch_rollout_tc_t(const EnvState<float> &s, const TcDev &w, const RolloutIO &ro, int max_episode_len,
+                                       cudaStream_t st) {
+  ActorIO io;
+  if (ro.info_i != nullptr || ro.info_f != nullptr)
+    return launch_tc2_t<SC, N, true, APAD, true>(s, w, io, ro, max_episode_len, s.B, st);
+  return launch_tc2_t<SC, N, true, APAD>(s, w, io, ro, max_episode_len, s.B, st);
+}
+
 cudaError_t launch_rollout_tc(const EnvStateAny &a, const TcDev &w, const RolloutIO &ro, cudaStream_t st) {
   EnvState<float> s = typed<float>(a);
   s.track = 1;  // the fused rollout always keeps the episode counters (mpe_track_returns)
-  ActorIO io;
-  if (a.scenario == kReference) return launch_tc2_t<kReference, 2, true, 16>(s, w, io, ro, a.max_episode_len, a.B, st);
-  if (a.scenario == kSpeaker) return launch_tc2_t<kSpeaker, 2, true, 8>(s, w, io, ro, a.max_episode_len, a.B, st);
-  if (a.N == 2) return launch_tc2_t<kSpread, 2, true, 8>(s, w, io, ro, a.max_episode_len, a.B, st);
-  if (a.N == 3) return launch_tc2_t<kSpread, 3, true, 8>(s, w, io, ro, a.max_episode_len, a.B, st);
+  const int L = a.max_episode_len;
+  if (a.scenario == kReference) return launch_rollout_tc_t<kReference, 2, 16>(s, w, ro, L, st);
+  if (a.scenario == kSpeaker) return launch_rollout_tc_t<kSpeaker, 2, 8>(s, w, ro, L, st);
+  if (a.N == 2) return launch_rollout_tc_t<kSpread, 2, 8>(s, w, ro, L, st);
+  if (a.N == 3) return launch_rollout_tc_t<kSpread, 3, 8>(s, w, ro, L, st);
   return cudaErrorInvalidValue;
 }
 

@@ -384,9 +384,14 @@ class BatchedMultiAgentEnv(object):
         return np.array(list(out), dtype=np.float64)
 
     # ------------------------------------------------------------------ fused rollout
-    def rollout(self, actor, T, step0=None, record=False, replay=None):
+    def rollout(self, actor, T, step0=None, record=False, replay=None, info=False):
         """T fused iterations of experiments/run.py:36-65 (act -> step -> reward -> auto-reset).
         ``record`` returns per-step (obs_next[T,B,N,D], rew[T,B,N], act_u[T,B,N], act_c[T,B,N] | None).
+        ``info`` also records upstream's ``benchmark_data`` of every step, bit for bit what ``step(info=True)`` returns
+        for it: the call returns (obs_next, rew, act_u, act_c, {'info_i': int32 [T,B,N+1], 'info_f': fp32 [T,B]}),
+        the first four None without ``record``.  info_i holds the collisions per agent and the occupied landmarks
+        (fullobs_collect_treasure: the 0 / 1 flags per agent and a zero), info_f the sum of min distances (None for
+        fullobs_collect_treasure).
         ``replay`` (a DeviceReplayBuffer) receives every env-step's transition (obs_t, act, sum of rewards, obs_t+1,
         done = 0) in step-major, then env order, as ``T`` calls of ``replay.add`` with ``B`` transitions each would:
         obs_t is the observation the actor acted on, the post-reset one at an episode's first step.
@@ -406,14 +411,20 @@ class BatchedMultiAgentEnv(object):
             rew = self._empty(T, B, N)
             au = self._empty(T, B, N, dtype=torch.int32)
             ac = self._empty(T, B, N, dtype=torch.int32) if self.act_c > 0 else None
+        info_i = self._empty(T, B, N + 1, dtype=torch.int32) if info else None
+        info_f = self._empty(T, B) if info and self.scenario_name != 'fullobs_collect_treasure' else None
         if replay is None:
             _lib.check(self._lib.mpe_rollout(self._h, actor._h, int(T), C.c_uint64(step0), _lib.ptr(obs), _lib.ptr(rew),
-                                             _lib.ptr(au), _lib.ptr(ac), self._stream()), 'mpe_rollout')
+                                             _lib.ptr(au), _lib.ptr(ac), _lib.ptr(info_i), _lib.ptr(info_f),
+                                             self._stream()), 'mpe_rollout')
         else:
             _lib.check(self._lib.mpe_rollout_replay(self._h, actor._h, replay._h, int(T), C.c_uint64(step0),
                                                     _lib.ptr(obs), _lib.ptr(rew), _lib.ptr(au), _lib.ptr(ac),
-                                                    self._stream()), 'mpe_rollout_replay')
+                                                    _lib.ptr(info_i), _lib.ptr(info_f), self._stream()),
+                       'mpe_rollout_replay')
         self.global_step = step0 + int(T)
+        if info:
+            return obs, rew, au, ac, {'info_i': info_i, 'info_f': info_f}
         return (obs, rew, au, ac) if record else None
 
     def _check_replay(self, replay):

@@ -92,6 +92,21 @@ for scen, n, B, cap in (('simple_spread', None, 129, 300), ('simple_reference', 
     env.reset(mask=(torch.arange(B, device='cuda') % 2).to(torch.uint8))
     env.rollout(actor, 4, replay=rb)
     rb.collect()
+# rollouts that record benchmark_data (info_i / info_f) at ragged sizes: the fused kernel, the per-step path (large
+# team, FFMA actor, treasure) and the ring on both of its paths
+for scen, n, B, impl in (('simple_spread', None, 129, 'auto'), ('simple_reference', None, 257, 'auto'),
+                         ('simple_spread', 9, 41, 'auto'), ('simple_spread', None, 33, 'simt'),
+                         ('fullobs_collect_treasure', None, 77, 'auto')):
+    env = m.make_env(scen, n=n, num_envs=B, batched=True, seed=3, max_episode_len=3)
+    A = [5, env.act_c] if env.act_c else 5
+    actor = m.FusedActor(random_state_dict(env.obs_dim, A, 1), seed=3, impl=impl)
+    rb = m.DeviceReplayBuffer(2 * B + 1, env.n, env.obs_dim, A)
+    env.reset()
+    env.rollout(actor, 5, record=True, info=True)
+    env.rollout(actor, 4, replay=rb, info=True)
+    env.reset(mask=(torch.arange(B, device='cuda') % 2).to(torch.uint8))
+    env.rollout(actor, 4, replay=rb, info=True)
+    rb.collect()
 # weight loads from CUDA tensors: every actor image layout (tensor-core image written, D > 32 where it is not, the
 # dense3 region past the staged blob), sources at 4 B-aligned offsets of one flat buffer; the critic with both heads
 for D, A, model in ((10, 5, False), (21, [5, 10], False), (28, 5, True), (57, 5, True)):
